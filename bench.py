@@ -3,6 +3,7 @@
 
     python bench.py --gpus N --steps K --warmup W            # our arm (libdcr.so, sm_100a)
     python bench.py --impl reference --steps K --warmup W    # CPU arm: the oracle's C port on the host cores
+    python bench.py --steps K --warmup W --dump-outputs DIR  # also write the last timed step's outputs as DIR/<name>.npy
 
 One JSON line on stdout (rank 0).  A "step" is one full pass of the hot path over the whole graph: plan + edge
 kernels (+ all-gather and re-interleave when N > 1).  Timing: CUDA events per step on the launching stream, an L2
@@ -613,6 +614,9 @@ def run_ours(args):
     plan_ms = [s0.elapsed_time(e0) for (s0, _), (e0, _) in zip(step_ev, edge_ev)]
     tail_ms = [e1.elapsed_time(s1) for (_, s1), (_, e1) in zip(step_ev, edge_ev)]
 
+    # what the last timed step computed, copied before the untimed passes below reuse the result buffers
+    last = {k: v.clone() for k, v in res.items()} if (args.dump_outputs and rank == 0) else None
+
     def untimed_step():
         flush.zero_()
         sh.run()
@@ -750,6 +754,7 @@ def run_ours(args):
     if rank == 0 and world == 1 and not args.no_dense:
         try:
             line["dense"] = dense_bench(args, torch)
+            del line["dense"]["outputs"]
         except Exception as exc:
             line["dense"] = {"unavailable": repr(exc)[:300]}
     if args.workload == "arxiv" and not args.no_cuda_flavour:
@@ -767,6 +772,8 @@ def run_ours(args):
             line["cuda_flavour"] = cf
     if rank == 0 and not args.no_sdrf:
         line["sdrf"] = sdrf_bench(args, torch)
+    if last is not None:
+        dump_outputs(args.dump_outputs, last)
     if rank == 0:
         emit(line)
     if world > 1:
@@ -781,7 +788,7 @@ def cuda_flavour_bench(args, torch, dist, csr, esrc_np, edst_np, rowptr, world, 
     from dcr import bfc
     from dcr.dist import ShardedCudaBFC
     E = int(esrc_np.size)
-    steps, warmup = max(5, min(args.steps, 20)), 3
+    steps, warmup = args.steps, 3
     sc = ShardedCudaBFC(csr)
     for _ in range(warmup + (3 if world > 1 else 0)):
         flush.zero_()
@@ -851,6 +858,25 @@ def emit(line: dict):
     out.flush()
 
 
+DUMP_LIMIT_BYTES = 64 << 20
+
+
+def dump_outputs(path: str, arrays: dict):
+    """`--dump-outputs DIR`: one DIR/<name>.npy per output array of the timed path's last step, so that two builds can
+    be compared output for output on the same seeded inputs.  Integer fields are widened to float64, which holds them
+    exactly."""
+    host = {}
+    for name, t in arrays.items():
+        a = t.cpu().numpy()
+        host[name] = a if a.dtype in (np.float32, np.float64) else a.astype(np.float64)
+    total = sum(a.nbytes for a in host.values())
+    if total > DUMP_LIMIT_BYTES:
+        raise SystemExit(f"--dump-outputs: {total} bytes of outputs exceed the {DUMP_LIMIT_BYTES}-byte limit")
+    os.makedirs(path, exist_ok=True)
+    for name, a in host.items():
+        np.save(os.path.join(path, f"{name}.npy"), a)
+
+
 def dense_bench(args, torch) -> dict:
     """Config 4: the dense-regime tensor path on the squirrel-shaped graph (1 GPU): supports A2[i,j] on the edges via the
     hand-written tcgen05 int8 A·A kernel, the full cuda-flavour pass through it, and the sorted-list route beside it."""
@@ -862,7 +888,8 @@ def dense_bench(args, torch) -> dict:
     ws = torch.empty(int(bfc.L.load().dcr_bfc_support_tc_workspace_bytes(n, csr.nnz)), dtype=torch.uint8, device="cuda")
     tri = torch.empty(csr.nnz, dtype=torch.int32, device="cuda")
     flush = torch.empty(256 << 20, dtype=torch.uint8, device="cuda")
-    steps, warmup = max(5, min(args.steps, 20)), 3
+    steps, warmup = args.steps, 3
+    last = {}
 
     def timed(fn):
         for _ in range(warmup):
@@ -872,7 +899,7 @@ def dense_bench(args, torch) -> dict:
             flush.zero_()
             e0, e1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
             e0.record()
-            fn()
+            last["out"] = fn()
             e1.record()
             e1.synchronize()
             out.append(e0.elapsed_time(e1))
@@ -882,6 +909,7 @@ def dense_bench(args, torch) -> dict:
     ws2 = torch.empty(int(bfc.L.load().dcr_bfc_cuda_flavour_tc_workspace_bytes(n, csr.nnz)), dtype=torch.uint8,
                       device="cuda")
     ms_full = timed(lambda: bfc.cuda_flavour_tc(csr, want_fields=False, workspace=ws2))
+    outputs = {k: last["out"][k] for k in ("tri", "c32")}        # per directed CSR entry
     ms_sparse = timed(lambda: bfc.support(csr, out=tri))
     ms_full_sparse = timed(lambda: bfc.cuda_flavour(csr, want_fields=False, tri=bfc.support(csr, out=tri)))
     same = bool(torch.equal(bfc.support_tc(csr), bfc.support(csr)))
@@ -902,6 +930,7 @@ def dense_bench(args, torch) -> dict:
                      "traffic": None, "support_tc_ms": ms_tc, "ops": ops},
         "sparse_path": {"support_ms": ms_sparse, "full_ms": ms_full_sparse,
                         "note": "sorted-list intersection kernels on the same CSR (dcr_bfc_support + dcr_bfc_cuda_flavour)"},
+        "outputs": outputs,
     }
 
 
@@ -938,6 +967,8 @@ def run_dense(args):
         raise SystemExit("bench.py needs a CUDA device")
     torch.cuda.set_device(0)
     d = dense_bench(args, torch)
+    if args.dump_outputs:
+        dump_outputs(args.dump_outputs, d["outputs"])
     line = {
         "metric": "bfc_edges_per_sec", "value": d["value"], "unit": "edges/s", "n_gpus": 1,
         "steps": d["steps"], "warmup": 3, "ms_per_step": d["ms_per_step"], "higher_is_better": True,
@@ -969,7 +1000,13 @@ def main():
     ap.add_argument("--no-cpu", action="store_true")
     ap.add_argument("--no-sdrf", action="store_true")
     ap.add_argument("--no-clocks", action="store_true", help="debug: do not sample clocks")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="write the arrays the timed path computed in its last step to DIR/<name>.npy (float32/float64)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl == "reference":
+        ap.error("--dump-outputs applies to our arm: the reference arm times seeded edge samples, not the full outputs")
     args.warmup = max(args.warmup, 3) if args.impl == "ours" else args.warmup
     if args.workload == "squirrel-dense":
         if args.impl == "reference":

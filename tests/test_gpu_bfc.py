@@ -555,6 +555,31 @@ def test_full_size_arxiv_shape_exact_against_c_oracle(paper_mode):
     assert np.array_equal(out["sq_i"].cpu().numpy() > 0, out["sq_j"].cpu().numpy() > 0)
 
 
+def test_bench_runs_the_requested_steps_and_dumps_the_outputs(tmp_path):
+    """`bench.py --steps K --dump-outputs DIR`: K timed steps, and DIR holds every field of the last one as float64,
+    equal to the C oracle on every edge of the workload."""
+    import json
+    import os
+    import subprocess
+    import sys
+    from conftest import REPO
+    from oracle.c_port import bfc_paper_c
+    sys.path.insert(0, REPO)
+    import bench
+    r = subprocess.run([sys.executable, os.path.join(REPO, "bench.py"), "--workload", "cora", "--steps", "2",
+                        "--warmup", "0", "--no-dense", "--no-cpu", "--no-sdrf", "--no-clocks",
+                        "--dump-outputs", str(tmp_path)], capture_output=True, text=True, timeout=600)
+    assert r.returncode == 0, r.stderr[-2000:]
+    d = json.loads(r.stdout)
+    assert d["steps"] == 2 and len(d["step_ms"]) == 2
+    _, _, rowptr, col, esrc, edst = bench.build_graph("cora")
+    ref = bfc_paper_c(rowptr, col, esrc, edst)
+    assert sorted(os.listdir(tmp_path)) == sorted(f"{k}.npy" for k in ref)
+    for k, want in ref.items():
+        got = np.load(tmp_path / f"{k}.npy")
+        assert got.dtype == np.float64 and np.array_equal(got, want), k
+
+
 def test_edge_centric_cuda_flavour_matches_per_entry_kernels_and_oracle():
     """dcr_bfc_cuda_edges (one work item per undirected edge, hub-hub edges by a CTA) against the per-entry kernels at
     every size incl. the arxiv shape, and against the dense oracle on small graphs; a single-GPU dcr_comm run of the

@@ -1,4 +1,4 @@
-"""CPU suite, part 4 (build container only): the reference's CONSUMERS of the hot path run unchanged.
+"""CPU suite, part 4: the reference's CONSUMERS of the hot path run unchanged.
 
 `models/gcn.py` and `experiment/training_loop.py` are imported from /root/reference without edits, on the
 `torch_geometric` stand-in, and trained on a synthetic node-classification task over a graph in exactly the form the
@@ -14,7 +14,6 @@ import pytest
 import torch
 
 REFERENCE = "/root/reference"
-pytestmark = pytest.mark.skipif(not os.path.isdir(os.path.join(REFERENCE, "models")), reason="reference checkout absent")
 
 
 def _import_reference_consumers():
@@ -43,6 +42,7 @@ def _synthetic_task(n, edge_index, classes=3, feats=16, seed=0):
     return InMemoryDataset(data, num_classes=classes), data
 
 
+@pytest.mark.skipif(not os.path.isdir(os.path.join(REFERENCE, "models")), reason="reference checkout absent")
 def test_reference_gcn_and_training_loop_run_unchanged_on_rewired_graph():
     gcn, loop = _import_reference_consumers()
     from dcr.synth import named_graph

@@ -14,7 +14,8 @@
 //   5. incremental refresh of the curvature of the dirty edges only (SURVEY.md App. H): edges at the four touched
 //      endpoints and edges closing a triangle with an edge whose support changed.
 // No host round trip inside the loop; one 8-int log record per iteration.  The loop is inherently sequential
-// (iteration t+1 needs the graph of iteration t), hence one CTA: "replicas only" across GPUs.
+// (iteration t+1 needs the graph of iteration t), hence one CTA per run; independent runs go side by side, one CTA
+// each, in one launch of the batch kernel (dcr_sdrf_run_batch).
 #include <algorithm>
 #include <cmath>
 #include <vector>
@@ -41,12 +42,14 @@ constexpr uint32_t IMP_MASKED = 0xffffffffu;   // bit pattern marking a masked c
 constexpr int STATUS_TOO_MANY_CANDIDATES = DCR_SDRF_TOO_MANY_CANDIDATES;
 
 // Optional phase timers (build with -DDCR_SDRF_PROFILE): cycles per phase summed over the iterations of a launch,
-// written to a device array read back with dcr_sdrf_phase_cycles().  Compiled out of the product library.
+// written to a device array read back with dcr_sdrf_phase_cycles().  Compiled out of the product library.  The array
+// is one global without atomics, so only the single-run kernel ticks (TIMED = true); the batch kernel, whose CTAs
+// would race on it, instantiates the loop body with TIMED = false.
 #ifdef DCR_SDRF_PROFILE
 __device__ unsigned long long g_sdrf_phase[16];
 #define SDRF_TICK(slot)                                                         \
     do {                                                                        \
-        if (threadIdx.x == 0) {                                                 \
+        if (TIMED && threadIdx.x == 0) {                                        \
             const long long now__ = clock64();                                  \
             g_sdrf_phase[slot] += (unsigned long long)(now__ - tick__);         \
             tick__ = now__;                                                     \
@@ -539,11 +542,14 @@ __global__ void sdrf_init_curvature_kernel(SdrfDev S, int top) {
 // ------------------------------------------------------------------------------------------------------------
 // the loop
 // ------------------------------------------------------------------------------------------------------------
-template <int MODE>
-__global__ void __launch_bounds__(SDRF_THREADS, 1)
-sdrf_loop_kernel(SdrfDev S, int loops, int remove_edges, float bound32, double bound64, double tau, int tau_inf,
-                 const double* __restrict__ uniforms, long long n_uniforms, int forced_choice, double guard,
-                 int32_t* __restrict__ log, dcr_sdrf_result* __restrict__ result) {
+// One run of the loop on the calling CTA.  Block-uniform arguments only; nothing here reads blockIdx or gridDim, so the
+// single-run kernel and every CTA of the batch kernel execute the same code on their own state.
+template <int MODE, bool TIMED>
+__device__ __forceinline__ void sdrf_loop_body(const SdrfDev& S, int loops, int remove_edges, float bound32,
+                                               double bound64, double tau, int tau_inf,
+                                               const double* __restrict__ uniforms, long long n_uniforms,
+                                               int forced_choice, double guard, int32_t* __restrict__ log,
+                                               dcr_sdrf_result* __restrict__ result) {
     __shared__ LoopShared sh;
     __shared__ DirScoreShared dsh;
     __shared__ int dirty_count, work_count, dred[2];
@@ -957,6 +963,42 @@ sdrf_loop_kernel(SdrfDev S, int loops, int remove_edges, float bound32, double b
     }
 }
 
+template <int MODE>
+__global__ void __launch_bounds__(SDRF_THREADS, 1)
+sdrf_loop_kernel(SdrfDev S, int loops, int remove_edges, float bound32, double bound64, double tau, int tau_inf,
+                 const double* __restrict__ uniforms, long long n_uniforms, int forced_choice, double guard,
+                 int32_t* __restrict__ log, dcr_sdrf_result* __restrict__ result) {
+    sdrf_loop_body<MODE, true>(S, loops, remove_edges, bound32, bound64, tau, tau_inf, uniforms, n_uniforms,
+                               forced_choice, guard, log, result);
+}
+
+// Per-run arguments of the batch kernel (dcr_sdrf_run_batch packs one per run into the caller's workspace).
+struct SdrfBatchDesc {
+    SdrfDev S;
+    int loops, forced_choice, tau_inf;
+    float bound32;
+    double bound64, tau;
+    const double* uniforms;
+    long long n_uniforms;
+    int32_t* log;
+    dcr_sdrf_result* result;
+};
+static_assert(sizeof(SdrfBatchDesc) % 8 == 0, "descriptor copied as 8-byte words");
+
+// B independent runs, one CTA each (gridDim.x = B; CTAs beyond one per SM run in later waves).  The descriptor is
+// copied to shared memory once, so the arena pointers are read from there rather than from global memory on every use.
+template <int MODE>
+__global__ void __launch_bounds__(SDRF_THREADS, 1)
+sdrf_batch_loop_kernel(const SdrfBatchDesc* __restrict__ descs, int remove_edges, double guard) {
+    __shared__ SdrfBatchDesc d;
+    constexpr int WORDS = sizeof(SdrfBatchDesc) / 8;
+    const unsigned long long* src = reinterpret_cast<const unsigned long long*>(descs + blockIdx.x);
+    if (threadIdx.x < WORDS) reinterpret_cast<unsigned long long*>(&d)[threadIdx.x] = src[threadIdx.x];
+    __syncthreads();
+    sdrf_loop_body<MODE, false>(d.S, d.loops, remove_edges, d.bound32, d.bound64, d.tau, d.tau_inf, d.uniforms,
+                                d.n_uniforms, d.forced_choice, guard, d.log, d.result);
+}
+
 // ------------------------------------------------------------------------------------------------------------
 // export
 // ------------------------------------------------------------------------------------------------------------
@@ -1198,6 +1240,61 @@ extern "C" int dcr_sdrf_run(dcr_sdrf* s, int loops, int remove_edges, double rem
     else if (s->mode == DCR_SDRF_MODE_BFC_DIRECTED) SDRF_LAUNCH(LOOP_DIRECTED);
     else SDRF_LAUNCH(LOOP_CLASSICAL);
 #undef SDRF_LAUNCH
+    DCR_LAUNCH_CHECK();
+    return 0;
+}
+
+extern "C" int64_t dcr_sdrf_batch_workspace_bytes(int count) {
+    return count < 1 ? 0 : (int64_t)count * (int64_t)sizeof(SdrfBatchDesc);
+}
+
+extern "C" int dcr_sdrf_run_batch(const dcr_sdrf_batch_run* runs, int count, int remove_edges, double guard,
+                                  void* workspace, int64_t workspace_bytes, void* stream) {
+    if (count < 1 || !runs) { set_error("dcr_sdrf_run_batch: count must be >= 1"); return 1; }
+    std::vector<SdrfBatchDesc> descs(count);
+    std::vector<const dcr_sdrf*> seen(count);
+    for (int b = 0; b < count; ++b) {
+        const dcr_sdrf_batch_run& r = runs[b];
+        if (!r.state) { set_error("dcr_sdrf_run_batch: run %d has no state", b); return 1; }
+        if (!r.result || (r.loops > 0 && !r.log)) { set_error("dcr_sdrf_run_batch: run %d: bad arguments", b); return 1; }
+        if (r.state->mode != runs[0].state->mode) {
+            set_error("dcr_sdrf_run_batch: run %d has loop mode %d, run 0 has %d (one mode per call)", b, r.state->mode,
+                      runs[0].state->mode);
+            return 1;
+        }
+        SdrfBatchDesc& d = descs[b];
+        d.S = r.state->dev;
+        d.loops = r.loops;
+        d.forced_choice = r.forced_choice;
+        d.tau_inf = std::isinf(r.tau) && r.tau > 0;
+        d.bound32 = (float)r.removal_bound;
+        d.bound64 = r.removal_bound;
+        d.tau = r.tau;
+        d.uniforms = r.uniforms;
+        d.n_uniforms = (long long)r.n_uniforms;
+        d.log = r.log;
+        d.result = r.result;
+        seen[b] = r.state;
+    }
+    std::sort(seen.begin(), seen.end());
+    if (std::adjacent_find(seen.begin(), seen.end()) != seen.end()) {
+        set_error("dcr_sdrf_run_batch: the same state appears twice (runs of one call must own their states)");
+        return 1;
+    }
+    if (!workspace || workspace_bytes < dcr_sdrf_batch_workspace_bytes(count)) {
+        set_error("dcr_sdrf_run_batch: workspace of dcr_sdrf_batch_workspace_bytes(%d) = %lld bytes required", count,
+                  (long long)dcr_sdrf_batch_workspace_bytes(count));
+        return 1;
+    }
+    if ((uintptr_t)workspace % alignof(SdrfBatchDesc)) { set_error("dcr_sdrf_run_batch: workspace must be 8-byte aligned"); return 1; }
+    cudaStream_t st = (cudaStream_t)stream;
+    // pageable source: the copy is staged before cudaMemcpyAsync returns, so `descs` may go out of scope
+    DCR_CUDA(cudaMemcpyAsync(workspace, descs.data(), sizeof(SdrfBatchDesc) * count, cudaMemcpyHostToDevice, st));
+    const SdrfBatchDesc* dd = (const SdrfBatchDesc*)workspace;
+    const int mode = runs[0].state->mode;
+    if (mode == DCR_SDRF_MODE_BFC) sdrf_batch_loop_kernel<LOOP_BFC><<<count, SDRF_THREADS, 0, st>>>(dd, remove_edges, guard);
+    else if (mode == DCR_SDRF_MODE_BFC_DIRECTED) sdrf_batch_loop_kernel<LOOP_DIRECTED><<<count, SDRF_THREADS, 0, st>>>(dd, remove_edges, guard);
+    else sdrf_batch_loop_kernel<LOOP_CLASSICAL><<<count, SDRF_THREADS, 0, st>>>(dd, remove_edges, guard);
     DCR_LAUNCH_CHECK();
     return 0;
 }

@@ -18,6 +18,13 @@ class SdrfResult(C.Structure):
                 ("pending_y", C.c_int32), ("reserved", C.c_int32)]
 
 
+class SdrfBatchRun(C.Structure):
+    """``dcr_sdrf_batch_run``: one run of ``dcr_sdrf_run_batch`` (pointers are device pointers)."""
+    _fields_ = [("state", C.c_void_p), ("loops", C.c_int32), ("forced_choice", C.c_int32),
+                ("removal_bound", C.c_double), ("tau", C.c_double), ("uniforms", C.c_void_p),
+                ("n_uniforms", C.c_int64), ("log", C.c_void_p), ("result", C.c_void_p)]
+
+
 # status codes of include/dcr.h
 SDRF_OK, SDRF_NEED_HOST, SDRF_PROB_NAN, SDRF_PROB_SUM, SDRF_REMOVE_NONEDGE, SDRF_NO_UNIFORM, SDRF_ARENA_FULL, \
     SDRF_TOO_MANY_CANDIDATES, SDRF_EMPTY_GRAPH = range(9)
@@ -73,6 +80,8 @@ SIGNATURES = {
     "dcr_sdrf_create_mode": (_I, [_I, _I, _P, _P, _P, _P, _L, C.POINTER(_P)]),
     "dcr_sdrf_destroy": (None, [_P]),
     "dcr_sdrf_run": (_I, [_P, _I, _I, _D, _D, _P, _L, _I, _D, _P, _P, _P]),
+    "dcr_sdrf_batch_workspace_bytes": (_L, [_I]),
+    "dcr_sdrf_run_batch": (_I, [_P, _I, _I, _D, _P, _L, _P]),
     "dcr_sdrf_pending_improvements": (_I, [_P, _P, _L, _P]),
     "dcr_sdrf_nnz": (_L, [_P]),
     "dcr_sdrf_export": (_I, [_P, _P, _P, _P, _P, _P, _P]),

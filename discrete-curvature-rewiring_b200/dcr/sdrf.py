@@ -227,3 +227,148 @@ def sdrf(edge_index, num_nodes: int, loops: int, remove_edges: bool, removal_bou
     if return_log:
         return edge_index_out, (np.concatenate(logs) if logs else np.zeros((0, L.SDRF_LOG_INTS), dtype=np.int32))
     return edge_index_out
+
+
+def batch_workspace(count: int, device) -> torch.Tensor:
+    """Device workspace for ``run_batch`` over up to ``count`` runs (8-byte aligned)."""
+    nbytes = int(L.load().dcr_sdrf_batch_workspace_bytes(int(count)))
+    return torch.empty(max(nbytes // 8, 1), dtype=torch.int64, device=device)
+
+
+def run_batch(states, loops, removal_bounds, taus, uniforms, forced, logs, remove_edges: bool, guard: float,
+              results: torch.Tensor, workspace: torch.Tensor):
+    """One ``dcr_sdrf_run_batch`` launch: run ``b`` continues ``states[b]`` for up to ``loops[b]`` iterations, drawing
+    from the device fp64 tensor ``uniforms[b]`` and logging into the device int32 tensor ``logs[b]`` (``[loops[b], 8]``,
+    may be ``None`` when ``loops[b] == 0``).  ``results`` is a device int32 ``[>= B, 8]`` tensor.  Returns the B result
+    dicts of ``SdrfState.run`` after ONE device-to-host copy."""
+    b = len(states)
+    runs = (L.SdrfBatchRun * b)()
+    for i, s in enumerate(states):
+        runs[i] = L.SdrfBatchRun(s.handle, int(loops[i]), int(forced[i]), float(removal_bounds[i]), float(taus[i]),
+                                 uniforms[i].data_ptr(), int(uniforms[i].numel()), L.ptr(logs[i]),
+                                 results[i].data_ptr())
+    L.check(L.load().dcr_sdrf_run_batch(runs, b, int(bool(remove_edges)), float(guard), workspace.data_ptr(),
+                                        workspace.numel() * workspace.element_size(), L.current_stream()),
+            "dcr_sdrf_run_batch")
+    keys = ("status", "iterations_done", "draws_used", "stopped", "pending_n", "pending_x", "pending_y")
+    return [dict(zip(keys, r)) for r in results[:b].cpu().tolist()]
+
+
+def _per_run(name: str, value, count: int) -> list:
+    is_seq = isinstance(value, (list, tuple)) or (isinstance(value, (np.ndarray, torch.Tensor)) and value.ndim > 0)
+    if not is_seq:
+        return [value] * count
+    out = list(value)
+    if len(out) != count:
+        raise ValueError(f"{name}: {len(out)} values for a batch of {count} runs")
+    return out
+
+
+def sdrf_batch(edge_indices, num_nodes, loops, remove_edges: bool, removal_bound, tau, *, uniforms,
+               guard: float = 1e-9, return_log: bool = False, is_undirected: bool = True, curv_type: str = "bfc",
+               return_exceptions: bool = False):
+    """B independent SDRF runs in one kernel launch, one CTA per run.  Run ``r`` computes exactly what
+    ``sdrf(edge_indices[r], num_nodes[r], loops[r], remove_edges, removal_bound[r], tau[r], uniforms=uniforms[r],
+    guard=guard, is_undirected=is_undirected, curv_type=curv_type)`` computes.
+
+    ``edge_indices``: a list / tuple of B inputs, or ONE input (array or tensor) shared by every run (its networkx
+    order is computed once).  ``num_nodes``, ``loops``, ``removal_bound``, ``tau``: scalars or length-B sequences.
+    ``uniforms``: a ``[B, loops]`` array or a list of B 1-d arrays; it fixes B.  The batch never reads numpy's global
+    generator (the draws of concurrent runs cannot be interleaved the way sequential calls would consume them).
+
+    Runs that need a host-side decision (``guard``) re-enter together in the next launch; a failing run does not stop
+    the others.  Returns a list of B ``edge_index`` arrays (and, with ``return_log``, a list of B logs).  A failed run
+    raises after the batch — the lowest-index one, with the type and message ``sdrf`` raises — or, with
+    ``return_exceptions``, leaves its exception in its ``edge_index`` slot (its log slot holds the iterations it
+    completed)."""
+    if isinstance(uniforms, np.ndarray) and uniforms.ndim != 2:
+        raise ValueError("uniforms: a [B, loops] array or a list of B 1-d arrays")
+    uni = [np.ascontiguousarray(u, dtype=np.float64) for u in uniforms]
+    count = len(uni)
+    if count < 1:
+        raise ValueError("sdrf_batch: an empty batch")
+    if any(u.ndim != 1 for u in uni):
+        raise ValueError("uniforms: a [B, loops] array or a list of B 1-d arrays")
+    shared_input = not isinstance(edge_indices, (list, tuple))
+    inputs = [edge_indices] * count if shared_input else _per_run("edge_indices", edge_indices, count)
+    nodes = [int(v) for v in _per_run("num_nodes", num_nodes, count)]
+    iters = [max(int(v), 0) for v in _per_run("loops", loops, count)]
+    bounds = [float(v) for v in _per_run("removal_bound", removal_bound, count)]
+    taus = _per_run("tau", tau, count)
+    if curv_type != "bfc" and curv_type not in CLASSICAL_MODES:
+        raise Exception(f"Method {curv_type} not available.")    # classical_curvatures.py:27-28
+    directed = curv_type == "bfc" and not is_undirected
+    L.require_cuda()
+
+    orders = {}
+
+    def order_of(r):
+        key = nodes[r] if shared_input else r
+        if key not in orders:
+            if curv_type != "bfc":
+                orders[key] = G.classical_order(inputs[r], nodes[r], keep_self_loops=True)
+            elif directed:
+                orders[key] = G.digraph_order(inputs[r], nodes[r], keep_self_loops=True)
+            else:
+                orders[key] = G.networkx_order(inputs[r], nodes[r], keep_self_loops=True)
+        return orders[key]
+
+    mode = (L.SDRF_MODE_BFC_DIRECTED if directed else L.SDRF_MODE_BFC) if curv_type == "bfc" \
+        else CLASSICAL_MODES[curv_type]
+    states = []
+    try:
+        for r in range(count):
+            o = order_of(r)
+            if directed:
+                states.append(SdrfState(o[0], o[1], max_additions=iters[r], mode=mode, in_rowptr=o[2], in_order=o[3]))
+            else:
+                states.append(SdrfState(o[0], o[1], max_additions=iters[r], mode=mode))
+        dev = states[0].device
+        # per run as in sdrf(): uniforms shorter than loops are padded with NaN ("not supplied")
+        padded = [np.concatenate([u, np.full(iters[r] - u.size, np.nan)]) if u.size < iters[r] else u
+                  for r, u in enumerate(uni)]
+        supplied = [int(np.count_nonzero(~np.isnan(u))) for u in padded]
+        u_dev = [torch.from_numpy(u).to(dev) for u in padded]
+        logs = [torch.empty((max(iters[r], 1), L.SDRF_LOG_INTS), dtype=torch.int32, device=dev) for r in range(count)]
+        results = torch.zeros((count, 8), dtype=torch.int32, device=dev)
+        workspace = batch_workspace(count, dev)
+        done, draws, forced = [0] * count, [0] * count, [-1] * count
+        errors = [None] * count
+        active = [r for r in range(count) if iters[r] > 0]
+        while active:
+            res = run_batch([states[r] for r in active], [iters[r] - done[r] for r in active],
+                            [bounds[r] for r in active], [taus[r] for r in active],
+                            [u_dev[r][draws[r]:supplied[r]] if supplied[r] > draws[r] else u_dev[r][:0] for r in active],
+                            [forced[r] for r in active], [logs[r][done[r]:] for r in active], remove_edges, guard,
+                            results, workspace)
+            again = []
+            for r, rr in zip(active, res):
+                forced[r] = -1
+                done[r] += rr["iterations_done"]
+                draws[r] += rr["draws_used"]
+                try:
+                    if rr["status"] == L.SDRF_NEED_HOST:
+                        imp = states[r].pending_improvements(rr["pending_n"])
+                        forced[r] = host_choice(imp, taus[r], float(padded[r][draws[r]]))
+                        again.append(r)
+                    elif rr["status"] != L.SDRF_OK:
+                        _raise_for_status(rr["status"])
+                except Exception as e:      # this run is over; the others go on
+                    errors[r] = e
+            active = again
+        outs, out_logs = [], []
+        for r in range(count):
+            out_logs.append(logs[r][: done[r]].cpu().numpy())
+            if errors[r] is not None:
+                outs.append(errors[r])
+                continue
+            rp, od = states[r].export()
+            outs.append((G.from_digraph_order if directed else G.from_networkx_order)(rp, od))
+    finally:
+        for s in states:
+            s.close()
+    if not return_exceptions:
+        first = next((e for e in errors if e is not None), None)
+        if first is not None:
+            raise first
+    return (outs, out_logs) if return_log else outs

@@ -291,6 +291,24 @@ void dcr_sdrf_destroy(dcr_sdrf* s);
 int dcr_sdrf_run(dcr_sdrf* s, int loops, int remove_edges, double removal_bound, double tau,
                  const double* uniforms, int64_t n_uniforms, int forced_choice, double guard, int32_t* log,
                  dcr_sdrf_result* result, void* stream);
+/* Batched runs: `count` independent loops in ONE launch, one persistent CTA per run (runs beyond one per SM wait for
+ * a free SM).  Each record carries what dcr_sdrf_run takes per run; remove_edges and guard apply to every run.  `runs`
+ * is a host array; the library packs one device descriptor per run into `workspace` (device memory of at least
+ * dcr_sdrf_batch_workspace_bytes(count) bytes, 8-byte aligned, reusable once the launch has been consumed in stream
+ * order) with one host-to-device copy on `stream`, then launches; it allocates nothing.  Status 1 before any launch
+ * for count < 1, a null state, the same state twice, states of different DCR_SDRF_MODE_* or a short workspace.
+ * Every run then behaves exactly as its own dcr_sdrf_run call would. */
+typedef struct dcr_sdrf_batch_run {      /* one run of dcr_sdrf_run_batch; pointers are device pointers */
+    dcr_sdrf* state;
+    int32_t loops, forced_choice;        /* as in dcr_sdrf_run                                          */
+    double removal_bound, tau;
+    const double* uniforms; int64_t n_uniforms;
+    int32_t* log;                        /* int32[loops][8]                                              */
+    dcr_sdrf_result* result;
+} dcr_sdrf_batch_run;
+int64_t dcr_sdrf_batch_workspace_bytes(int count);
+int dcr_sdrf_run_batch(const dcr_sdrf_batch_run* runs, int count, int remove_edges, double guard,
+                       void* workspace, int64_t workspace_bytes, void* stream);
 /* Improvements (fp64 of the fp32 differences, candidate order) of the pending iteration after NEED_HOST. */
 int dcr_sdrf_pending_improvements(dcr_sdrf* s, double* out, int64_t capacity, void* stream);
 /* Current number of directed entries (synchronises). */

@@ -8,23 +8,24 @@
 //   gamma     = max over squares of |N(k) ∩ M_j| resp. |N(m) ∩ M_i|           (:36-37; the "-1" removes i / j)
 // i.e. everything is a function of cnt(m) = |N(m) ∩ M_i| for m in M_j and cnt(k) = |N(k) ∩ M_j| for k in M_i.
 //
-// Mapping to the GPU (v11).  (a,b) = (i,j) or (j,i): b is the endpoint whose 2-hop lists are CHEAPER to stream
+// Mapping to the GPU.  (a,b) = (i,j) or (j,i): b is the endpoint whose 2-hop lists are CHEAPER to stream
 // (smaller S_b - d_a); a is the TESTED endpoint.  Edges are grouped by their tested endpoint (device counting sort),
-// so that the membership structures of N(a) — an open-addressing hash table and, in front of it, a hashed bitmap —
-// are built once per group and READ-ONLY afterwards:
-//   * LIGHT edges (<= HEAVY_STREAM streamed entries; 98.8 % of the edges and 80 % of the stream of the arxiv-shaped
-//     graph): ONE WARP PER EDGE.  For d_a <= 128 the table is private to the warp and kept while consecutive edges
-//     share a; above that the CTA builds one table for a run of edges of the same a and its warps pull edges from
-//     a shared counter.  The warp streams the lists N(m), m a pure neighbour of b, as ONE flat stream: the (begin,
-//     prefix) of up to 32 lists live in the lanes' registers, the owner of flat element f is found with one
-//     warp-wide OR-reduction of the "a list starts here" bits plus a popc, and the list data come through shuffles —
-//     no per-element search loop, no shared-memory prefix arrays.  An element k is a bipartite edge (m,k) iff it is
-//     in N(a) (bitmap, then exact probe), is not b and is not a common neighbour (binary search in the sorted row
-//     of b — only the few elements that passed the table reach it).  Matches bump the list's counter (-> cnt(m))
-//     and a small per-warp hash keyed by the table slot (-> cnt(k)): #squares and gamma of BOTH endpoints from one
-//     scan.  A warp whose match hash fills up defers the edge to the CTA-team path (overflow list).
-//   * HEAVY edges (hub–hub, up to 2.5e5 streamed entries each) and every edge with d_a > 16384: one CTA per edge
-//     (the v10 CTA-team kernel below: slot counters in the table, CTA-wide flat stream cut into equal warp slices).
+// so that the membership structures of N(a) are built once per group and READ-ONLY afterwards.  The edge classes
+// below decide which kernel takes an edge:
+//   * ONE WARP PER EDGE for most edges.  For d_a <= 128 the table is private to the warp and kept while consecutive
+//     edges share a (paper_light_warp_kernel); above that the CTA of a group kernel builds one structure for a run of
+//     edges of the same a and its warps pull edges from a shared counter (warp_edge).  The warp streams the lists
+//     N(m), m a pure neighbour of b, 32 heads at a time (warp_chunk): long lists one by one, the short ones as ONE flat
+//     stream whose owner arithmetic lives in the lanes' registers — no per-element search loop, no shared-memory
+//     prefix arrays.  An element k is a bipartite edge (m,k) iff it is in N(a) (filter, then exact test), is not b and
+//     is not a common neighbour (an exact set of T = N(a) ∩ N(b), or a mark in the d_a <= 128 table).  Matches bump
+//     the list's counter (-> cnt(m)) and a match hash keyed by k (-> cnt(k)): #squares and gamma of BOTH endpoints
+//     from one scan.  A warp whose match hash fills up leaves the edge to its CTA, which retries it at the end of the
+//     run (cta_edge_retry: the CTA-wide hash, then a hash in global memory).
+//   * COOPERATIVE edges (streams too long for one warp; hub–hub edges reach 2.5e5 streamed entries): one CTA of a
+//     group kernel per edge (cta_edge), drained first; the longest are SPLIT into parts that different CTAs process.
+//   * hashed mode, d_a > 16384: the CTA-team kernel (paper_edge_kernel), one 1024-thread CTA per edge, its table of
+//     N(a) and slot counters in global memory, the CTA-wide flat stream cut into equal warp slices.
 // Global traffic is at most the algorithmic gather of SURVEY.md §8d (which charges BOTH sides' 2-hop lists): the
 // two endpoint lists once and the cheaper side's 2-hop lists once per edge.  The CSR of the benchmark graphs is
 // L2-resident, so the kernel is bound by instruction issue / L1 gathers / shared-memory probes, not by DRAM.
@@ -39,16 +40,21 @@ namespace dcr {
 
 constexpr uint32_t EMPTY = 0xffffffffu;
 constexpr uint32_t KEYMASK = 0x3fffffffu;
-// Edge classes.  d_a = degree of the TESTED endpoint (the one whose neighbour set goes into the hash table).
-//   L0  d_a <= 128, stream <= COOP_L0    warp per edge, warp-private 256-slot table
-//   G1  d_a <= 1024, stream <= COOP_G    CTA-shared 2048-slot table, 8 warps, warp per edge
-//   G2  d_a <= 16384, stream <= COOP_G   CTA-shared 32768-slot table, 16 warps, warp per edge
-//   C1 / C2  the longer streams          same kernels and tables as G1 / G2, one CTA per edge, drained FIRST
-//   X   d_a > 16384                      1024-thread CTA team, table and 32-bit counters in global memory (L2)
-//   dense mode (n <= DENSE_MAX_N): L0 as above, everything else in ONE group class (G1 id) whose membership
-//   structure is an exact bitmap over all node ids in shared memory — no table, no false positives, any degree
-//   (an edge whose per-warp match hash fills up is retried by its CTA with the CTA-wide hash, and if that fills up
-//    too, with a hash in global memory sized for the largest degree)
+// Edge classes.  d_a = degree of the TESTED endpoint (the one whose neighbour set goes into the membership structure).
+// Hashed mode (n > DENSE_MAX_N, or forced): a hashed bitmap in front of a key-only open-addressing table.
+//   L0  d_a <= 128, stream <= COOP_L0    paper_light_warp_kernel: warp per edge, warp-private 256-slot table
+//   G1  d_a <= 1024, stream <= COOP_G    paper_group_kernel: CTA-shared 2048-slot table, 8 warps, warp per edge
+//   G2  d_a <= 16384, stream <= COOP_G   paper_group_kernel: CTA-shared 32768-slot table, 16 warps, warp per edge
+//   C1 / C2  the longer streams          the group kernels of G1 / G2 (C1 also takes the long streams of L0), one CTA
+//                                        per edge, drained FIRST
+//   X   d_a > 16384, any stream          paper_edge_kernel: 1024-thread CTA team, table and 32-bit counters in global
+//                                        memory (L2)
+// Dense mode (n <= DENSE_MAX_N): L0 as above; every other edge is G1 or C1, and ONE group kernel takes both, its
+// membership structure an exact bitmap over all node ids in shared memory — no table, no false positives, any degree.
+// G2, C2 and X stay empty.
+// In both modes an edge that a group kernel's warp cannot finish (its match hash fills up, or more than TRI_DEFER
+// triangles) is retried by the warp's CTA with the CTA-wide hash, and if that fills up too, with a hash in global
+// memory sized for the largest degree.
 enum { CL_L0 = 0, CL_G1, CL_G2, CL_C1, CL_C2, CL_X, N_CLASSES };   // C1 / C2: the cooperative edges of G1 / G2
 constexpr int CLASS_DA0 = 128, CLASS_DA1 = 1024, CLASS_DA2 = 16384;
 #ifndef DCR_COOP_L0
@@ -103,15 +109,13 @@ constexpr long long SIZE_B1 = 2048, SIZE_B2 = 512;
 constexpr int RUN_EDGES = DCR_RUN_EDGES;
 __host__ __device__ inline int run_table_of(int cls) { return cls == CL_G2 ? 1 : 0; }
 __host__ __device__ inline int coop_class_of(int cls) { return cls == CL_G2 ? CL_C2 : CL_C1; }
-constexpr int BIG_SLOTS = 32768, BIG_THREADS = 1024;
-__host__ __device__ constexpr int heads_per_thread(int team) { return team >= 1024 ? 1 : 4; }   // CTA stream state must fit beside the table
+// Class X (CTA-team kernel): BIG_THREADS threads, one head of N(vb) per thread and round; its stream state is
+// pre[BIG_THREADS+1] | beg[BIG_THREADS] | cnt[BIG_THREADS] (+ padding) in shared memory.
+constexpr int BIG_THREADS = 1024, BIG_STREAM_INTS = 3 * BIG_THREADS + 8;
 // Membership pre-filter: a hashed bitmap of N(va) (bit index = node id mod B).  Almost every streamed element is NOT
 // a neighbour of va, and the bitmap says so with one shared-memory load and no loop; only the few elements whose bit
 // is set (true members + d_a/B false positives) go on to the exact hash probe.
-constexpr int BIG_BITS = 131072, GLOBAL_BITS = 1048576;
-__host__ __device__ constexpr int filter_bits(int team, bool global_table) {
-    return global_table ? GLOBAL_BITS : BIG_BITS;
-}
+constexpr int GLOBAL_BITS = 1048576;
 #ifndef DCR_UNROLL
 #define DCR_UNROLL 4
 #endif
@@ -163,7 +167,6 @@ constexpr int Q_WORDS = 2 * Q_CAP;
 // — TB_WORDS slots in the warp's scratch on the warp path (edges with |T| > TRI_DEFER go to the CTA path), sized for
 // |T| on the CTA path (shared memory up to TSET_WORDS slots, this CTA's region of global memory beyond).  The d_a <=
 // 128 kernel marks the slots of T in its table of N(va) instead.
-enum { TRI_SET = 0 };
 constexpr int TB_WORDS = 64;
 constexpr int TRI_DEFER = 32;                // light edges with more triangles go to the CTA path
 
@@ -207,7 +210,7 @@ struct PaperArgs {
     long long coop;        // stream length above which an edge is cooperative for THIS call (>= COOP_L0 / COOP_G)
     int n;
     int dense;             // 1: n is small enough for an exact bitmap of N(va) in shared memory (classes L0 + G1 only)
-    uint32_t* gtables;     // class-X tables in global memory, gslots per CTA
+    uint32_t* gtables;     // class-X tables in global memory: gslots keys + gslots slot counters per CTA
     uint32_t gslots;
     uint32_t* ghash;       // last-resort match hashes in global memory: 2*ghash_cap words per CTA of a group kernel
     uint32_t ghash_cap;
@@ -218,13 +221,12 @@ struct PaperArgs {
 
 __device__ __forceinline__ uint32_t hash_slot(uint32_t key, int shift) { return (key * 2654435761u) >> shift; }
 
-// slot of `key` in the table, or -1.  A table in GLOBAL memory is filled with L2 atomics by other warps of the
-// CTA, so it is read with ld.global.cg (L2) — an L1 line fetched during the build phase may be stale.
-template <bool GLOBAL>
+// slot of `key` in the class-X table, or -1.  The table lives in global memory and is filled with L2 atomics by
+// other warps of the CTA, so it is read with ld.global.cg (L2) — an L1 line fetched during the build phase may be stale.
 __device__ __forceinline__ int probe_slot(const uint32_t* tab, uint32_t mask, int shift, uint32_t key, uint32_t& val) {
     uint32_t h = hash_slot(key, shift);
     while (true) {
-        const uint32_t v = GLOBAL ? __ldcg(tab + h) : tab[h];
+        const uint32_t v = __ldcg(tab + h);
         if (v == EMPTY) return -1;
         if ((v & KEYMASK) == key) { val = v; return (int)h; }
         h = (h + 1) & mask;
@@ -232,12 +234,11 @@ __device__ __forceinline__ int probe_slot(const uint32_t* tab, uint32_t mask, in
 }
 
 // insert key with `tag`, or OR the tag into an existing entry; returns true if the key was already present
-template <bool GLOBAL>
 __device__ __forceinline__ bool insert_or_tag(uint32_t* tab, uint32_t mask, int shift, uint32_t key, uint32_t tag) {
     uint32_t h = hash_slot(key, shift);
     const uint32_t val = key | (tag << 30);
     while (true) {
-        uint32_t v = GLOBAL ? __ldcg(tab + h) : tab[h];
+        uint32_t v = __ldcg(tab + h);
         if (v == EMPTY) {
             v = atomicCAS(&tab[h], EMPTY, val);
             if (v == EMPTY) return false;
@@ -271,25 +272,6 @@ __device__ __forceinline__ double paper_value(int d1, int d2, int tri, int sq1, 
 // planning kernels: S_v, per-edge class/bucket, bucket offsets, order
 // ------------------------------------------------------------------------------------------------------------
 // S_v = sum of the degrees of v's neighbours (the two row offsets of a neighbour share a sector).
-#ifdef DCR_NODE_S_WARP      // (tuning build: the round-1 kernel, one warp per vertex)
-__global__ void __launch_bounds__(256) node_s_kernel(const int32_t* __restrict__ rowptr, const int32_t* __restrict__ colidx,
-                                                     int n, int64_t* __restrict__ node_s) {
-    const int lane = threadIdx.x & 31;
-    for (int q = threadIdx.x >> 5; q < 32; q += 8) {
-        const int v = blockIdx.x * 32 + q;
-        if (v >= n) return;
-        const int b = rowptr[v], e = rowptr[v + 1];
-        int64_t s = 0;
-        for (int p = b + lane; p < e; p += 32) {
-            const int k = colidx[p];
-            s += rowptr[k + 1] - rowptr[k];
-        }
-#pragma unroll
-        for (int o = 16; o; o >>= 1) s += __shfl_xor_sync(FULL, s, o);
-        if (lane == 0) node_s[v] = s;
-    }
-}
-#else
 // 32 vertices per 256-thread CTA.  Rows of up to 64 entries: eight lanes per vertex (the average degree of the benchmark
 // graphs is 14-76: a warp per vertex leaves most lanes idle); rows of up to 2048 entries: one warp; longer rows (hubs: a
 // single warp would walk 6893 entries for 100 us after the rest of the kernel is done): the whole CTA.
@@ -347,8 +329,6 @@ __global__ void __launch_bounds__(256) node_s_kernel(const int32_t* __restrict__
         }
     }
 }
-
-#endif
 
 constexpr int BUCKET_TRIVIAL = 255, BUCKET_SPLIT = 254;
 
@@ -578,7 +558,7 @@ __global__ void __launch_bounds__(256) order_kernel(PaperArgs a) {
     a.ova[pos] = (uint32_t)r.va;
 }
 
-// where a class kernel finds its work: a range of `order` (classes) or the overflow list
+// where a class kernel finds its work: the class's range of `order`
 struct WorkSource { const uint32_t* order; unsigned int count; unsigned int* next; };
 __device__ __forceinline__ WorkSource work_source(const PaperArgs& a, int cls) {
     WorkSource w;
@@ -588,31 +568,17 @@ __device__ __forceinline__ WorkSource work_source(const PaperArgs& a, int cls) {
     return w;
 }
 
-// Slot counters: 16 bit per slot packed in 32-bit words for the shared-memory tables (a count is at most the number
-// of streamed lists, and classes 0-2 cap it far below 65536 only through d_b — see the saturation note in the
-// kernel), 32 bit per slot for the global-memory tables.
-template <bool GLOBAL>
-__device__ __forceinline__ void slot_count_add(uint32_t* cnt, int h) {
-    if (GLOBAL) atomicAdd(&cnt[h], 1u);
-    else atomicAdd(&cnt[h >> 1], (h & 1) ? 0x10000u : 1u);
-}
-template <bool GLOBAL>
-__device__ __forceinline__ uint32_t slot_count_get(const uint32_t* cnt, uint32_t h) {
-    if (GLOBAL) return __ldcg(cnt + h);
-    return (cnt[h >> 1] >> ((h & 1) * 16)) & 0xffffu;
-}
-
 // The flat stream: `pre` = exclusive prefix sums of the list lengths (pre[l+1]-pre[l] = length of list l), `beg` =
 // first CSR slot of each list, `lcnt` = per-list match counters, all in shared memory.  This warp handles the flat
 // elements [f_begin, f_end) in windows of 32*UNROLL; lane f%32 takes element f.  `lw` = a list index with
 // pre[lw] <= f_begin.  Windows that lie inside one list (most elements belong to long lists) take a fast path with
 // no per-element owner search.  An element first meets the bitmap filter `bm`; only if its bit is set the exact
 // probe runs.  A match (key present with tag 1, and not vb itself — the table holds all of N(va)) bumps the list's
-// counter and the matched key's slot counter.
-template <bool GLOBAL>
+// counter and the matched key's 32-bit slot counter `cnt[h]`.
 __device__ __forceinline__ void flat_scan(const int32_t* __restrict__ colidx, const uint32_t* tab, uint32_t* cnt,
-                                          uint32_t mask, int shift, const uint32_t* bm, uint32_t bmask, const int* pre,
+                                          uint32_t mask, int shift, const uint32_t* bm, const int* pre,
                                           const int* beg, int* lcnt, int lw, int f_begin, int f_end, int lane, int vb) {
+    constexpr uint32_t bmask = (uint32_t)GLOBAL_BITS - 1u;
     for (int F = f_begin; F < f_end; F += 32 * UNROLL) {
         while (pre[lw + 1] <= F) ++lw;                       // warp-uniform
         const int win = min(32 * UNROLL, f_end - F);
@@ -646,10 +612,10 @@ __device__ __forceinline__ void flat_scan(const int32_t* __restrict__ colidx, co
             const uint32_t kk = (uint32_t)k[u];
             if (k[u] >= 0 && k[u] != vb && ((bm[(kk & bmask) >> 5] >> (kk & 31u)) & 1u)) {
                 uint32_t v;
-                const int h = probe_slot<GLOBAL>(tab, mask, shift, kk, v);
+                const int h = probe_slot(tab, mask, shift, kk, v);
                 if (h >= 0 && (v >> 30) == 1u) {
                     atomicAdd(&lcnt[lu[u]], 1);
-                    slot_count_add<GLOBAL>(cnt, h);
+                    atomicAdd(&cnt[h], 1u);
                 }
             }
         }
@@ -657,46 +623,35 @@ __device__ __forceinline__ void flat_scan(const int32_t* __restrict__ colidx, co
 }
 
 // (begin, length) of the neighbour list of head m if m is a PURE neighbour of vb (not va, not in the table), else (0,0)
-template <bool GLOBAL>
 __device__ __forceinline__ void pure_head(const PaperArgs& a, const uint32_t* tab, uint32_t mask, int shift, int m,
                                           int va, int& b, int& d) {
     b = 0;
     d = 0;
     uint32_t v;
-    if (m != va && probe_slot<GLOBAL>(tab, mask, shift, (uint32_t)m, v) < 0) {
+    if (m != va && probe_slot(tab, mask, shift, (uint32_t)m, v) < 0) {
         b = a.rowptr[m];
         d = a.rowptr[m + 1] - b;
     }
 }
 
-// CTA team: up to HEADS = heads_per_thread*THREADS heads per round; the CTA-wide flat stream is cut into equal contiguous ranges,
+// CTA team: BIG_THREADS heads per round, one per thread; the CTA-wide flat stream is cut into equal contiguous ranges,
 // one per warp, so every warp streams the same number of elements whatever the list-length distribution (a hub's
-// list next to twenty short ones does not serialise).  `cs` = pre[HEADS+1] | beg[HEADS] | cnt[HEADS].
-template <int THREADS, bool GLOBAL>
+// list next to twenty short ones does not serialise).  `cs` = pre[BIG_THREADS+1] | beg[BIG_THREADS] | cnt[BIG_THREADS].
 __device__ __forceinline__ void scan_cta(const PaperArgs& a, const uint32_t* tab, uint32_t* cnt, uint32_t mask, int shift,
-                                         const uint32_t* bm, uint32_t bmask, int list_begin, int list_len, int va,
-                                         int vb, int* cs, int* s_warp_tot, int& sq, int& gmax) {
-    constexpr int HPT = heads_per_thread(THREADS);   // heads per thread
-    constexpr int HEADS = HPT * THREADS;
-    constexpr int NW = THREADS / 32;
+                                         const uint32_t* bm, int list_begin, int list_len, int va, int vb, int* cs,
+                                         int* s_warp_tot, int& sq, int& gmax) {
+    constexpr int NW = BIG_THREADS / 32;
     const int tid = threadIdx.x, lane = tid & 31, warp = tid >> 5;
-    int* pre = cs;                 // [HEADS + 1]
-    int* beg = cs + HEADS + 1;     // [HEADS]
-    int* lcnt = beg + HEADS;       // [HEADS]
-    for (int h0 = 0; h0 < list_len; h0 += HEADS) {
-        const int nh = min(HEADS, list_len - h0);
-        int deg[HPT], run = 0;
-#pragma unroll
-        for (int q = 0; q < HPT; ++q) {
-            const int t = tid * HPT + q;
-            int b = 0, d = 0;
-            if (t < nh) pure_head<GLOBAL>(a, tab, mask, shift, a.colidx[list_begin + h0 + t], va, b, d);
-            beg[t] = b;
-            lcnt[t] = 0;
-            deg[q] = d;
-            run += d;
-        }
-        int inc = run;                            // exclusive scan of `run` over the CTA
+    int* pre = cs;                      // [BIG_THREADS + 1]
+    int* beg = cs + BIG_THREADS + 1;    // [BIG_THREADS]
+    int* lcnt = beg + BIG_THREADS;      // [BIG_THREADS]
+    for (int h0 = 0; h0 < list_len; h0 += BIG_THREADS) {
+        const int nh = min(BIG_THREADS, list_len - h0);
+        int b = 0, d = 0;
+        if (tid < nh) pure_head(a, tab, mask, shift, a.colidx[list_begin + h0 + tid], va, b, d);
+        beg[tid] = b;
+        lcnt[tid] = 0;
+        int inc = d;                              // exclusive scan of `d` over the CTA
 #pragma unroll
         for (int o = 1; o < 32; o <<= 1) {
             const int up = __shfl_up_sync(FULL, inc, o);
@@ -704,30 +659,27 @@ __device__ __forceinline__ void scan_cta(const PaperArgs& a, const uint32_t* tab
         }
         if (lane == 31) s_warp_tot[warp] = inc;
         __syncthreads();
-        int off = inc - run;
+        int off = inc - d;
         for (int w = 0; w < warp; ++w) off += s_warp_tot[w];
-#pragma unroll
-        for (int q = 0; q < HPT; ++q) {
-            pre[tid * HPT + q] = off;
-            off += deg[q];
-        }
-        if (tid == THREADS - 1) pre[HEADS] = off;
+        pre[tid] = off;
+        off += d;
+        if (tid == BIG_THREADS - 1) pre[BIG_THREADS] = off;
         __syncthreads();
-        const int total = pre[HEADS];
+        const int total = pre[BIG_THREADS];
         if (total > 0) {
             const int per_warp = ((total + NW * 32 - 1) / (NW * 32)) * 32;
             const int f_begin = warp * per_warp, f_end = min(total, f_begin + per_warp);
             if (f_begin < f_end) {
-                int lo = 0, hi = HEADS;            // first l with pre[l+1] > f_begin (warp-uniform search)
+                int lo = 0, hi = BIG_THREADS;      // first l with pre[l+1] > f_begin (warp-uniform search)
                 while (lo < hi) {
                     const int mid = (lo + hi) >> 1;
                     if (pre[mid + 1] <= f_begin) lo = mid + 1; else hi = mid;
                 }
-                flat_scan<GLOBAL>(a.colidx, tab, cnt, mask, shift, bm, bmask, pre, beg, lcnt, lo, f_begin, f_end, lane, vb);
+                flat_scan(a.colidx, tab, cnt, mask, shift, bm, pre, beg, lcnt, lo, f_begin, f_end, lane, vb);
             }
             __syncthreads();
-            for (int t = tid; t < nh; t += THREADS) {
-                const int c = lcnt[t];
+            if (tid < nh) {
+                const int c = lcnt[tid];
                 sq += c > 0;
                 gmax = max(gmax, c);
             }
@@ -736,38 +688,26 @@ __device__ __forceinline__ void scan_cta(const PaperArgs& a, const uint32_t* tab
     }
 }
 
-// CTA-team kernel (heavy edges, global-table edges, overflow list): the CTA is the team of one edge at a time.
-template <int TEAM, int MAX_SLOTS, bool GLOBAL_TABLE>
-__global__ void __launch_bounds__(TEAM, 1)
+// CTA-team kernel (class X of hashed mode: d_a > 16384, beyond the shared-memory tables): the CTA is the team of one
+// edge at a time.  The table of N(va) (gslots keys, tag in bits 30-31) and its 32-bit slot counters (gslots more words)
+// live in this CTA's region of `gtables` in global memory (L2); the bitmap filter and the stream state in shared memory.
+__global__ void __launch_bounds__(BIG_THREADS, 1)
 paper_edge_kernel(PaperArgs a, int cls) {
-    constexpr int NWARPS = TEAM / 32;
-    constexpr int CTA_STREAM = 3 * heads_per_thread(TEAM) * TEAM + 8;
+    constexpr int NWARPS = BIG_THREADS / 32;
+    constexpr uint32_t bmask = (uint32_t)GLOBAL_BITS - 1u;
     extern __shared__ uint32_t smem_dyn[];
     __shared__ unsigned int s_idx;
     __shared__ int s_warp_tot[NWARPS];
     __shared__ int s_red[5];  // tri, sq(lists), g(lists), sq(slots), g(slots)
 
-    const int lane = threadIdx.x & 31;
-    constexpr int team_threads = TEAM;
-    const int team_tid = (int)threadIdx.x;
-    // shared-memory carve-up: [stream state][bitmap filter][table keys][slot counters]
-    constexpr int FBITS = filter_bits(TEAM, GLOBAL_TABLE);
-    constexpr uint32_t bmask = (uint32_t)FBITS - 1u;
+    const int tid = threadIdx.x, lane = tid & 31;
+    // shared-memory carve-up: [stream state][bitmap filter]
     int* st = (int*)smem_dyn;
-    uint32_t* bm = smem_dyn + CTA_STREAM;
-    uint32_t* sm_tab = smem_dyn + CTA_STREAM + FBITS / 32;
-    uint32_t* tab;
-    uint32_t* cnt;
-    if (GLOBAL_TABLE) {
-        tab = a.gtables + (size_t)blockIdx.x * a.gslots * 2;
-        cnt = tab + a.gslots;
-    } else {
-        tab = sm_tab;
-        cnt = sm_tab + MAX_SLOTS;
-    }
+    uint32_t* bm = smem_dyn + BIG_STREAM_INTS;
+    uint32_t* tab = a.gtables + (size_t)blockIdx.x * a.gslots * 2;
+    uint32_t* cnt = tab + a.gslots;
     const WorkSource ws = work_source(a, cls);
     const unsigned int cnum = ws.count;
-    const uint32_t max_slots = GLOBAL_TABLE ? a.gslots : (uint32_t)MAX_SLOTS;
     // edges per work-stealing step: a run of one va, usually — but never so long that the CTAs run out of steps
     const unsigned int GRAB = min(16u, max(1u, cnum / (gridDim.x * 8u)));
 
@@ -794,18 +734,18 @@ paper_edge_kernel(PaperArgs a, int cls) {
 
             if (va != cur_va) {
                 // table of N(va), every key with tag 1: power of two >= 8*d_a (load factor <= 1/8 keeps probe
-                // chains short and uniform across the lanes of a warp), capped by the class's table
-                const int lg = min(32 - __clz(max(8 * da, 64) - 1), 31 - __clz(max_slots));
+                // chains short and uniform across the lanes of a warp), capped by the CTA's region
+                const int lg = min(32 - __clz(max(8 * da, 64) - 1), 31 - __clz(a.gslots));
                 slots = 1u << lg;
                 mask = slots - 1;
                 shift = 32 - lg;
-                for (uint32_t s = team_tid; s < slots; s += team_threads) tab[s] = EMPTY;
-                for (uint32_t s = team_tid; s < (GLOBAL_TABLE ? slots : slots / 2); s += team_threads) cnt[s] = 0u;
-                for (uint32_t s = team_tid; s < (uint32_t)FBITS / 32; s += team_threads) bm[s] = 0u;
+                for (uint32_t s = tid; s < slots; s += BIG_THREADS) tab[s] = EMPTY;
+                for (uint32_t s = tid; s < slots; s += BIG_THREADS) cnt[s] = 0u;
+                for (uint32_t s = tid; s < (uint32_t)GLOBAL_BITS / 32; s += BIG_THREADS) bm[s] = 0u;
                 __syncthreads();
-                for (int p = team_tid; p < da; p += team_threads) {
+                for (int p = tid; p < da; p += BIG_THREADS) {
                     const uint32_t k = (uint32_t)a.colidx[sa + p];
-                    insert_or_tag<GLOBAL_TABLE>(tab, mask, shift, k, 1u);
+                    insert_or_tag(tab, mask, shift, k, 1u);
                     atomicOr(&bm[(k & bmask) >> 5], 1u << (k & 31u));
                 }
                 __syncthreads();
@@ -813,10 +753,10 @@ paper_edge_kernel(PaperArgs a, int cls) {
             }
             // common neighbours: heads of N(vb) found in the table get bit 31 (tag 3: never a match, never a head)
             int tri = 0;
-            for (int p = team_tid; p < db; p += team_threads) {
+            for (int p = tid; p < db; p += BIG_THREADS) {
                 const int m = a.colidx[sb + p];
                 uint32_t v;
-                const int h = (m == va) ? -1 : probe_slot<GLOBAL_TABLE>(tab, mask, shift, (uint32_t)m, v);
+                const int h = (m == va) ? -1 : probe_slot(tab, mask, shift, (uint32_t)m, v);
                 if (h >= 0) {
                     atomicOr(&tab[h], 2u << 30);
                     ++tri;
@@ -828,7 +768,7 @@ paper_edge_kernel(PaperArgs a, int cls) {
 
             // the scan: lists of the pure neighbours of vb, matches against the pure neighbours of va
             int sqL = 0, gL = 0, sqS = 0, gS = 0;
-            scan_cta<TEAM, GLOBAL_TABLE>(a, tab, cnt, mask, shift, bm, bmask, sb, db, va, vb, st, s_warp_tot, sqL, gL);
+            scan_cta(a, tab, cnt, mask, shift, bm, sb, db, va, vb, st, s_warp_tot, sqL, gL);
             sqL = warp_sum(sqL);
             gL = warp_max(gL);
             if (lane == 0 && sqL) { atomicAdd(&s_red[1], sqL); atomicMax(&s_red[2], gL); }
@@ -838,17 +778,16 @@ paper_edge_kernel(PaperArgs a, int cls) {
             // nothing).  Walks N(va) (d_a probes) instead of sweeping the table and zeroes the counters it reads,
             // so the table is clean for the next edge of the same va.
             if (sqL > 0) {
-                for (int p = team_tid; p < da; p += team_threads) {
+                for (int p = tid; p < da; p += BIG_THREADS) {
                     const int k = a.colidx[sa + p];
                     uint32_t v;
-                    const int h = probe_slot<GLOBAL_TABLE>(tab, mask, shift, (uint32_t)k, v);
+                    const int h = probe_slot(tab, mask, shift, (uint32_t)k, v);
                     if (h >= 0 && (v >> 30) == 1u) {
-                        const int c = (int)slot_count_get<GLOBAL_TABLE>(cnt, (uint32_t)h);
+                        const int c = (int)__ldcg(cnt + (uint32_t)h);
                         if (c > 0) {
                             ++sqS;
                             gS = max(gS, c);
-                            if (GLOBAL_TABLE) cnt[h] = 0u;
-                            else atomicAnd(&cnt[h >> 1], (h & 1) ? 0x0000ffffu : 0xffff0000u);
+                            cnt[h] = 0u;
                         }
                     }
                 }
@@ -858,7 +797,7 @@ paper_edge_kernel(PaperArgs a, int cls) {
                 __syncthreads();
                 sqS = s_red[3]; gS = s_red[4];
             }
-            if (team_tid == 0) {
+            if (tid == 0) {
                 const int sq_i = swapped ? sqL : sqS, sq_j = swapped ? sqS : sqL;
                 const int gamma = (sqL > 0 && sqS > 0) ? max(gL, gS) : 0;
                 a.out_tri[t] = tri;
@@ -868,10 +807,10 @@ paper_edge_kernel(PaperArgs a, int cls) {
             }
             // undo the common-neighbour marks so the table is N(va) with tag 1 again
             if (tri > 0) {
-                for (int p = team_tid; p < db; p += team_threads) {
+                for (int p = tid; p < db; p += BIG_THREADS) {
                     const int m = a.colidx[sb + p];
                     uint32_t v;
-                    const int h = (m == va) ? -1 : probe_slot<GLOBAL_TABLE>(tab, mask, shift, (uint32_t)m, v);
+                    const int h = (m == va) ? -1 : probe_slot(tab, mask, shift, (uint32_t)m, v);
                     if (h >= 0) atomicAnd(&tab[h], 0x7fffffffu);
                 }
             }
@@ -907,10 +846,10 @@ __device__ __forceinline__ bool bitmap_test(const uint32_t* bm, uint32_t bmask, 
     return (bm[(k & bmask) >> 5] >> (k & 31u)) & 1u;
 }
 
-// Table geometry for a tested endpoint of degree d_a: power of two >= FILL*d_a slots (>= 64), key-only.
-template <int MAX_SLOTS, int FILL>
+// Table geometry for a tested endpoint of degree d_a: power of two >= 2*d_a slots (>= 64), key-only.
+template <int MAX_SLOTS>
 __device__ __forceinline__ void ro_geometry(int da, uint32_t& mask, int& shift) {
-    const int lg = min(32 - __clz(max(FILL * da, 64) - 1), ilog2_c(MAX_SLOTS));
+    const int lg = min(32 - __clz(max(2 * da, 64) - 1), ilog2_c(MAX_SLOTS));
     mask = (1u << lg) - 1u;
     shift = 32 - lg;
 }
@@ -982,7 +921,7 @@ struct MatchHash {
 // Everything a warp needs to test streamed elements of one edge (va tested, vb streamed) against the CTA-level or
 // warp-level structures of the group kernels: membership in N(va), the structure that answers "k in T", the match
 // hash, the warp's candidate queue and the per-list match counters the queue entries point into.
-template <bool DENSE, int TM>
+template <bool DENSE>
 struct EdgeCtx {
     const int32_t* __restrict__ colidx;
     Member<DENSE> mem;
@@ -1005,7 +944,6 @@ struct EdgeCtx {
     int* lcnt;               // per-list match counters
     int va, vb, sb, db;
     bool ovf;
-    __device__ __forceinline__ void set_ovf(const EdgeCtx& o) { ovf = o.ovf; }
     __device__ __forceinline__ bool in_triangle(uint32_t kk) const {
         uint32_t h = ((kk * 2654435761u) >> tb_shift) & tb_mask;
         while (true) {
@@ -1032,15 +970,6 @@ __device__ __forceinline__ void tri_set_insert(uint32_t* ts, uint32_t mask, int 
         if (v == EMPTY || v == kk) return;
         h = (h + 1) & mask;
     }
-}
-
-// the u-th of N registers (u is not a compile-time constant: a select chain instead of local memory)
-template <int N>
-__device__ __forceinline__ int pick(const int (&v)[N], int u) {
-    int r = v[0];
-#pragma unroll
-    for (int q = 1; q < N; ++q) r = (u == q) ? v[q] : r;
-    return r;
 }
 
 // Append this window's candidates (bit u of hm: element k[u] of this lane passed the filter) to the warp's queue: one
@@ -1071,10 +1000,9 @@ __device__ __forceinline__ void q_flush(Ctx& cx, int lane) {
 }
 
 // The filter of one window: bit u of the result says that element k[u] of this lane may be a match.  The filter word of
-// element u is rotated so that the element's bit lands on bit u (one funnel shift) and merged with one and-or; with
-// VB_TEST the streamed endpoint itself — it sits in every streamed list and in N(va) — is dropped here, otherwise
-// handle() drops it.
-template <bool VB_TEST, class Ctx, int N>
+// element u is rotated so that the element's bit lands on bit u (one funnel shift) and merged with one and-or; the
+// streamed endpoint itself — it sits in every streamed list and in N(va) — is dropped here.
+template <class Ctx, int N>
 __device__ __forceinline__ uint32_t filter_window(const Ctx& cx, const int (&k)[N]) {
     uint32_t w[N];
 #pragma unroll
@@ -1082,18 +1010,16 @@ __device__ __forceinline__ uint32_t filter_window(const Ctx& cx, const int (&k)[
     uint32_t hm = 0;
 #pragma unroll
     for (int u = 0; u < N; ++u) hm |= __funnelshift_r(w[u], w[u], (uint32_t)k[u] - (uint32_t)u) & (1u << u);
-    if (VB_TEST) {
 #pragma unroll
-        for (int u = 0; u < N; ++u) if (k[u] == cx.vb) hm &= ~(1u << u);
-    }
+    for (int u = 0; u < N; ++u) if (k[u] == cx.vb) hm &= ~(1u << u);
     return hm;
 }
 
 // `len` consecutive entries of ONE neighbour list, streamed by the whole warp (p already includes the lane offset);
 // candidates go to the queue with `owner` as their list.  Full windows carry no bounds test at all; lanes past the
 // end of the last window test va, which is never a member of N(va).
-template <bool VB_TEST, class Ctx>
-__device__ __forceinline__ void stream_list_t(Ctx& cx, const int32_t* __restrict__ p, int len, int owner, int pad, int lane) {
+template <class Ctx>
+__device__ __forceinline__ void stream_list(Ctx& cx, const int32_t* __restrict__ p, int len, int owner, int lane) {
     int own[UNROLL];
 #pragma unroll
     for (int u = 0; u < UNROLL; ++u) own[u] = owner;
@@ -1102,7 +1028,7 @@ __device__ __forceinline__ void stream_list_t(Ctx& cx, const int32_t* __restrict
         int k[UNROLL];
 #pragma unroll
         for (int u = 0; u < UNROLL; ++u) k[u] = __ldg(p + F + 32 * u);
-        const uint32_t hm = filter_window<VB_TEST>(cx, k);
+        const uint32_t hm = filter_window(cx, k);
         if (__any_sync(FULL, hm != 0u)) {
             q_push(cx, hm, k, own, lane);
             if (cx.qn >= Q_FLUSH) q_flush(cx, lane);
@@ -1112,26 +1038,22 @@ __device__ __forceinline__ void stream_list_t(Ctx& cx, const int32_t* __restrict
     if (rem) {
         int k[UNROLL];
 #pragma unroll
-        for (int u = 0; u < UNROLL; ++u) k[u] = (32 * u + lane < rem) ? __ldg(p + full + 32 * u) : pad;
-        const uint32_t hm = filter_window<VB_TEST>(cx, k);
+        for (int u = 0; u < UNROLL; ++u) k[u] = (32 * u + lane < rem) ? __ldg(p + full + 32 * u) : cx.va;
+        const uint32_t hm = filter_window(cx, k);
         if (__any_sync(FULL, hm != 0u)) {
             q_push(cx, hm, k, own, lane);
             if (cx.qn >= Q_FLUSH) q_flush(cx, lane);
         }
     }
 }
-template <class Ctx>
-__device__ __forceinline__ void stream_list(Ctx& cx, const int32_t* __restrict__ p, int len, int owner, int lane) {
-    stream_list_t<true>(cx, p, len, owner, cx.va, lane);
-}
 // (out-of-line copies work on a register copy of the context: through the reference every store to shared memory
 //  would force the context's fields to be re-read from the caller's stack frame)
 template <class Ctx>
 __device__ __noinline__ void stream_list_call(Ctx& cx_ref, const int32_t* __restrict__ p, int len, int owner, int lane) {
     Ctx cx = cx_ref;
-    stream_list_t<true>(cx, p, len, owner, cx.va, lane);
+    stream_list(cx, p, len, owner, lane);
     cx_ref.qn = cx.qn;
-    cx_ref.set_ovf(cx);
+    cx_ref.ovf = cx.ovf;
 }
 
 // One chunk of 32 heads of N(vb) by one warp; lane l holds head l of the chunk: (mb, md) = (begin, length) of its
@@ -1142,7 +1064,7 @@ __device__ __noinline__ void stream_list_call(Ctx& cx_ref, const int32_t* __rest
 // go through the queue; the chunk ends with the queue drained and the per-list counters folded into the lane-partial
 // sq_b (#lists with a match) and g_b (largest per-list count).
 template <class Ctx>
-__device__ __forceinline__ void warp_chunk_impl(Ctx& cx, int mb, int md, int* st, int lane, int& sq_b, int& g_b) {
+__device__ __forceinline__ void warp_chunk(Ctx& cx, int mb, int md, int* st, int lane, int& sq_b, int& g_b) {
     const int32_t* __restrict__ colidx = cx.colidx;
     const uint32_t lm0 = __ballot_sync(FULL, md >= LONG_LIST);
     const bool shortl = md > 1 && md < LONG_LIST;               // (a list that holds only vb cannot match)
@@ -1196,7 +1118,7 @@ __device__ __forceinline__ void warp_chunk_impl(Ctx& cx, int mb, int md, int* st
                 const int f = Fu + lane;
                 k[u] = f < total ? __ldg(colidx + bs + f) : cx.va;
             }
-            const uint32_t hm = filter_window<true>(cx, k);
+            const uint32_t hm = filter_window(cx, k);
             if (__any_sync(FULL, hm != 0u)) {
                 q_push(cx, hm, k, own, lane);
                 if (cx.qn >= Q_FLUSH) q_flush(cx, lane);
@@ -1210,34 +1132,30 @@ __device__ __forceinline__ void warp_chunk_impl(Ctx& cx, int mb, int md, int* st
     __syncwarp();
 }
 
-// the d_a <= 128 kernel inlines the chunk; the group kernels — several callers, much more code around — share ONE copy
-template <class Ctx>
-__device__ __forceinline__ void warp_chunk(Ctx& cx, int mb, int md, int* st, int lane, int& sq_b, int& g_b) {
-    warp_chunk_impl(cx, mb, md, st, lane, sq_b, g_b);
-}
+// the warp paths inline the chunk; cta_edge calls this out-of-line copy
 template <class Ctx>
 __device__ __noinline__ void warp_chunk_call(Ctx& cx_ref, int mb, int md, int* st, int lane, int& sq_b_ref, int& g_b_ref) {
     Ctx cx = cx_ref;
     int sq_b = sq_b_ref, g_b = g_b_ref;
-    warp_chunk_impl(cx, mb, md, st, lane, sq_b, g_b);
+    warp_chunk(cx, mb, md, st, lane, sq_b, g_b);
     sq_b_ref = sq_b;
     g_b_ref = g_b;
     cx_ref.qn = cx.qn;
-    cx_ref.set_ovf(cx);
+    cx_ref.ovf = cx.ovf;
 }
 
 // One edge by one warp over the CTA-level membership structure (group kernels).  `st` = the warp's scratch, `tb` =
-// its exact triangle set (TSLOTS words), `mh` = its match hash (2*CAP words, all zero on entry and on exit), `q` = its
+// its exact triangle set (TB_WORDS words), `mh` = its match hash (2*CAP words, all zero on entry and on exit), `q` = its
 // candidate queue.  Writes the four integer fields of local edge t and returns true, or returns false when the match
 // hash filled up or the edge has too many triangles for the warp's set (nothing written; the hash is clean again).
-template <int CAP, int TSLOTS, bool DENSE, bool CAN_DEFER>
+template <int CAP, bool DENSE>
 __device__ __forceinline__ bool warp_edge(const PaperArgs& a, const Member<DENSE>& mem, uint32_t t, int va, int* st,
                                           uint32_t* tb, uint32_t* mh, uint32_t* q, int lane) {
     const int64_t e = a.e_first + (int64_t)t * a.e_stride;
     const int i = a.esrc[e], j = a.edst[e];
     const bool swapped = (va == j);                      // stream i's side, test j
-    EdgeCtx<DENSE, TRI_SET> cx;
-    cx.colidx = a.colidx; cx.mem = mem; cx.tb = tb; cx.tb_mask = TSLOTS - 1; cx.tb_shift = 32 - ilog2_c(TSLOTS);
+    EdgeCtx<DENSE> cx;
+    cx.colidx = a.colidx; cx.mem = mem; cx.tb = tb; cx.tb_mask = TB_WORDS - 1; cx.tb_shift = 32 - ilog2_c(TB_WORDS);
     cx.tb_global = false; cx.hash.init(mh, st + WS_NDIST, CAP);
     cx.q = q; cx.qn = 0; cx.lcnt = st + WS_LCNT;
     cx.va = va;
@@ -1256,15 +1174,15 @@ __device__ __forceinline__ bool warp_edge(const PaperArgs& a, const Member<DENSE
         if (c < 32) mbits |= in ? (1u << c) : 0u;
     }
     tri = __reduce_add_sync(FULL, tri);
-    // the warp's exact set of T holds TSLOTS/2 keys: a richer edge goes to the CTA path
-    if (CAN_DEFER && tri > TRI_DEFER) return false;
+    // the warp's exact set of T holds TB_WORDS/2 keys: a richer edge goes to the CTA path
+    if (tri > TRI_DEFER) return false;
     if (tri > 0) {
-        for (int p = lane; p < TSLOTS; p += 32) tb[p] = EMPTY;
+        for (int p = lane; p < TB_WORDS; p += 32) tb[p] = EMPTY;
         __syncwarp();
         for (int p = lane, c = 0; p < cx.db; p += 32, ++c) {
             if (c < 32 && !((mbits >> c) & 1u)) continue;
             const uint32_t m = (uint32_t)a.colidx[cx.sb + p];
-            if (c < 32 || ((int)m != va && mem.has(m))) tri_set_insert(tb, TSLOTS - 1, 32 - ilog2_c(TSLOTS), m);
+            if (c < 32 || ((int)m != va && mem.has(m))) tri_set_insert(tb, TB_WORDS - 1, 32 - ilog2_c(TB_WORDS), m);
         }
     } else if (lane == 0) {
         tb[0] = EMPTY;                                   // an empty set is recognised by its first probe ...
@@ -1323,8 +1241,6 @@ struct L0Ctx {
     int qn;
     int* lcnt;
     int va, vb, sb, db;
-    static constexpr int Q_ENTRY_WORDS = 2;
-    __device__ __forceinline__ void set_ovf(const L0Ctx&) {}
     __device__ __forceinline__ void q_store(int pos, uint32_t k, uint32_t list) { ((uint2*)q)[pos] = make_uint2(k, list); }
     __device__ __forceinline__ void q_load(int pos, uint32_t& k, uint32_t& list) const {
         const uint2 v = ((const uint2*)q)[pos];
@@ -1450,7 +1366,7 @@ __global__ void __launch_bounds__(L0_WARPS * 32, L0_CTAS_PER_SM) paper_light_war
             const int va = (int)ova[q];
             if (va != cur_va) {
                 const int sa = a.rowptr[va], da = a.rowptr[va + 1] - sa;
-                ro_geometry<L0_SLOTS, 2>(da, cx.mask, cx.shift);
+                ro_geometry<L0_SLOTS>(da, cx.mask, cx.shift);
                 for (uint32_t s = lane; s <= cx.mask; s += 32) tab[s] = EMPTY;
                 for (int s = lane; s < L0_BITS / 32; s += 32) bm[s] = 0u;
                 __syncwarp();
@@ -1503,7 +1419,7 @@ __device__ __noinline__ void cta_edge(const PaperArgs& a, const Member<DENSE>& m
     const int64_t e = a.e_first + (int64_t)t * a.e_stride;
     const int i = a.esrc[e], j = a.edst[e];
     const bool swapped = (va == j);
-    EdgeCtx<DENSE, TRI_SET> cx;
+    EdgeCtx<DENSE> cx;
     cx.colidx = a.colidx; cx.mem = mem;
     cx.hash.init(hash_words, se ? &se->n_distinct : s_acc + 4, hash_cap);
     cx.q = q_all + warp * (Q_CAP * cx.Q_ENTRY_WORDS); cx.qn = 0; cx.lcnt = st + WS_LCNT;
@@ -1700,7 +1616,7 @@ __device__ __noinline__ void build_member(const PaperArgs& a, Member<DENSE>& mem
             }
         }
     } else {
-        ro_geometry<MAX_SLOTS, 2>(da, mem.mask, mem.shift);
+        ro_geometry<MAX_SLOTS>(da, mem.mask, mem.shift);
 #pragma unroll 1
         for (uint32_t s = tid; s <= mem.mask; s += THREADS) tab[s] = EMPTY;
 #pragma unroll 1
@@ -1834,7 +1750,7 @@ __global__ void __launch_bounds__(NWARPS * 32, CTAS_PER_SM) paper_group_kernel(P
             my = __shfl_sync(FULL, my, 0);
             if ((int)my >= q_end) break;
             const uint32_t t = ord[my];
-            if (!warp_edge<CAP, TB_WORDS, DENSE, true>(a, mem, t, va, st, tb, mh, q_all + warp * QW, lane) && lane == 0)
+            if (!warp_edge<CAP, DENSE>(a, mem, t, va, st, tb, mh, q_all + warp * QW, lane) && lane == 0)
                 s_defer[atomicAdd(&s_ndefer, 1)] = t;     // too many triangles / distinct matches for one warp: CTA path
         }
         __syncthreads();                                  // every warp is done with the run
@@ -2009,9 +1925,8 @@ static int paper_pass(const int32_t* rowptr, const int32_t* colidx, int n, int m
     PaperAux& ax = g_aux[dev];
     std::lock_guard<std::mutex> guard(ax.mu);
     bool& attr_done = ax.attr_done;
-    constexpr int big_stream = 3 * heads_per_thread(BIG_THREADS) * BIG_THREADS + 8;
     const int dense_words = (n + 63) / 64 * 2;       // even: what follows the bitmaps in shared memory is 8-byte aligned
-    const int smem_x = (big_stream + GLOBAL_BITS / 32) * (int)sizeof(int);
+    const int smem_x = (BIG_STREAM_INTS + GLOBAL_BITS / 32) * (int)sizeof(int);
     constexpr int WARP_WORDS = TB_WORDS + WSTATE_INTS + Q_WORDS;     // per warp of a group kernel, beside its match hash
     constexpr int WARP_WORDS_D = TB_WORDS + WSTATE_INTS + Q_CAP;     // dense mode: one-word queue entries
     const int smem_l0 = L0_WARPS * (L0_BITS / 32 + L0_PER_WARP) * (int)sizeof(uint32_t);
@@ -2022,8 +1937,7 @@ static int paper_pass(const int32_t* rowptr, const int32_t* colidx, int n, int m
     auto* k_g2 = paper_group_kernel<G2_WARPS, G2_SLOTS, G2_BITS, G2_CAP, 1, false>;
     auto* k_gd = paper_group_kernel<GD_WARPS, 64, 32, GD_CAP, GD_CTAS_PER_SM, true>;
     if (!attr_done) {
-        DCR_CUDA(cudaFuncSetAttribute(paper_edge_kernel<BIG_THREADS, BIG_SLOTS, true>,
-                                      cudaFuncAttributeMaxDynamicSharedMemorySize, smem_x));
+        DCR_CUDA(cudaFuncSetAttribute(paper_edge_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, smem_x));
         DCR_CUDA(cudaFuncSetAttribute(paper_light_warp_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, smem_l0));
         DCR_CUDA(cudaFuncSetAttribute(k_g1, cudaFuncAttributeMaxDynamicSharedMemorySize, smem_g1));
         DCR_CUDA(cudaFuncSetAttribute(k_g2, cudaFuncAttributeMaxDynamicSharedMemorySize, smem_g2));
@@ -2056,7 +1970,7 @@ static int paper_pass(const int32_t* rowptr, const int32_t* colidx, int n, int m
 #endif
     } else {
         if (L.gslots) {
-            paper_edge_kernel<BIG_THREADS, BIG_SLOTS, true><<<L.g_ctas, BIG_THREADS, smem_x, aux[2]>>>(a, CL_X);
+            paper_edge_kernel<<<L.g_ctas, BIG_THREADS, smem_x, aux[2]>>>(a, CL_X);
             DCR_LAUNCH_CHECK();
         }
         k_g2<<<sms, G2_WARPS * 32, smem_g2, st>>>(a, CL_G2, 0);

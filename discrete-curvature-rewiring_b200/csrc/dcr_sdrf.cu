@@ -24,7 +24,7 @@
 
 namespace dcr {
 
-// Loop flavours (template parameter of the loop kernel; DCR_SDRF_MODE_* of dcr.h map onto them):
+// Loop flavours (template parameter of the loop kernel; loop_kernels() maps DCR_SDRF_MODE_* of dcr.h onto them):
 //   LOOP_BFC       sdrf_cuda_bfc, is_undirected=True   (rewiring/sdrf_cuda_bfc.py:14-93) — symmetric arena, maintained
 //                  supports, closed-form curvature and scoring (dcr_score.cuh)
 //   LOOP_DIRECTED  sdrf_cuda_bfc, is_undirected=False  (:47-49, :72-73, :87-88) — rows [0,n) hold the successors,
@@ -61,7 +61,6 @@ __device__ unsigned long long g_sdrf_phase[16];
 
 struct SdrfDev {
     int n;
-    int rows;             // n, or 2n for the directed loop (row n+v = predecessors of v)
     int ctype;            // classical loop: 0 = '1d', 1 = 'augmented', 2 = 'haantjes'
     int cap_total;        // arena slots
     int row_cap_max;      // capacity of the per-row scratch arrays
@@ -112,8 +111,6 @@ struct Reduce {     // shared-memory scratch for the block primitives
     double d[SDRF_WARPS];
     long long l[SDRF_WARPS];
     Best best;
-    double dsum;
-    long long lsum;
 };
 
 __device__ Best block_best(Best a, Reduce* r) {
@@ -155,23 +152,6 @@ __device__ void block_best2(Best& a, Best& b, Reduce* r, Reduce* r2) {
     __syncthreads();
 }
 
-__device__ long long block_sum_ll(long long v, Reduce* r) {
-    const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
-#pragma unroll
-    for (int o = 16; o; o >>= 1) v += __shfl_xor_sync(FULL, v, o);
-    if (lane == 0) r->l[warp] = v;
-    __syncthreads();
-    if (threadIdx.x == 0) {
-        long long s = 0;
-        for (int w = 0; w < SDRF_WARPS; ++w) s += r->l[w];
-        r->lsum = s;
-    }
-    __syncthreads();
-    long long out = r->lsum;
-    __syncthreads();
-    return out;
-}
-
 // exclusive prefix over threads (thread order) + total
 __device__ long long block_exscan_ll(long long v, long long* total, Reduce* r) {
     const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
@@ -191,28 +171,6 @@ __device__ long long block_exscan_ll(long long v, long long* total, Reduce* r) {
     __syncthreads();
     *total = tot;
     return off + inc - v;
-}
-
-__device__ double block_exscan_d(double v, double* total, Reduce* r) {
-    const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
-    double inc = v;
-#pragma unroll
-    for (int o = 1; o < 32; o <<= 1) {
-        double t = __shfl_up_sync(FULL, inc, o);
-        if (lane >= o) inc = __dadd_rn(inc, t);
-    }
-    double excl = __shfl_up_sync(FULL, inc, 1);   // exclusive within the warp without a subtraction
-    if (lane == 0) excl = 0.0;
-    if (lane == 31) r->d[warp] = inc;
-    __syncthreads();
-    double off = 0.0, tot = 0.0;
-    for (int w = 0; w < SDRF_WARPS; ++w) {
-        if (w < warp) off = __dadd_rn(off, r->d[w]);
-        tot = __dadd_rn(tot, r->d[w]);
-    }
-    __syncthreads();
-    *total = tot;
-    return __dadd_rn(off, excl);
 }
 
 // exclusive prefixes of a (count, fp64 sum) pair over the threads, plus both totals: one primitive, two barriers
@@ -260,23 +218,10 @@ struct LoopShared {
     int choice, k, l;
     int status, stop, can_add, do_remove;
     double below, above;      // normalised CDF just below / at the chosen candidate
-    int cnt_a, cnt_b;         // generic counters
-    int edit_pos, edit_ok;
+    int cnt_a;                // wlist fill of toggle_supports
+    int edit_pos;             // ord_erase: slot of the erased id
 };
 
-template <class T>
-__device__ void shift_right(T* a, int lo, int hi) {   // a[lo+1 .. hi] = a[lo .. hi-1]
-    for (int top = hi; top > lo; top -= SDRF_THREADS) {
-        const int base = max(lo, top - SDRF_THREADS);
-        const int idx = base + threadIdx.x;
-        T v{};
-        const bool on = idx < top;
-        if (on) v = a[idx];
-        __syncthreads();
-        if (on) a[idx + 1] = v;
-        __syncthreads();
-    }
-}
 template <class T>
 __device__ void shift_left(T* a, int lo, int hi) {    // a[lo-1 .. hi-2] = a[lo .. hi-1]
     for (int base = lo; base < hi; base += SDRF_THREADS) {
@@ -318,7 +263,7 @@ __device__ void shift_left3(const SdrfDev& S, int lo, int hi) {
 }
 
 // make room for one more entry in row v (relocate to the arena top with doubled capacity when full)
-__device__ bool row_reserve(const SdrfDev& S, int v, LoopShared* sh) {
+__device__ bool row_reserve(const SdrfDev& S, int v) {
     const int len = S.rlen[v], cap = S.rcap[v], start = S.rstart[v], self = S.selfl[v];
     __syncthreads();
     if (len + self < cap) return true;     // (the insertion-order row is `self` entries longer than the sorted one)
@@ -346,8 +291,8 @@ __device__ bool row_reserve(const SdrfDev& S, int v, LoopShared* sh) {
 }
 
 // insert `key` into row v (must not be present); new entry gets supp = 0, c32 = 0
-__device__ bool row_insert(const SdrfDev& S, int v, int key, LoopShared* sh) {
-    if (!row_reserve(S, v, sh)) return false;
+__device__ bool row_insert(const SdrfDev& S, int v, int key) {
+    if (!row_reserve(S, v)) return false;
     const int start = S.rstart[v], len = S.rlen[v];
     const int pos = start + lower_bound(S.col, start, len, key);
     __syncthreads();
@@ -364,19 +309,22 @@ __device__ bool row_insert(const SdrfDev& S, int v, int key, LoopShared* sh) {
     return true;
 }
 
+// erase `key` (must be present) from the insertion-order list S.ord[start .. start+olen)
+__device__ void ord_erase(const SdrfDev& S, int start, int olen, int key, LoopShared* sh) {
+    if (threadIdx.x == 0) sh->edit_pos = -1;
+    __syncthreads();
+    for (int t = threadIdx.x; t < olen; t += SDRF_THREADS)
+        if (S.ord[start + t] == key) sh->edit_pos = start + t;
+    __syncthreads();
+    shift_left(S.ord, sh->edit_pos + 1, start + olen);
+}
+
 // delete `key` from row v (must be present)
 __device__ void row_delete(const SdrfDev& S, int v, int key, LoopShared* sh) {
     const int start = S.rstart[v], len = S.rlen[v];
     const int pos = find_sorted(S.col, start, len, key);
-    if (threadIdx.x == 0) sh->edit_pos = -1;
-    __syncthreads();
-    const int olen = len + S.selfl[v];
-    for (int t = threadIdx.x; t < olen; t += SDRF_THREADS)
-        if (S.ord[start + t] == key) sh->edit_pos = start + t;
-    __syncthreads();
-    const int opos = sh->edit_pos;
     shift_left3(S, pos + 1, start + len);
-    shift_left(S.ord, opos + 1, start + olen);
+    ord_erase(S, start, len + S.selfl[v], key, sh);
     if (threadIdx.x == 0) {
         S.owner[start + len - 1] = -1;
         S.c32[start + len - 1] = 0.0f;    // free slots hold 0
@@ -385,11 +333,12 @@ __device__ void row_delete(const SdrfDev& S, int v, int key, LoopShared* sh) {
     __syncthreads();
 }
 
+// append the entry (a,b) to the dirty list; undirected callers pass (min, max) so an edge always names one slot
 __device__ __forceinline__ void push_dirty(const SdrfDev& S, int* counter, int a, int b) {
     const int p = atomicAdd(counter, 1);
     if (p < S.dirty_cap) {
-        S.dirty[2 * p] = min(a, b);
-        S.dirty[2 * p + 1] = max(a, b);
+        S.dirty[2 * p] = a;
+        S.dirty[2 * p + 1] = b;
     }
 }
 
@@ -403,8 +352,14 @@ __device__ void toggle_supports(const SdrfDev& S, const GraphView& g, int k, int
     if (threadIdx.x == 0) sh->cnt_a = 0;
     __syncthreads();
     // every edge at k and at l is dirty (degree change)
-    for (int t = threadIdx.x; t < dk; t += SDRF_THREADS) push_dirty(S, dirty_count, k, S.col[sk + t]);
-    for (int t = threadIdx.x; t < dl; t += SDRF_THREADS) push_dirty(S, dirty_count, l, S.col[sl + t]);
+    for (int t = threadIdx.x; t < dk; t += SDRF_THREADS) {
+        const int w = S.col[sk + t];
+        push_dirty(S, dirty_count, min(k, w), max(k, w));
+    }
+    for (int t = threadIdx.x; t < dl; t += SDRF_THREADS) {
+        const int w = S.col[sl + t];
+        push_dirty(S, dirty_count, min(l, w), max(l, w));
+    }
     // W = N(k) ∩ N(l): four support entries per common neighbour change by delta
     for (int t = threadIdx.x; t < dk; t += SDRF_THREADS) {
         const int w = S.col[sk + t];
@@ -432,7 +387,7 @@ __device__ void toggle_supports(const SdrfDev& S, const GraphView& g, int k, int
             const int z = S.col[sw + p];
             if (z == k || z == l) continue;
             if (find_sorted(S.col, sk, dk, z) >= 0 || find_sorted(S.col, sl, dl, z) >= 0)
-                push_dirty(S, dirty_count, w, z);
+                push_dirty(S, dirty_count, min(w, z), max(w, z));
         }
     }
     __syncthreads();
@@ -477,28 +432,21 @@ __device__ __forceinline__ float classical_loop_curvature(const SdrfDev& S, int 
 // C[i,j] reads d_in[i], d_out[j], N_out(i), N_in(j), A2[i,*] over N_in(j) and A2[*,j] over N_out(i)
 // (bfc_cuda.py:20-44); A2[a,b] changes iff (a = k and l -> b) or (b = l and a -> k).  Hence: the entries leaving k
 // and l, the entries arriving at k and l, and the entries i -> j with i -> k and l -> j.
-__device__ __forceinline__ void push_dirty_pair(const SdrfDev& S, int* counter, int a, int b) {
-    const int p = atomicAdd(counter, 1);
-    if (p < S.dirty_cap) {
-        S.dirty[2 * p] = a;
-        S.dirty[2 * p + 1] = b;
-    }
-}
 __device__ void directed_mark_dirty(const SdrfDev& S, int k, int l, int* dirty_count) {
     const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
     const int n = S.n;
     const int sok = S.rstart[k], nok = S.rlen[k], sol = S.rstart[l], nol = S.rlen[l];
     const int sik = S.rstart[n + k], nik = S.rlen[n + k], sil = S.rstart[n + l], nil = S.rlen[n + l];
-    for (int t = threadIdx.x; t < nok; t += SDRF_THREADS) push_dirty_pair(S, dirty_count, k, S.col[sok + t]);
-    for (int t = threadIdx.x; t < nol; t += SDRF_THREADS) push_dirty_pair(S, dirty_count, l, S.col[sol + t]);
-    for (int t = threadIdx.x; t < nik; t += SDRF_THREADS) push_dirty_pair(S, dirty_count, S.col[sik + t], k);
-    for (int t = threadIdx.x; t < nil; t += SDRF_THREADS) push_dirty_pair(S, dirty_count, S.col[sil + t], l);
+    for (int t = threadIdx.x; t < nok; t += SDRF_THREADS) push_dirty(S, dirty_count, k, S.col[sok + t]);
+    for (int t = threadIdx.x; t < nol; t += SDRF_THREADS) push_dirty(S, dirty_count, l, S.col[sol + t]);
+    for (int t = threadIdx.x; t < nik; t += SDRF_THREADS) push_dirty(S, dirty_count, S.col[sik + t], k);
+    for (int t = threadIdx.x; t < nil; t += SDRF_THREADS) push_dirty(S, dirty_count, S.col[sil + t], l);
     for (int t = warp; t < nik; t += SDRF_WARPS) {
         const int i = S.col[sik + t];
         const int soi = S.rstart[i], noi = S.rlen[i];
         for (int p = lane; p < noi; p += 32) {
             const int j = S.col[soi + p];
-            if (find_sorted(S.col, sol, nol, j) >= 0) push_dirty_pair(S, dirty_count, i, j);
+            if (find_sorted(S.col, sol, nol, j) >= 0) push_dirty(S, dirty_count, i, j);
         }
     }
     __syncthreads();
@@ -608,24 +556,20 @@ __device__ __forceinline__ void sdrf_loop_body(const SdrfDev& S, int loops, int 
             }
             const int xu = (int)block_best(Best{0.0f, umin}, &sh.red).key;
             const int xru = (int)block_best(Best{0.0f, umax}, &sh.red).key;
-            unsigned long long pmin = ~0ull, pmax = ~0ull;
-            {
-                // (the insertion-order row holds the node itself where its loop was added: G.edges reports it there)
-                const int st = S.rstart[xu], len = S.rlen[xu];
-                for (int t = tid; t < len + S.selfl[xu]; t += SDRF_THREADS) {
+            // this thread's first position in u's insertion-order row of an entry (u, v >= u) of value `val` (the row
+            // holds the node itself where its loop was added: G.edges reports it there)
+            auto first_pos = [&](int u, float val) {
+                const int st = S.rstart[u], len = S.rlen[u];
+                unsigned long long p = ~0ull;
+                for (int t = tid; t < len + S.selfl[u]; t += SDRF_THREADS) {
                     const int v = S.ord[st + t];
-                    const bool hit = v == xu ? classical_loop_curvature(S, xu) == vmin
-                                             : (v > xu && S.c32[find_sorted(S.col, st, len, v)] == vmin);
-                    if (hit) pmin = min(pmin, (unsigned long long)t);
+                    const bool hit = v == u ? classical_loop_curvature(S, u) == val
+                                            : (v > u && S.c32[find_sorted(S.col, st, len, v)] == val);
+                    if (hit) p = min(p, (unsigned long long)t);
                 }
-                const int st2 = S.rstart[xru], len2 = S.rlen[xru];
-                for (int t = tid; t < len2 + S.selfl[xru]; t += SDRF_THREADS) {
-                    const int v = S.ord[st2 + t];
-                    const bool hit = v == xru ? classical_loop_curvature(S, xru) == vmax
-                                              : (v > xru && S.c32[find_sorted(S.col, st2, len2, v)] == vmax);
-                    if (hit) pmax = min(pmax, (unsigned long long)t);
-                }
-            }
+                return p;
+            };
+            unsigned long long pmin = first_pos(xu, vmin), pmax = first_pos(xru, vmax);
             pmin = block_best(Best{0.0f, pmin}, &sh.red).key;
             pmax = block_best(Best{0.0f, pmax}, &sh.red).key;
             if (tid == 0) {
@@ -864,8 +808,8 @@ __device__ __forceinline__ void sdrf_loop_body(const SdrfDev& S, int loops, int 
         const int k = sh.k, l = sh.l;
         constexpr int L_ROW = (MODE == LOOP_DIRECTED);  // directed: the mirror entry lives in the predecessor rows
         if (k >= 0) {                                   // :69-73
-            bool ok = row_insert(S, k, l, &sh);
-            ok = ok && row_insert(S, L_ROW * S.n + l, k, &sh);
+            bool ok = row_insert(S, k, l);
+            ok = ok && row_insert(S, L_ROW * S.n + l, k);
             if (!ok) {
                 if (tid == 0) sh.status = DCR_SDRF_ARENA_FULL;
                 __syncthreads();
@@ -880,27 +824,19 @@ __device__ __forceinline__ void sdrf_loop_body(const SdrfDev& S, int loops, int 
         }
         if (sh.do_remove == 2) {                        // G.remove_edge(0, 0): only the insertion-order rows change (A[0,0] = 0 already)
             for (int row = 0; row <= (MODE == LOOP_DIRECTED ? S.n : 0); row += max(S.n, 1)) {   // node 0's row(s)
-                const int start = S.rstart[row], olen = S.rlen[row] + 1;
-                if (tid == 0) sh.edit_pos = -1;
-                __syncthreads();
-                for (int t = tid; t < olen; t += SDRF_THREADS)
-                    if (S.ord[start + t] == 0) sh.edit_pos = start + t;
-                __syncthreads();
-                shift_left(S.ord, sh.edit_pos + 1, start + olen);
+                ord_erase(S, S.rstart[row], S.rlen[row] + 1, 0, &sh);
                 if (tid == 0) S.selfl[row] = 0;
                 __syncthreads();
             }
         } else if (sh.do_remove == 3) {                 // classical loop: G.remove_edge(u, u) — degree - 2, u no longer its own neighbour
             const int u = sh.xr, start = S.rstart[u], len = S.rlen[u];
-            if (tid == 0) sh.edit_pos = -1;
-            __syncthreads();
-            for (int t = tid; t < len + 1; t += SDRF_THREADS)
-                if (S.ord[start + t] == u) sh.edit_pos = start + t;
-            __syncthreads();
-            shift_left(S.ord, sh.edit_pos + 1, start + len + 1);
+            ord_erase(S, start, len + 1, u, &sh);
             if (tid == 0) S.selfl[u] = 0;
             __syncthreads();
-            for (int t = tid; t < len; t += SDRF_THREADS) push_dirty(S, &dirty_count, u, S.col[start + t]);   // every edge at u changes
+            for (int t = tid; t < len; t += SDRF_THREADS) {                 // every edge at u changes
+                const int w = S.col[start + t];
+                push_dirty(S, &dirty_count, min(u, w), max(u, w));
+            }
             __syncthreads();
         } else if (sh.do_remove) {                      // :84-88
             const int xr = sh.xr, yr = sh.yr;
@@ -999,6 +935,25 @@ sdrf_batch_loop_kernel(const SdrfBatchDesc* __restrict__ descs, int remove_edges
                                 d.n_uniforms, d.forced_choice, guard, d.log, d.result);
 }
 
+// the kernels of the loop flavour that runs DCR_SDRF_MODE_* `mode`
+struct LoopKernels {
+    decltype(&sdrf_init_curvature_kernel<LOOP_BFC>) init;
+    decltype(&sdrf_loop_kernel<LOOP_BFC>) single;
+    decltype(&sdrf_batch_loop_kernel<LOOP_BFC>) batch;
+};
+static LoopKernels loop_kernels(int mode) {
+    switch (mode) {
+    case DCR_SDRF_MODE_BFC:
+        return {sdrf_init_curvature_kernel<LOOP_BFC>, sdrf_loop_kernel<LOOP_BFC>, sdrf_batch_loop_kernel<LOOP_BFC>};
+    case DCR_SDRF_MODE_BFC_DIRECTED:
+        return {sdrf_init_curvature_kernel<LOOP_DIRECTED>, sdrf_loop_kernel<LOOP_DIRECTED>,
+                sdrf_batch_loop_kernel<LOOP_DIRECTED>};
+    default:
+        return {sdrf_init_curvature_kernel<LOOP_CLASSICAL>, sdrf_loop_kernel<LOOP_CLASSICAL>,
+                sdrf_batch_loop_kernel<LOOP_CLASSICAL>};
+    }
+}
+
 // ------------------------------------------------------------------------------------------------------------
 // export
 // ------------------------------------------------------------------------------------------------------------
@@ -1050,7 +1005,6 @@ using namespace dcr;
 struct dcr_sdrf {
     SdrfDev dev;
     void* slab;           // one allocation backing every array
-    int32_t pending_n;
     int mode;             // DCR_SDRF_MODE_*
     int64_t n_self;       // nodes that list themselves (self-loops of G)
 };
@@ -1137,7 +1091,6 @@ static int sdrf_create_impl(int n, int mode, const int32_t* rowptr_host, const i
     s->n_self = n_self;
     SdrfDev& D = s->dev;
     D.n = n;
-    D.rows = rows;
     D.ctype = mode >= DCR_SDRF_MODE_1D ? mode - DCR_SDRF_MODE_1D : 0;
     D.cap_total = (int)cap_total;
     const int64_t row_cap_max = (int64_t)d1 + max_additions + 2;
@@ -1169,7 +1122,6 @@ static int sdrf_create_impl(int n, int mode, const int32_t* rowptr_host, const i
     D.imp = carve<uint32_t>(p, D.imp_cap); D.pend = carve<double>(p, D.imp_cap);
     D.dirty = carve<int32_t>(p, (size_t)2 * D.dirty_cap); D.work = carve<int32_t>(p, D.dirty_cap);
     D.wlist = carve<int32_t>(p, D.row_cap_max);
-    s->pending_n = 0;
 
     auto fail = [&](cudaError_t err, const char* what) {
         cudaFree(s->slab);
@@ -1194,13 +1146,8 @@ static int sdrf_create_impl(int n, int mode, const int32_t* rowptr_host, const i
     SDRF_TRY(cudaMemcpy(D.scalars, scal, sizeof(scal), cudaMemcpyHostToDevice));
     if (sum_cap > 0) {
         const int ctas = (int)std::min<int64_t>((sum_cap + 7) / 8, (int64_t)sm_count() * 8);
-        if (directed) {
-            sdrf_init_curvature_kernel<LOOP_DIRECTED><<<ctas, 256>>>(D, (int)sum_cap);
-        } else {
-            sdrf_init_support_kernel<<<ctas, 256>>>(D, (int)sum_cap);
-            if (mode == DCR_SDRF_MODE_BFC) sdrf_init_curvature_kernel<LOOP_BFC><<<ctas, 256>>>(D, (int)sum_cap);
-            else sdrf_init_curvature_kernel<LOOP_CLASSICAL><<<ctas, 256>>>(D, (int)sum_cap);
-        }
+        if (!directed) sdrf_init_support_kernel<<<ctas, 256>>>(D, (int)sum_cap);
+        loop_kernels(mode).init<<<ctas, 256>>>(D, (int)sum_cap);
         SDRF_TRY(cudaGetLastError());
     }
     SDRF_TRY(cudaDeviceSynchronize());
@@ -1231,15 +1178,9 @@ extern "C" int dcr_sdrf_run(dcr_sdrf* s, int loops, int remove_edges, double rem
                             dcr_sdrf_result* result, void* stream) {
     if (!s || !result || (loops > 0 && !log)) { set_error("dcr_sdrf_run: bad arguments"); return 1; }
     const int tau_inf = std::isinf(tau) && tau > 0;
-    cudaStream_t st = (cudaStream_t)stream;
-#define SDRF_LAUNCH(MODE)                                                                                              \
-    sdrf_loop_kernel<MODE><<<1, SDRF_THREADS, 0, st>>>(s->dev, loops, remove_edges, (float)removal_bound, removal_bound, \
-                                                       tau, tau_inf, uniforms, (long long)n_uniforms, forced_choice,    \
-                                                       guard, log, result)
-    if (s->mode == DCR_SDRF_MODE_BFC) SDRF_LAUNCH(LOOP_BFC);
-    else if (s->mode == DCR_SDRF_MODE_BFC_DIRECTED) SDRF_LAUNCH(LOOP_DIRECTED);
-    else SDRF_LAUNCH(LOOP_CLASSICAL);
-#undef SDRF_LAUNCH
+    loop_kernels(s->mode).single<<<1, SDRF_THREADS, 0, (cudaStream_t)stream>>>(
+        s->dev, loops, remove_edges, (float)removal_bound, removal_bound, tau, tau_inf, uniforms, (long long)n_uniforms,
+        forced_choice, guard, log, result);
     DCR_LAUNCH_CHECK();
     return 0;
 }
@@ -1290,11 +1231,8 @@ extern "C" int dcr_sdrf_run_batch(const dcr_sdrf_batch_run* runs, int count, int
     cudaStream_t st = (cudaStream_t)stream;
     // pageable source: the copy is staged before cudaMemcpyAsync returns, so `descs` may go out of scope
     DCR_CUDA(cudaMemcpyAsync(workspace, descs.data(), sizeof(SdrfBatchDesc) * count, cudaMemcpyHostToDevice, st));
-    const SdrfBatchDesc* dd = (const SdrfBatchDesc*)workspace;
-    const int mode = runs[0].state->mode;
-    if (mode == DCR_SDRF_MODE_BFC) sdrf_batch_loop_kernel<LOOP_BFC><<<count, SDRF_THREADS, 0, st>>>(dd, remove_edges, guard);
-    else if (mode == DCR_SDRF_MODE_BFC_DIRECTED) sdrf_batch_loop_kernel<LOOP_DIRECTED><<<count, SDRF_THREADS, 0, st>>>(dd, remove_edges, guard);
-    else sdrf_batch_loop_kernel<LOOP_CLASSICAL><<<count, SDRF_THREADS, 0, st>>>(dd, remove_edges, guard);
+    loop_kernels(runs[0].state->mode).batch<<<count, SDRF_THREADS, 0, st>>>((const SdrfBatchDesc*)workspace,
+                                                                             remove_edges, guard);
     DCR_LAUNCH_CHECK();
     return 0;
 }

@@ -12,12 +12,6 @@ class DcrError(RuntimeError):
     pass
 
 
-class SdrfResult(C.Structure):
-    _fields_ = [("status", C.c_int32), ("iterations_done", C.c_int32), ("draws_used", C.c_int32),
-                ("stopped", C.c_int32), ("pending_n", C.c_int32), ("pending_x", C.c_int32),
-                ("pending_y", C.c_int32), ("reserved", C.c_int32)]
-
-
 class SdrfBatchRun(C.Structure):
     """``dcr_sdrf_batch_run``: one run of ``dcr_sdrf_run_batch`` (pointers are device pointers)."""
     _fields_ = [("state", C.c_void_p), ("loops", C.c_int32), ("forced_choice", C.c_int32),

@@ -18,6 +18,8 @@ from . import lib as L
 # numpy's own messages for the ValueErrors np.random.choice raises (sdrf_cuda_bfc.py:64-68)
 _MSG_NAN = "probabilities contain NaN"
 _MSG_SUM = "probabilities do not sum to 1"
+# the fields of dcr_sdrf_result that the host reads, in record order
+_RESULT_KEYS = ("status", "iterations_done", "draws_used", "stopped", "pending_n", "pending_x", "pending_y")
 
 
 def host_choice(improvements: np.ndarray, tau, u: float) -> int:
@@ -90,9 +92,7 @@ class SdrfState:
                                       float(tau), uniforms.data_ptr(), int(uniforms.numel()), int(forced_choice),
                                       float(guard), log.data_ptr(), self._result.data_ptr(), L.current_stream()),
                 "dcr_sdrf_run")
-        r = self._result.cpu().tolist()
-        res = {"status": r[0], "iterations_done": r[1], "draws_used": r[2], "stopped": r[3], "pending_n": r[4],
-               "pending_x": r[5], "pending_y": r[6]}
+        res = dict(zip(_RESULT_KEYS, self._result.cpu().tolist()))
         return res, log[: res["iterations_done"]]
 
     def pending_improvements(self, n: int) -> np.ndarray:
@@ -155,6 +155,31 @@ def _raise_for_status(status: int):
 CLASSICAL_MODES = {"1d": L.SDRF_MODE_1D, "augmented": L.SDRF_MODE_AUGMENTED, "haantjes": L.SDRF_MODE_HAANTJES}
 
 
+def _loop_mode(curv_type: str, is_undirected: bool):
+    """``(L.SDRF_MODE_*, order)`` of the loop that runs ``curv_type``: ``order(edge_index, num_nodes)`` lists the input
+    in the insertion order that loop starts from (``_new_state`` takes its result)."""
+    if curv_type == "bfc":
+        if is_undirected:    # G keeps self-loops (sdrf_cuda_bfc.py:31), A does not (:29)
+            return L.SDRF_MODE_BFC, lambda ei, n: G.networkx_order(ei, n, keep_self_loops=True)
+        return L.SDRF_MODE_BFC_DIRECTED, lambda ei, n: G.digraph_order(ei, n, keep_self_loops=True)
+    if curv_type in CLASSICAL_MODES:
+        return CLASSICAL_MODES[curv_type], lambda ei, n: G.classical_order(ei, n, keep_self_loops=True)
+    raise Exception(f"Method {curv_type} not available.")    # classical_curvatures.py:27-28
+
+
+def _new_state(mode: int, order: tuple, loops: int) -> SdrfState:
+    """State of one run from its ``order`` (``_loop_mode``); the directed order also carries the predecessor lists."""
+    return SdrfState(order[0], order[1], max(int(loops), 0), mode, *order[2:])
+
+
+def _pad_uniforms(uniforms, loops: int):
+    """``uniforms`` as fp64, padded with NaN ("not supplied") to ``loops`` values, and the number supplied."""
+    u = np.ascontiguousarray(uniforms, dtype=np.float64)
+    if u.size < loops:
+        u = np.concatenate([u, np.full(loops - u.size, np.nan)])
+    return u, int(np.count_nonzero(~np.isnan(u)))
+
+
 def sdrf(edge_index, num_nodes: int, loops: int, remove_edges: bool, removal_bound: float, tau,
          uniforms: np.ndarray | None = None, guard: float = 1e-9, return_log: bool = False,
          state_out: list | None = None, is_undirected: bool = True, curv_type: str = "bfc"):
@@ -170,29 +195,14 @@ def sdrf(edge_index, num_nodes: int, loops: int, remove_edges: bool, removal_bou
     ends up advanced by the number of draws actually used.
     """
     L.require_cuda()
-    directed = False
-    if curv_type == "bfc":
-        if is_undirected:
-            rowptr, order = G.networkx_order(edge_index, num_nodes, keep_self_loops=True)    # G keeps them (:31), A does not (:29)
-            state = SdrfState(rowptr, order, max_additions=max(int(loops), 0))
-        else:
-            directed = True
-            s_rp, s_ord, p_rp, p_ord = G.digraph_order(edge_index, num_nodes, keep_self_loops=True)
-            state = SdrfState(s_rp, s_ord, max_additions=max(int(loops), 0), mode=L.SDRF_MODE_BFC_DIRECTED,
-                              in_rowptr=p_rp, in_order=p_ord)
-    elif curv_type in CLASSICAL_MODES:
-        rowptr, order = G.classical_order(edge_index, num_nodes, keep_self_loops=True)
-        state = SdrfState(rowptr, order, max_additions=max(int(loops), 0), mode=CLASSICAL_MODES[curv_type])
-    else:
-        raise Exception(f"Method {curv_type} not available.")    # classical_curvatures.py:27-28
+    mode, order = _loop_mode(curv_type, is_undirected)
+    directed = mode == L.SDRF_MODE_BFC_DIRECTED
+    state = _new_state(mode, order(edge_index, num_nodes), loops)
     own_stream = uniforms is None
     if own_stream:
         rng_state = np.random.get_state()
         uniforms = np.random.random_sample(max(int(loops), 0))
-    uniforms = np.ascontiguousarray(uniforms, dtype=np.float64)
-    if uniforms.size < max(loops, 0):
-        uniforms = np.concatenate([uniforms, np.full(loops - uniforms.size, np.nan)])  # NaN = "not supplied"
-    n_supplied = int(np.count_nonzero(~np.isnan(uniforms)))
+    uniforms, n_supplied = _pad_uniforms(uniforms, max(loops, 0))
     u_dev = torch.from_numpy(uniforms).to(state.device)
     logs = []
     done = draws = 0
@@ -250,8 +260,7 @@ def run_batch(states, loops, removal_bounds, taus, uniforms, forced, logs, remov
     L.check(L.load().dcr_sdrf_run_batch(runs, b, int(bool(remove_edges)), float(guard), workspace.data_ptr(),
                                         workspace.numel() * workspace.element_size(), L.current_stream()),
             "dcr_sdrf_run_batch")
-    keys = ("status", "iterations_done", "draws_used", "stopped", "pending_n", "pending_x", "pending_y")
-    return [dict(zip(keys, r)) for r in results[:b].cpu().tolist()]
+    return [dict(zip(_RESULT_KEYS, r)) for r in results[:b].cpu().tolist()]
 
 
 def _per_run(name: str, value, count: int) -> list:
@@ -295,39 +304,20 @@ def sdrf_batch(edge_indices, num_nodes, loops, remove_edges: bool, removal_bound
     iters = [max(int(v), 0) for v in _per_run("loops", loops, count)]
     bounds = [float(v) for v in _per_run("removal_bound", removal_bound, count)]
     taus = _per_run("tau", tau, count)
-    if curv_type != "bfc" and curv_type not in CLASSICAL_MODES:
-        raise Exception(f"Method {curv_type} not available.")    # classical_curvatures.py:27-28
-    directed = curv_type == "bfc" and not is_undirected
+    mode, order = _loop_mode(curv_type, is_undirected)
+    directed = mode == L.SDRF_MODE_BFC_DIRECTED
     L.require_cuda()
 
-    orders = {}
-
-    def order_of(r):
-        key = nodes[r] if shared_input else r
-        if key not in orders:
-            if curv_type != "bfc":
-                orders[key] = G.classical_order(inputs[r], nodes[r], keep_self_loops=True)
-            elif directed:
-                orders[key] = G.digraph_order(inputs[r], nodes[r], keep_self_loops=True)
-            else:
-                orders[key] = G.networkx_order(inputs[r], nodes[r], keep_self_loops=True)
-        return orders[key]
-
-    mode = (L.SDRF_MODE_BFC_DIRECTED if directed else L.SDRF_MODE_BFC) if curv_type == "bfc" \
-        else CLASSICAL_MODES[curv_type]
+    orders = {}     # a shared input is put in order once per node count
     states = []
     try:
         for r in range(count):
-            o = order_of(r)
-            if directed:
-                states.append(SdrfState(o[0], o[1], max_additions=iters[r], mode=mode, in_rowptr=o[2], in_order=o[3]))
-            else:
-                states.append(SdrfState(o[0], o[1], max_additions=iters[r], mode=mode))
+            key = nodes[r] if shared_input else r
+            if key not in orders:
+                orders[key] = order(inputs[r], nodes[r])
+            states.append(_new_state(mode, orders[key], iters[r]))
         dev = states[0].device
-        # per run as in sdrf(): uniforms shorter than loops are padded with NaN ("not supplied")
-        padded = [np.concatenate([u, np.full(iters[r] - u.size, np.nan)]) if u.size < iters[r] else u
-                  for r, u in enumerate(uni)]
-        supplied = [int(np.count_nonzero(~np.isnan(u))) for u in padded]
+        padded, supplied = zip(*(_pad_uniforms(u, iters[r]) for r, u in enumerate(uni)))
         u_dev = [torch.from_numpy(u).to(dev) for u in padded]
         logs = [torch.empty((max(iters[r], 1), L.SDRF_LOG_INTS), dtype=torch.int32, device=dev) for r in range(count)]
         results = torch.zeros((count, 8), dtype=torch.int32, device=dev)

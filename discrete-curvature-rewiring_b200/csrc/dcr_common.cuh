@@ -139,4 +139,22 @@ __device__ __forceinline__ float closing_finish(const ClosingFirst& f, long long
     return __double2float_rn(__dadd_rn(w, (double)f.c32));
 }
 
+// The paper-flavour value (bfc_naive.py:31-32 / :39-40) evaluated left to right in fp64 with explicitly rounded
+// operations; shared by the paper pass (dcr_bfc_paper.cu) and the paper-flavour SDRF loop (dcr_sdrf.cu).
+__device__ __forceinline__ double paper_value(int d1, int d2, int tri, int sq1, int sq2, int gamma) {
+    const int dmax = max(d1, d2), dmin = min(d1, d2);
+    double t = __ddiv_rn(2.0, (double)d1);
+    t = __dadd_rn(t, __ddiv_rn(2.0, (double)d2));
+    t = __dadd_rn(t, -2.0);
+    t = __dadd_rn(t, __ddiv_rn((double)(2 * (long long)tri), (double)dmax));
+    t = __dadd_rn(t, __ddiv_rn((double)tri, (double)dmin));
+    if (sq1 > 0 && sq2 > 0) {
+        double u = __ddiv_rn(1.0, (double)gamma);
+        u = __ddiv_rn(u, (double)dmax);
+        u = __dmul_rn(u, (double)(sq1 + sq2));
+        t = __dadd_rn(t, u);
+    }
+    return t;
+}
+
 }  // namespace dcr

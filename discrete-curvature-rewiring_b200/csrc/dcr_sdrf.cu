@@ -18,6 +18,7 @@
 // each, in one launch of the batch kernel (dcr_sdrf_run_batch).
 #include <algorithm>
 #include <cmath>
+#include <type_traits>
 #include <vector>
 
 #include "dcr_directed.cuh"
@@ -31,7 +32,9 @@ namespace dcr {
 //                  rows [n,2n) the predecessors; curvature and scoring by the definition (dcr_directed.cuh)
 //   LOOP_CLASSICAL sdrf_no_cuda with '1d' / 'augmented' / 'haantjes' (rewiring/sdrf_no_cuda.py:9-68,
 //                  curvature/classical_curvatures.py:6-46) — integer curvatures from the maintained degrees / supports
-enum { LOOP_BFC = 0, LOOP_DIRECTED = 1, LOOP_CLASSICAL = 2 };
+//   LOOP_PAPER     sdrf_no_cuda's loop with bfc_naive.bfc_edge as the curvature — fp64 paper-flavour values per entry
+//                  (paper_eval), scoring in closed form plus one warp per cell of x's row and y's column (DESIGN §4.9)
+enum { LOOP_BFC = 0, LOOP_DIRECTED = 1, LOOP_CLASSICAL = 2, LOOP_PAPER = 3 };
 
 #ifndef DCR_SDRF_THREADS
 #define DCR_SDRF_THREADS 1024
@@ -39,6 +42,7 @@ enum { LOOP_BFC = 0, LOOP_DIRECTED = 1, LOOP_CLASSICAL = 2 };
 constexpr int SDRF_THREADS = DCR_SDRF_THREADS;
 constexpr int SDRF_WARPS = SDRF_THREADS / 32;
 constexpr uint32_t IMP_MASKED = 0xffffffffu;   // bit pattern marking a masked cell in the improvement matrix
+constexpr unsigned long long IMP_MASKED64 = ~0ull;   // (LOOP_PAPER's fp64 cells; a NaN, which no improvement is)
 constexpr int STATUS_TOO_MANY_CANDIDATES = DCR_SDRF_TOO_MANY_CANDIDATES;
 
 // Optional phase timers (build with -DDCR_SDRF_PROFILE): cycles per phase summed over the iterations of a launch,
@@ -75,11 +79,13 @@ struct SdrfDev {
     int32_t* ord;         // arena: neighbour ids in insertion order (same row offsets)
     int32_t* supp;        // arena: #common neighbours of the entry's edge (A2[i,j])
     float* c32;           // arena: cuda-flavour curvature of the entry
+                          // (LOOP_PAPER keeps no supports and no fp32 value: supp / c32 hold the high / low word of the
+                          //  entry's fp64 paper-flavour value, so every arena edit moves it unchanged; see paper_get)
     int32_t* owner;       // arena: row id of the slot, -1 = free
     int32_t* flag;        // arena: dedupe flags for the refresh
     int32_t* scalars;     // [0] arena_top, [1] nnz
     int32_t* base1; int32_t* base2; int32_t* posI; int32_t* posJ;   // score scratch [row_cap_max]
-    uint32_t* imp;        // improvement matrix (fp32 bits)
+    uint32_t* imp;        // improvement matrix (fp32 bits; LOOP_PAPER: fp64 bits, two words per cell)
     double* pend;         // compact improvements of a pending iteration
     int32_t* dirty;       // pairs (a,b): 2*dirty_cap ints
     int32_t* work;        // slots to refresh: dirty_cap ints
@@ -89,15 +95,19 @@ struct SdrfDev {
 // ------------------------------------------------------------------------------------------------------------
 // block-wide primitives (SDRF_THREADS threads, every thread calls)
 // ------------------------------------------------------------------------------------------------------------
-struct Best { float v; unsigned long long key; };   // "smaller v wins, then smaller key"
+template <class V>
+struct BestT { V v; unsigned long long key; };   // "smaller v wins, then smaller key"
+using Best = BestT<float>;                       // (the paper loop compares fp64 values: BestT<double>)
 
-__device__ __forceinline__ Best best_of(Best a, Best b) {
+template <class V>
+__device__ __forceinline__ BestT<V> best_of(BestT<V> a, BestT<V> b) {
     return (b.v < a.v || (b.v == a.v && b.key < a.key)) ? b : a;
 }
-__device__ __forceinline__ Best warp_best(Best a) {
+template <class V>
+__device__ __forceinline__ BestT<V> warp_best(BestT<V> a) {
 #pragma unroll
     for (int o = 16; o; o >>= 1) {
-        Best b;
+        BestT<V> b;
         b.v = __shfl_xor_sync(FULL, a.v, o);
         b.key = __shfl_xor_sync(FULL, a.key, o);
         a = best_of(a, b);
@@ -110,23 +120,32 @@ struct Reduce {     // shared-memory scratch for the block primitives
     unsigned long long k[SDRF_WARPS];
     double d[SDRF_WARPS];
     long long l[SDRF_WARPS];
-    Best best;
+    union { Best best; BestT<double> best_d; };
 };
 
-__device__ Best block_best(Best a, Reduce* r) {
+template <class V>
+__device__ BestT<V> block_best(BestT<V> a, Reduce* r) {
+    constexpr bool F64 = sizeof(V) == 8;         // fp64 values go through r->d and r->best_d
     const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
     a = warp_best(a);
-    if (lane == 0) { r->v[warp] = a.v; r->k[warp] = a.key; }
-    __syncthreads();
-    if (warp == 0) {
-        Best b;
-        b.v = lane < SDRF_WARPS ? r->v[lane] : INFINITY;
-        b.key = lane < SDRF_WARPS ? r->k[lane] : ~0ull;
-        b = warp_best(b);
-        if (lane == 0) r->best = b;
+    if (lane == 0) {
+        if constexpr (F64) r->d[warp] = a.v; else r->v[warp] = a.v;
+        r->k[warp] = a.key;
     }
     __syncthreads();
-    Best out = r->best;
+    if (warp == 0) {
+        BestT<V> b;
+        if constexpr (F64) b.v = lane < SDRF_WARPS ? r->d[lane] : (V)INFINITY;
+        else b.v = lane < SDRF_WARPS ? r->v[lane] : INFINITY;
+        b.key = lane < SDRF_WARPS ? r->k[lane] : ~0ull;
+        b = warp_best(b);
+        if (lane == 0) {
+            if constexpr (F64) r->best_d = b; else r->best = b;
+        }
+    }
+    __syncthreads();
+    BestT<V> out;
+    if constexpr (F64) out = r->best_d; else out = r->best;
     __syncthreads();
     return out;
 }
@@ -220,6 +239,11 @@ struct LoopShared {
     double below, above;      // normalised CDF just below / at the chosen candidate
     int cnt_a;                // wlist fill of toggle_supports
     int edit_pos;             // ord_erase: slot of the erased id
+};
+// the paper loop's extra fields: fp64 extremes and the fields of bfc(x,y) that every interior cell starts from
+struct LoopSharedPaper : LoopShared {
+    double cxy_d, cmax_d;
+    int tri, sq_x, sq_y, gamma;
 };
 
 template <class T>
@@ -331,6 +355,16 @@ __device__ void row_delete(const SdrfDev& S, int v, int key, LoopShared* sh) {
         S.rlen[v] = len - 1;
     }
     __syncthreads();
+}
+
+// LOOP_PAPER: the fp64 value of the entry at `slot`, stored as its high word in supp and its low word in c32 (bit moves
+// only: nothing does float arithmetic on those words in this loop); a free or new slot reads +0.0
+__device__ __forceinline__ double paper_get(const SdrfDev& S, int slot) {
+    return __hiloint2double(S.supp[slot], __float_as_int(S.c32[slot]));
+}
+__device__ __forceinline__ void paper_put(const SdrfDev& S, int slot, double v) {
+    S.supp[slot] = __double2hiint(v);
+    S.c32[slot] = __int_as_float(__double2loint(v));
 }
 
 // append the entry (a,b) to the dirty list; undirected callers pass (min, max) so an edge always names one slot
@@ -453,6 +487,146 @@ __device__ void directed_mark_dirty(const SdrfDev& S, int k, int l, int* dirty_c
 }
 
 // ------------------------------------------------------------------------------------------------------------
+// paper loop: bfc_naive.bfc_edge over the arena's sorted rows (DESIGN §4.9)
+// ------------------------------------------------------------------------------------------------------------
+// The arena graph plus at most one VIRTUAL edge {p,q} that is not in it (p = q = -1: none): candidate scoring
+// evaluates bfc(x,y) on G + (i,j) without editing the arena.
+struct PaperView {
+    GraphView g;
+    int p, q;
+    __device__ __forceinline__ int deg(int a) const { return g.degree(a) + (a == p || a == q); }
+    // t-th neighbour of a: the sorted row, then the virtual neighbour
+    __device__ __forceinline__ int nb(int a, int t) const {
+        return t < g.degree(a) ? g.col[g.begin(a) + t] : (a == p ? q : p);
+    }
+    __device__ __forceinline__ bool has(int a, int b) const {
+        return (a == p && b == q) || (a == q && b == p) || find_sorted(g.col, g.begin(a), g.degree(a), b) >= 0;
+    }
+};
+
+// For the edge (a,b) and k in N(a): c(k) = |N(k) ∩ M_b| with M_b = N(b) \ N(a) \ {a} when k is in M_a (then k is a
+// square at a iff c(k) > 0, and bfc_naive.py:36-37 gives gamma = max c(k)); -1 when k = b or k is a common
+// neighbour (a triangle).  Serial over the shorter of N(k) and N(b).
+__device__ __forceinline__ int paper_c(const PaperView& v, int a, int b, int k) {
+    if (k == b || v.has(b, k)) return -1;
+    const int dk = v.deg(k), db = v.deg(b);
+    int c = 0;
+    if (dk <= db) {
+        for (int s = 0; s < dk; ++s) {
+            const int w = v.nb(k, s);
+            c += w != a && v.has(b, w) && !v.has(a, w);
+        }
+    } else {
+        for (int s = 0; s < db; ++s) {
+            const int w = v.nb(b, s);
+            c += w != a && !v.has(a, w) && v.has(k, w);
+        }
+    }
+    return c;
+}
+
+// bfc_naive.bfc_edge(G, u, v) of the edge (u,v) (warp-cooperative, every lane returns it): the int 0 of :18-19 when
+// deg_min == 1, else paper_value over tri, |□_u|, |□_v| and gamma — bit-identical to the paper pass.
+__device__ double paper_eval(const PaperView& v, int u, int w, int lane) {
+    const int du = v.deg(u), dw = v.deg(w);
+    if (min(du, dw) <= 1) return 0.0;
+    int tri = 0, sq_u = 0, sq_w = 0, gam = 0;
+    for (int t = lane; t < du; t += 32) {
+        const int k = v.nb(u, t);
+        const int c = paper_c(v, u, w, k);
+        tri += c < 0 && k != w;
+        sq_u += c > 0;
+        gam = max(gam, c);
+    }
+    for (int t = lane; t < dw; t += 32) {
+        const int c = paper_c(v, w, u, v.nb(w, t));
+        sq_w += c > 0;
+        gam = max(gam, c);
+    }
+    return paper_value(du, dw, warp_sum(tri), warp_sum(sq_u), warp_sum(sq_w), warp_max(gam));
+}
+
+// Paper loop: edges whose bfc_edge may change when {k,l} is toggled (call with the edge present).  For an edge (u,v)
+// away from k and l, N(u), N(v), tri and M_u, M_v stay; only c(k) or c(l) can change, and only when k is in M_u and
+// l in M_v (or mirrored).  Hence: the edges at k and at l, and the edges (a,b) with a in N(k), b in N(l).  Each
+// directed entry is pushed at most once by the second part: at most 2 nnz pairs per toggle.
+__device__ void paper_mark_dirty(const SdrfDev& S, int k, int l, int* dirty_count) {
+    const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
+    const int sk = S.rstart[k], dk = S.rlen[k], sl = S.rstart[l], dl = S.rlen[l];
+    for (int t = threadIdx.x; t < dk; t += SDRF_THREADS) {
+        const int w = S.col[sk + t];
+        push_dirty(S, dirty_count, min(k, w), max(k, w));
+    }
+    for (int t = threadIdx.x; t < dl; t += SDRF_THREADS) {
+        const int w = S.col[sl + t];
+        push_dirty(S, dirty_count, min(l, w), max(l, w));
+    }
+    for (int t = warp; t < dk; t += SDRF_WARPS) {
+        const int a = S.col[sk + t];
+        if (a == l) continue;                                  // (its edges are at l)
+        const int sa = S.rstart[a], da = S.rlen[a];
+        for (int p = lane; p < da; p += 32) {
+            const int b = S.col[sa + p];
+            if (b != k && find_sorted(S.col, sl, dl, b) >= 0) push_dirty(S, dirty_count, min(a, b), max(a, b));
+        }
+    }
+    __syncthreads();
+}
+
+// Paper loop: improvements bfc(x,y) on G + (i,j) minus bfc(x,y) on G for every cell, fp64 bits into imp64 (masked
+// cells as the other loops).  With c(k) of (x,y) computed once (base1 over N(x), base2 over N(y)):
+//   i in M_x, j in M_y : degrees and tri stay, c(i) and c(j) grow by one, nothing else moves —
+//                        |□_x| += [c(i) = 0], |□_y| += [c(j) = 0], gamma = max(gamma, c(i) + 1, c(j) + 1);
+//   i or j a common neighbour : nothing bfc(x,y) reads changes, improvement 0;
+//   i = x (row n_i - 1) or j = y (column n_j - 1) : one warp per cell, paper_eval with the virtual edge (i,j).
+template <class NbI, class NbJ>
+__device__ void paper_score(const SdrfDev& S, const GraphView& g, int x, int y, NbI nbI, int n_i, NbJ nbJ, int n_j,
+                            double cxy, unsigned long long* imp64, LoopSharedPaper* sh) {
+    const int tid = threadIdx.x, lane = tid & 31, warp = tid >> 5;
+    const PaperView none{g, -1, -1};
+    const int mi = n_i - 1, mj = n_j - 1;              // x's and y's neighbours (x and y themselves come last)
+    if (tid == 0) { sh->tri = 0; sh->sq_x = 0; sh->sq_y = 0; sh->gamma = 0; }
+    __syncthreads();
+    for (int t = tid; t < mi + mj; t += SDRF_THREADS) {
+        const bool ys = t >= mi;
+        const int c = ys ? paper_c(none, y, x, nbJ(t - mi)) : paper_c(none, x, y, nbI(t));
+        (ys ? S.base2 : S.base1)[ys ? t - mi : t] = c;
+        if (c > 0) {
+            atomicAdd(ys ? &sh->sq_y : &sh->sq_x, 1);
+            atomicMax(&sh->gamma, c);
+        }
+        if (!ys && c < 0 && nbI(t) != y) atomicAdd(&sh->tri, 1);
+    }
+    __syncthreads();
+    const int dx = S.rlen[x], dy = S.rlen[y];
+    const int tri = sh->tri, sq_x = sh->sq_x, sq_y = sh->sq_y, gam = sh->gamma;
+    const long long cells = (long long)n_i * n_j;
+    for (long long c = tid; c < cells; c += SDRF_THREADS) {
+        const int I = (int)(c / n_j), J = (int)(c - (long long)I * n_j);
+        const int i = nbI(I), j = nbJ(J);
+        if (i == j || edge_slot(g, i, j) >= 0) { imp64[c] = IMP_MASKED64; continue; }
+        if (I == mi || J == mj) continue;                                // the warp pass below
+        const int ci = S.base1[I], cj = S.base2[J];
+        double d = 0.0;
+        if (ci >= 0 && cj >= 0) {
+            const double after = min(dx, dy) <= 1 ? 0.0
+                                 : paper_value(dx, dy, tri, sq_x + (ci == 0), sq_y + (cj == 0),
+                                               max(gam, max(ci, cj) + 1));
+            d = __dsub_rn(after, cxy);
+        }
+        imp64[c] = (unsigned long long)__double_as_longlong(d);
+    }
+    for (int t = warp; t < mi + mj; t += SDRF_WARPS) {
+        const bool row = t < mj;
+        const int I = row ? mi : t - mj, J = row ? t : mj;
+        const int i = nbI(I), j = nbJ(J);
+        if (i == j || edge_slot(g, i, j) >= 0) continue;
+        const double after = paper_eval(PaperView{g, i, j}, x, y, lane);
+        if (lane == 0) imp64[(long long)I * n_j + J] = (unsigned long long)__double_as_longlong(__dsub_rn(after, cxy));
+    }
+}
+
+// ------------------------------------------------------------------------------------------------------------
 // initialisation kernels over arena slots (multi-CTA)
 // ------------------------------------------------------------------------------------------------------------
 __global__ void sdrf_init_support_kernel(SdrfDev S, int top) {
@@ -473,6 +647,11 @@ __global__ void sdrf_init_curvature_kernel(SdrfDev S, int top) {
     for (int s = (blockIdx.x * blockDim.x + threadIdx.x) >> 5; s < top; s += warps) {
         const int a = S.owner[s];
         if (a < 0) continue;
+        if constexpr (MODE == LOOP_PAPER) {
+            const double c = paper_eval(PaperView{{S.rstart, S.rlen, S.col}, -1, -1}, a, S.col[s], lane);
+            if (lane == 0) paper_put(S, s, c);
+            continue;
+        }
         float c;
         if constexpr (MODE == LOOP_DIRECTED) {
             if (a >= S.n) continue;                 // predecessor rows carry no curvature
@@ -487,6 +666,11 @@ __global__ void sdrf_init_curvature_kernel(SdrfDev S, int top) {
     }
 }
 
+__device__ __forceinline__ float val_min(float a, float b) { return fminf(a, b); }
+__device__ __forceinline__ float val_max(float a, float b) { return fmaxf(a, b); }
+__device__ __forceinline__ double val_min(double a, double b) { return fmin(a, b); }
+__device__ __forceinline__ double val_max(double a, double b) { return fmax(a, b); }
+
 // ------------------------------------------------------------------------------------------------------------
 // the loop
 // ------------------------------------------------------------------------------------------------------------
@@ -498,7 +682,19 @@ __device__ __forceinline__ void sdrf_loop_body(const SdrfDev& S, int loops, int 
                                                const double* __restrict__ uniforms, long long n_uniforms,
                                                int forced_choice, double guard, int32_t* __restrict__ log,
                                                dcr_sdrf_result* __restrict__ result) {
-    __shared__ LoopShared sh;
+    constexpr bool PAPER = MODE == LOOP_PAPER;
+    constexpr bool NX_LOOP = MODE == LOOP_CLASSICAL || PAPER;     // sdrf_no_cuda's loop: min / max over G.edges
+    using Val = std::conditional_t<PAPER, double, float>;         // entry values, extremes and improvements
+    using Bits = std::conditional_t<PAPER, unsigned long long, uint32_t>;   // improvement matrix cells
+    constexpr Bits MASKED = PAPER ? IMP_MASKED64 : IMP_MASKED;
+    auto imp_at = [&](long long f) -> Bits { return reinterpret_cast<const Bits*>(S.imp)[f]; };
+    auto value = [&](int s) -> Val {
+        if constexpr (PAPER) return paper_get(S, s); else return S.c32[s];
+    };
+    auto imp_val = [](Bits b) -> Val {
+        if constexpr (PAPER) return __longlong_as_double((long long)b); else return __uint_as_float(b);
+    };
+    __shared__ std::conditional_t<PAPER, LoopSharedPaper, LoopShared> sh;
     __shared__ DirScoreShared dsh;
     __shared__ int dirty_count, work_count, dred[2];
     const int tid = threadIdx.x, lane = tid & 31, warp = tid >> 5;
@@ -514,27 +710,27 @@ __device__ __forceinline__ void sdrf_loop_body(const SdrfDev& S, int loops, int 
 #endif
     for (; it < loops; ++it) {
         const int top = S.scalars[0];
-        if constexpr (MODE == LOOP_CLASSICAL) {
+        if constexpr (NX_LOOP) {
             // ---- 1c. min(G.edges, key=curvature) / max(...) (sdrf_no_cuda.py:27, :59-61) --------------------
             // G.edges lists every edge once, from its first endpoint in node order, neighbours in insertion order:
             // the first minimum is at the smallest u that has an entry (u, v > u) with the minimal value, and among
             // those at the earliest position of u's insertion-order row.  The maximum is taken over the same C_t
             // (curv_dict predates the addition; the new edge is excluded, :59).
-            float vmin = INFINITY, vmax = -INFINITY;
+            Val vmin = INFINITY, vmax = -INFINITY;
             for (int s = tid; s < top; s += SDRF_THREADS) {
                 if (S.owner[s] < 0) continue;
-                const float v = S.c32[s];
-                vmin = fminf(vmin, v);
-                vmax = fmaxf(vmax, v);
+                const Val v = value(s);
+                vmin = val_min(vmin, v);
+                vmax = val_max(vmax, v);
             }
-            for (int u = tid; u < S.n; u += SDRF_THREADS) {     // the loop edges (u,u) of G.edges
+            for (int u = tid; !PAPER && u < S.n; u += SDRF_THREADS) {     // the loop edges (u,u) of G.edges
                 if (!S.selfl[u]) continue;
                 const float v = classical_loop_curvature(S, u);
                 vmin = fminf(vmin, v);
                 vmax = fmaxf(vmax, v);
             }
-            vmin = block_best(Best{vmin, 0ull}, &sh.red).v;
-            vmax = -block_best(Best{-vmax, 0ull}, &sh.red).v;
+            vmin = block_best(BestT<Val>{vmin, 0ull}, &sh.red).v;
+            vmax = -block_best(BestT<Val>{-vmax, 0ull}, &sh.red).v;
             if (!(vmin <= vmax)) {                              // no edges: min() of an empty sequence
                 if (tid == 0) sh.status = DCR_SDRF_EMPTY_GRAPH;
                 __syncthreads();
@@ -544,11 +740,11 @@ __device__ __forceinline__ void sdrf_loop_body(const SdrfDev& S, int loops, int 
             for (int s = tid; s < top; s += SDRF_THREADS) {
                 const int o = S.owner[s];
                 if (o < 0 || S.col[s] < o) continue;
-                const float v = S.c32[s];
+                const Val v = value(s);
                 if (v == vmin) umin = min(umin, (unsigned long long)o);
                 if (v == vmax) umax = min(umax, (unsigned long long)o);
             }
-            for (int u = tid; u < S.n; u += SDRF_THREADS) {
+            for (int u = tid; !PAPER && u < S.n; u += SDRF_THREADS) {
                 if (!S.selfl[u]) continue;
                 const float v = classical_loop_curvature(S, u);
                 if (v == vmin) umin = min(umin, (unsigned long long)u);
@@ -558,13 +754,13 @@ __device__ __forceinline__ void sdrf_loop_body(const SdrfDev& S, int loops, int 
             const int xru = (int)block_best(Best{0.0f, umax}, &sh.red).key;
             // this thread's first position in u's insertion-order row of an entry (u, v >= u) of value `val` (the row
             // holds the node itself where its loop was added: G.edges reports it there)
-            auto first_pos = [&](int u, float val) {
+            auto first_pos = [&](int u, Val val) {
                 const int st = S.rstart[u], len = S.rlen[u];
                 unsigned long long p = ~0ull;
                 for (int t = tid; t < len + S.selfl[u]; t += SDRF_THREADS) {
                     const int v = S.ord[st + t];
                     const bool hit = v == u ? classical_loop_curvature(S, u) == val
-                                            : (v > u && S.c32[find_sorted(S.col, st, len, v)] == val);
+                                            : (v > u && value(find_sorted(S.col, st, len, v)) == val);
                     if (hit) p = min(p, (unsigned long long)t);
                 }
                 return p;
@@ -574,8 +770,10 @@ __device__ __forceinline__ void sdrf_loop_body(const SdrfDev& S, int loops, int 
             pmax = block_best(Best{0.0f, pmax}, &sh.red).key;
             if (tid == 0) {
                 sh.have_min = 1; sh.have_max = 1;
-                sh.x = xu;  sh.y = S.ord[S.rstart[xu] + (int)pmin];   sh.cxy = vmin;
-                sh.xr = xru; sh.yr = S.ord[S.rstart[xru] + (int)pmax]; sh.cmax = vmax;
+                sh.x = xu;  sh.y = S.ord[S.rstart[xu] + (int)pmin];
+                sh.xr = xru; sh.yr = S.ord[S.rstart[xru] + (int)pmax];
+                if constexpr (PAPER) { sh.cxy_d = vmin; sh.cmax_d = vmax; }
+                else { sh.cxy = vmin; sh.cmax = vmax; }
             }
         } else {
         // ---- 1. argmin / argmax of C_t (sdrf_cuda_bfc.py:40-42, :80-82) ---------------------------------
@@ -644,6 +842,8 @@ __device__ __forceinline__ void sdrf_loop_body(const SdrfDev& S, int loops, int 
             } else if constexpr (MODE == LOOP_DIRECTED) {
                 directed_score_prepare(g, gin, x, y, nbI, n_i, nbJ, n_j, sc, &dsh, dred);
                 directed_score_cells(g, gin, x, y, nbI, n_i, nbJ, n_j, sc, &dsh, put);
+            } else if constexpr (PAPER) {
+                paper_score(S, g, x, y, nbI, n_i, nbJ, n_j, sh.cxy_d, reinterpret_cast<unsigned long long*>(S.imp), &sh);
             } else {
                 // sdrf_no_cuda.py:41-46 in closed form: adding (i,j) changes curvature(x,y) only when it touches x or y.
                 // i == x (then j in N(y)\N(x)): deg x + 1 and one more triangle; j == y mirrored; every other
@@ -670,11 +870,11 @@ __device__ __forceinline__ void sdrf_loop_body(const SdrfDev& S, int loops, int 
         double local = 0.0;
         int bad = 0;
         for (long long f = f_lo; f < f_hi; ++f) {
-            const uint32_t bits = S.imp[f];
-            if (bits == IMP_MASKED) continue;
+            const Bits bits = imp_at(f);
+            if (bits == MASKED) continue;
             ++my_cnt;
             if (weigh) {
-                const double e = exp(__dmul_rn((double)__uint_as_float(bits), tau));
+                const double e = exp(__dmul_rn((double)imp_val(bits), tau));
                 if (!(e <= 1.7976931348623157e308)) bad = 1;   // inf or NaN
                 local = __dadd_rn(local, e);
             }
@@ -695,7 +895,7 @@ __device__ __forceinline__ void sdrf_loop_body(const SdrfDev& S, int loops, int 
                 if (forced_choice >= my_off && forced_choice < my_off + my_cnt) {
                     long long c = my_off;
                     for (long long f = f_lo; f < f_hi; ++f) {
-                        if (S.imp[f] == IMP_MASKED) continue;
+                        if (imp_at(f) == MASKED) continue;
                         if (c == forced_choice) { sh.chosen_flat = f; sh.choice = (int)c; break; }
                         ++c;
                     }
@@ -708,17 +908,17 @@ __device__ __forceinline__ void sdrf_loop_body(const SdrfDev& S, int loops, int 
                 }
             } else if (tau_inf) {
                 // softmax.py:5-8: one-hot at the first maximum; the draw then returns that index for any u in [0,1)
-                Best b{INFINITY, ~0ull};
+                BestT<Val> b{(Val)INFINITY, ~0ull};
                 for (long long f = f_lo; f < f_hi; ++f) {
-                    const uint32_t bits = S.imp[f];
-                    if (bits == IMP_MASKED) continue;
-                    b = best_of(b, Best{-__uint_as_float(bits), (unsigned long long)f});
+                    const Bits bits = imp_at(f);
+                    if (bits == MASKED) continue;
+                    b = best_of(b, BestT<Val>{-imp_val(bits), (unsigned long long)f});
                 }
                 b = block_best(b, &sh.red);
                 const long long fstar = (long long)b.key;
                 if (fstar >= f_lo && fstar < f_hi) {
                     long long c = my_off;
-                    for (long long f = f_lo; f < fstar; ++f) c += S.imp[f] != IMP_MASKED;
+                    for (long long f = f_lo; f < fstar; ++f) c += imp_at(f) != MASKED;
                     sh.chosen_flat = fstar;
                     sh.choice = (int)c;
                 }
@@ -737,9 +937,9 @@ __device__ __forceinline__ void sdrf_loop_body(const SdrfDev& S, int loops, int 
                 long long c = my_off, found_c = 0;
                 double run = carry;
                 for (long long f = f_lo; f < f_hi; ++f) {
-                    const uint32_t bits = S.imp[f];
-                    if (bits == IMP_MASKED) continue;
-                    const double e = exp(__dmul_rn((double)__uint_as_float(bits), tau));
+                    const Bits bits = imp_at(f);
+                    if (bits == MASKED) continue;
+                    const double e = exp(__dmul_rn((double)imp_val(bits), tau));
                     const double prev = run;
                     run = __dadd_rn(run, e);
                     if (__ddiv_rn(run, total) > u) {
@@ -766,9 +966,9 @@ __device__ __forceinline__ void sdrf_loop_body(const SdrfDev& S, int loops, int 
                 if (near_boundary) {
                     long long cc = my_off;
                     for (long long f = f_lo; f < f_hi; ++f) {
-                        const uint32_t bits = S.imp[f];
-                        if (bits == IMP_MASKED) continue;
-                        S.pend[cc++] = (double)__uint_as_float(bits);
+                        const Bits bits = imp_at(f);
+                        if (bits == MASKED) continue;
+                        S.pend[cc++] = (double)imp_val(bits);
                     }
                     if (tid == 0) sh.status = DCR_SDRF_NEED_HOST;
                     __syncthreads();
@@ -779,7 +979,7 @@ __device__ __forceinline__ void sdrf_loop_body(const SdrfDev& S, int loops, int 
             if (tid == 0) {
                 const long long f = sh.chosen_flat;
                 const int ck = nbI((int)(f / n_j)), cl = nbJ((int)(f % n_j));
-                const bool swap = (MODE == LOOP_CLASSICAL) && ck > cl;           // sorted(...) (sdrf_no_cuda.py:37,50)
+                const bool swap = NX_LOOP && ck > cl;                            // sorted(...) (sdrf_no_cuda.py:37,50)
                 sh.k = swap ? cl : ck;
                 sh.l = swap ? ck : cl;
             }
@@ -790,11 +990,14 @@ __device__ __forceinline__ void sdrf_loop_body(const SdrfDev& S, int loops, int 
         SDRF_TICK(2);   // selection
         // ---- removal decision on the SAME C_t (:79-91) --------------------------------------------------
         if (tid == 0 && remove_edges && !sh.stop) {
-            // BFC: fp32 compare, torch casts the Python float (:83); classical: Python int > float (sdrf_no_cuda.py:62)
-            const bool above = (MODE == LOOP_CLASSICAL) ? ((double)sh.cmax > bound64) : (sh.cmax > bound32);
+            // BFC: fp32 compare, torch casts the Python float (:83); classical: Python int > float (sdrf_no_cuda.py:62);
+            // paper: Python float > float
+            bool above;
+            if constexpr (PAPER) above = sh.cmax_d > bound64;
+            else above = (MODE == LOOP_CLASSICAL) ? ((double)sh.cmax > bound64) : (sh.cmax > bound32);
             if (above) {
                 if (sh.have_max) sh.do_remove = (MODE == LOOP_CLASSICAL && sh.xr == sh.yr) ? 3 : 1;   // 3: the maximum is a loop edge
-                else if (MODE != LOOP_CLASSICAL && S.selfl[0]) sh.do_remove = 2;   // (0,0) fallback and G has the loop 0-0: it goes
+                else if (!NX_LOOP && S.selfl[0]) sh.do_remove = 2;   // (0,0) fallback and G has the loop 0-0: it goes
                 else sh.status = DCR_SDRF_REMOVE_NONEDGE;                // (0,0) fallback beat a negative bound
             } else if (!sh.can_add) {
                 sh.stop = 1;
@@ -819,6 +1022,7 @@ __device__ __forceinline__ void sdrf_loop_body(const SdrfDev& S, int loops, int 
             __syncthreads();
             SDRF_TICK(3);   // insert rows
             if constexpr (MODE == LOOP_DIRECTED) directed_mark_dirty(S, k, l, &dirty_count);
+            else if constexpr (PAPER) paper_mark_dirty(S, k, l, &dirty_count);
             else toggle_supports<MODE == LOOP_BFC>(S, g, k, l, +1, &dirty_count, &sh);
             SDRF_TICK(4);   // supports + dirty (add)
         }
@@ -841,6 +1045,7 @@ __device__ __forceinline__ void sdrf_loop_body(const SdrfDev& S, int loops, int 
         } else if (sh.do_remove) {                      // :84-88
             const int xr = sh.xr, yr = sh.yr;
             if constexpr (MODE == LOOP_DIRECTED) directed_mark_dirty(S, xr, yr, &dirty_count);
+            else if constexpr (PAPER) paper_mark_dirty(S, xr, yr, &dirty_count);
             else toggle_supports<MODE == LOOP_BFC>(S, g, xr, yr, -1, &dirty_count, &sh);
             row_delete(S, xr, yr, &sh);
             row_delete(S, L_ROW * S.n + yr, xr, &sh);
@@ -865,6 +1070,15 @@ __device__ __forceinline__ void sdrf_loop_body(const SdrfDev& S, int loops, int 
         for (int t = warp; t < nwk; t += SDRF_WARPS) {
             const int s = S.work[t];
             const int a = S.owner[s], b = S.col[s];
+            if constexpr (PAPER) {
+                const double c = paper_eval(PaperView{g, -1, -1}, a, b, lane);
+                if (lane == 0) {
+                    paper_put(S, s, c);
+                    paper_put(S, edge_slot(g, b, a), c);
+                    S.flag[s] = 0;
+                }
+                continue;
+            }
             float c;
             if constexpr (MODE == LOOP_DIRECTED) c = directed_entry_curvature(g, gin, a, b, lane).c32;
             else if constexpr (MODE == LOOP_CLASSICAL) c = classical_curvature(S, a, b, s);
@@ -948,6 +1162,8 @@ static LoopKernels loop_kernels(int mode) {
     case DCR_SDRF_MODE_BFC_DIRECTED:
         return {sdrf_init_curvature_kernel<LOOP_DIRECTED>, sdrf_loop_kernel<LOOP_DIRECTED>,
                 sdrf_batch_loop_kernel<LOOP_DIRECTED>};
+    case DCR_SDRF_MODE_BFC_PAPER:
+        return {sdrf_init_curvature_kernel<LOOP_PAPER>, sdrf_loop_kernel<LOOP_PAPER>, sdrf_batch_loop_kernel<LOOP_PAPER>};
     default:
         return {sdrf_init_curvature_kernel<LOOP_CLASSICAL>, sdrf_loop_kernel<LOOP_CLASSICAL>,
                 sdrf_batch_loop_kernel<LOOP_CLASSICAL>};
@@ -993,6 +1209,14 @@ __global__ void sdrf_export_rows_kernel(SdrfDev S, const int32_t* rowptr, int32_
         }
     }
 }
+__global__ void sdrf_export_c64_kernel(SdrfDev S, const int32_t* rowptr, double* c64) {
+    const int lane = threadIdx.x & 31;
+    const int warps = (gridDim.x * blockDim.x) >> 5;
+    for (int v = (blockIdx.x * blockDim.x + threadIdx.x) >> 5; v < S.n; v += warps) {
+        const int s = S.rstart[v], d = S.rlen[v], o = rowptr[v];
+        for (int t = lane; t < d; t += 32) c64[o + t] = paper_get(S, s + t);
+    }
+}
 __global__ void sdrf_copy_pending_kernel(const double* pend, double* out, long long n) {
     for (long long t = blockIdx.x * (long long)blockDim.x + threadIdx.x; t < n; t += (long long)gridDim.x * blockDim.x)
         out[t] = pend[t];
@@ -1022,8 +1246,9 @@ static int sdrf_create_impl(int n, int mode, const int32_t* rowptr_host, const i
                             const int32_t* in_rowptr_host, const int32_t* in_order_host, int64_t max_additions,
                             dcr_sdrf** out) {
     if (n <= 0 || !rowptr_host || !out) { set_error("dcr_sdrf_create: bad arguments"); return 1; }
-    if (mode < DCR_SDRF_MODE_BFC || mode > DCR_SDRF_MODE_HAANTJES) { set_error("dcr_sdrf_create: unknown mode"); return 1; }
+    if (mode < DCR_SDRF_MODE_BFC || mode > DCR_SDRF_MODE_BFC_PAPER) { set_error("dcr_sdrf_create: unknown mode"); return 1; }
     const bool directed = mode == DCR_SDRF_MODE_BFC_DIRECTED;
+    const bool paper = mode == DCR_SDRF_MODE_BFC_PAPER;
     if (directed && !in_rowptr_host) { set_error("dcr_sdrf_create: the directed mode needs the predecessor lists"); return 1; }
     const int rows = directed ? 2 * n : n;
     int64_t nnz = rowptr_host[n];             // (entries of the insertion-order lists; self entries are subtracted below)
@@ -1041,6 +1266,7 @@ static int sdrf_create_impl(int n, int mode, const int32_t* rowptr_host, const i
             int hits = 0;
             for (int t = 0; t < len; ++t) hits += src[t] == me;
             if (hits > 1) { set_error("dcr_sdrf_create: node %d lists itself more than once", me); return 1; }
+            if (hits && paper) { set_error("dcr_sdrf_create: node %d lists itself (the paper-flavour loop takes no self-loops)", me); return 1; }
             selfl[v] = hits;
             if (v < n) n_self += hits;                 // (counted once per node: the successor / neighbour rows)
             len -= hits;
@@ -1091,13 +1317,14 @@ static int sdrf_create_impl(int n, int mode, const int32_t* rowptr_host, const i
     s->n_self = n_self;
     SdrfDev& D = s->dev;
     D.n = n;
-    D.ctype = mode >= DCR_SDRF_MODE_1D ? mode - DCR_SDRF_MODE_1D : 0;
+    D.ctype = (mode >= DCR_SDRF_MODE_1D && mode <= DCR_SDRF_MODE_HAANTJES) ? mode - DCR_SDRF_MODE_1D : 0;
     D.cap_total = (int)cap_total;
     const int64_t row_cap_max = (int64_t)d1 + max_additions + 2;
     D.row_cap_max = (int)std::min<int64_t>(row_cap_max, 0x7ffffff0LL);
     // candidate matrix: (deg x + 1)(deg y + 1) <= the product of the two longest rows after all additions
     D.imp_cap = std::min<int64_t>(((int64_t)d1 + max_additions + 2) * ((int64_t)d2 + max_additions + 2), (int64_t)1 << 28);
-    // dirty pairs of one iteration: two toggles, each at most the entries at four rows + the closing edges
+    // dirty pairs of one iteration: two toggles, each at most the entries at four rows + the closing edges (paper loop:
+    // the entries at k and l + at most one pair per directed entry, so 2 nnz per toggle, paper_mark_dirty)
     D.dirty_cap = (int)std::min<int64_t>(4 * (nnz + 2 * max_additions) + 4096, 0x3ffffff0LL);
     size_t bytes = 0;
     auto add = [&](size_t count, size_t elem) { bytes += (count * elem + 255) / 256 * 256; };
@@ -1105,7 +1332,7 @@ static int sdrf_create_impl(int n, int mode, const int32_t* rowptr_host, const i
     for (int i = 0; i < 6; ++i) add(cap_total, 4);           // col ord supp c32 owner flag
     add(8, 4);                                               // scalars
     for (int i = 0; i < 4; ++i) add(D.row_cap_max, 4);       // base1 base2 posI posJ
-    add(D.imp_cap, 4); add(D.imp_cap, 8);                    // imp, pend
+    add(D.imp_cap, paper ? 8 : 4); add(D.imp_cap, 8);        // imp, pend
     add((size_t)2 * D.dirty_cap, 4); add(D.dirty_cap, 4);    // dirty, work
     add(D.row_cap_max, 4);                                   // wlist
     cudaError_t e = cudaMalloc(&s->slab, bytes);
@@ -1119,7 +1346,7 @@ static int sdrf_create_impl(int n, int mode, const int32_t* rowptr_host, const i
     D.scalars = carve<int32_t>(p, 8);
     D.base1 = carve<int32_t>(p, D.row_cap_max); D.base2 = carve<int32_t>(p, D.row_cap_max);
     D.posI = carve<int32_t>(p, D.row_cap_max); D.posJ = carve<int32_t>(p, D.row_cap_max);
-    D.imp = carve<uint32_t>(p, D.imp_cap); D.pend = carve<double>(p, D.imp_cap);
+    D.imp = carve<uint32_t>(p, (paper ? 2 : 1) * D.imp_cap); D.pend = carve<double>(p, D.imp_cap);
     D.dirty = carve<int32_t>(p, (size_t)2 * D.dirty_cap); D.work = carve<int32_t>(p, D.dirty_cap);
     D.wlist = carve<int32_t>(p, D.row_cap_max);
 
@@ -1146,7 +1373,7 @@ static int sdrf_create_impl(int n, int mode, const int32_t* rowptr_host, const i
     SDRF_TRY(cudaMemcpy(D.scalars, scal, sizeof(scal), cudaMemcpyHostToDevice));
     if (sum_cap > 0) {
         const int ctas = (int)std::min<int64_t>((sum_cap + 7) / 8, (int64_t)sm_count() * 8);
-        if (!directed) sdrf_init_support_kernel<<<ctas, 256>>>(D, (int)sum_cap);
+        if (!directed && !paper) sdrf_init_support_kernel<<<ctas, 256>>>(D, (int)sum_cap);   // (paper: no supports)
         loop_kernels(mode).init<<<ctas, 256>>>(D, (int)sum_cap);
         SDRF_TRY(cudaGetLastError());
     }
@@ -1278,6 +1505,18 @@ extern "C" int dcr_sdrf_export_order(dcr_sdrf* s, int32_t* rowptr_order, int32_t
     DCR_LAUNCH_CHECK();
     const int ctas = std::max(1, std::min((s->dev.n + 7) / 8, sm_count() * 8));
     sdrf_export_order_kernel<<<ctas, 256, 0, st>>>(s->dev, rowptr_order, order_out);
+    DCR_LAUNCH_CHECK();
+    return 0;
+}
+
+extern "C" int dcr_sdrf_export_c64(dcr_sdrf* s, int32_t* rowptr, double* c64_sorted, void* stream) {
+    if (!s || !rowptr || !c64_sorted) { set_error("dcr_sdrf_export_c64: bad arguments"); return 1; }
+    if (s->mode != DCR_SDRF_MODE_BFC_PAPER) { set_error("dcr_sdrf_export_c64: only DCR_SDRF_MODE_BFC_PAPER keeps fp64 values"); return 1; }
+    cudaStream_t st = (cudaStream_t)stream;
+    sdrf_export_rowptr_kernel<<<1, SDRF_THREADS, 0, st>>>(s->dev, rowptr, 0);
+    DCR_LAUNCH_CHECK();
+    const int ctas = std::max(1, std::min((s->dev.n + 7) / 8, sm_count() * 8));
+    sdrf_export_c64_kernel<<<ctas, 256, 0, st>>>(s->dev, rowptr, c64_sorted);
     DCR_LAUNCH_CHECK();
     return 0;
 }

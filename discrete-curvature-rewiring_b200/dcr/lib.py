@@ -22,7 +22,7 @@ class SdrfBatchRun(C.Structure):
 # status codes of include/dcr.h
 SDRF_OK, SDRF_NEED_HOST, SDRF_PROB_NAN, SDRF_PROB_SUM, SDRF_REMOVE_NONEDGE, SDRF_NO_UNIFORM, SDRF_ARENA_FULL, \
     SDRF_TOO_MANY_CANDIDATES, SDRF_EMPTY_GRAPH = range(9)
-SDRF_MODE_BFC, SDRF_MODE_BFC_DIRECTED, SDRF_MODE_1D, SDRF_MODE_AUGMENTED, SDRF_MODE_HAANTJES = range(5)
+SDRF_MODE_BFC, SDRF_MODE_BFC_DIRECTED, SDRF_MODE_1D, SDRF_MODE_AUGMENTED, SDRF_MODE_HAANTJES, SDRF_MODE_BFC_PAPER = range(6)
 SDRF_LOG_INTS = 8
 
 _P = C.c_void_p
@@ -80,6 +80,7 @@ SIGNATURES = {
     "dcr_sdrf_nnz": (_L, [_P]),
     "dcr_sdrf_export": (_I, [_P, _P, _P, _P, _P, _P, _P]),
     "dcr_sdrf_export_order": (_I, [_P, _P, _P, _P]),
+    "dcr_sdrf_export_c64": (_I, [_P, _P, _P, _P]),
 }
 
 _lib = None

@@ -105,10 +105,22 @@ class SdrfState:
         return int(self.lib.dcr_sdrf_nnz(self.handle))
 
     def export(self, with_curvature: bool = False):
-        """Current graph: ``(rowptr, order)`` numpy (networkx order); with curvature also sorted col / c32 / tri."""
+        """Current graph: ``(rowptr, order)`` numpy (networkx order); with curvature also sorted col / c32 / tri.  The
+        paper-flavour mode (``L.SDRF_MODE_BFC_PAPER``) keeps no fp32 curvature and no supports: its curvature is the fp64
+        ``bfc_edge`` value of every entry (sorted order) and ``tri`` is ``None``."""
         nnz = self.nnz()
         dev = self.device
         rowptr = torch.empty(self.n + 1, dtype=torch.int32, device=dev)
+        if with_curvature and self.mode == L.SDRF_MODE_BFC_PAPER:
+            order = torch.empty(max(nnz, 1), dtype=torch.int32, device=dev)
+            col = torch.empty(max(nnz, 1), dtype=torch.int32, device=dev)
+            c64 = torch.empty(max(nnz, 1), dtype=torch.float64, device=dev)
+            L.check(self.lib.dcr_sdrf_export(self.handle, rowptr.data_ptr(), order.data_ptr(), col.data_ptr(), 0, 0,
+                                             L.current_stream()), "dcr_sdrf_export")
+            L.check(self.lib.dcr_sdrf_export_c64(self.handle, rowptr.data_ptr(), c64.data_ptr(), L.current_stream()),
+                    "dcr_sdrf_export_c64")
+            return (rowptr.cpu().numpy(), order[:nnz].cpu().numpy(), col[:nnz].cpu().numpy(), c64[:nnz].cpu().numpy(),
+                    None)
         if self.n_self and not with_curvature:
             # nodes that list themselves (self-loops of G): the insertion-order rows are longer than the adjacency rows
             order = torch.empty(max(nnz + self.n_self, 1), dtype=torch.int32, device=dev)
@@ -155,6 +167,16 @@ def _raise_for_status(status: int):
 CLASSICAL_MODES = {"1d": L.SDRF_MODE_1D, "augmented": L.SDRF_MODE_AUGMENTED, "haantjes": L.SDRF_MODE_HAANTJES}
 
 
+def _paper_order(edge_index, num_nodes: int):
+    """``classical_order`` for ``curv_type='bfc_paper'``: bfc_naive.bfc_edge counts a node's degree and neighbours the
+    networkx way, which gives a self-loop no meaning in the curvature, so an input with one is refused."""
+    rowptr, order = G.classical_order(edge_index, num_nodes, keep_self_loops=True)
+    rows = np.repeat(np.arange(rowptr.size - 1), np.diff(rowptr.astype(np.int64)))
+    if np.any(order == rows):
+        raise NotImplementedError("curv_type='bfc_paper' does not take graphs with self-loops")
+    return rowptr, order
+
+
 def _loop_mode(curv_type: str, is_undirected: bool):
     """``(L.SDRF_MODE_*, order)`` of the loop that runs ``curv_type``: ``order(edge_index, num_nodes)`` lists the input
     in the insertion order that loop starts from (``_new_state`` takes its result)."""
@@ -164,6 +186,10 @@ def _loop_mode(curv_type: str, is_undirected: bool):
         return L.SDRF_MODE_BFC_DIRECTED, lambda ei, n: G.digraph_order(ei, n, keep_self_loops=True)
     if curv_type in CLASSICAL_MODES:
         return CLASSICAL_MODES[curv_type], lambda ei, n: G.classical_order(ei, n, keep_self_loops=True)
+    if curv_type == "bfc_paper":
+        if not is_undirected:
+            raise NotImplementedError("curv_type='bfc_paper' runs on undirected graphs only")
+        return L.SDRF_MODE_BFC_PAPER, _paper_order
     raise Exception(f"Method {curv_type} not available.")    # classical_curvatures.py:27-28
 
 
@@ -189,6 +215,8 @@ def sdrf(edge_index, num_nodes: int, loops: int, remove_edges: bool, removal_bou
     ``curv_type='bfc'``: ``sdrf_cuda_bfc`` (rewiring/sdrf_cuda_bfc.py:14-93), undirected or — ``is_undirected=False`` —
     on the ``DiGraph`` of the input with single directed entries added / removed (:47-49, :72-73, :87-88).
     ``curv_type`` in ``'1d' | 'augmented' | 'haantjes'``: ``sdrf_no_cuda`` (rewiring/sdrf_no_cuda.py:9-68).
+    ``curv_type='bfc_paper'``: ``sdrf_no_cuda``'s loop with the paper-flavour curvature ``bfc_naive.bfc_edge``
+    (curvature/bfc_naive.py:7-40) in fp64; undirected inputs without self-loops (``NotImplementedError`` otherwise).
 
     ``uniforms``: the doubles ``np.random`` would produce (one per iteration that has candidates).  When omitted
     they are taken from numpy's global legacy generator exactly as the reference consumes it: the global state

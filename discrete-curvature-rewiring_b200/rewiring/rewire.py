@@ -5,6 +5,8 @@
 * ``'bfc'``                              -> the device-resident BFC loop (``rewiring.sdrf_cuda_bfc``), undirected
 * ``'1d'`` / ``'augmented'`` / ``'haantjes'`` -> the classical-curvature loop on the same device kernel
   (``rewiring.sdrf_no_cuda``)
+* ``'bfc_paper'``                        -> the same loop with the paper-flavour curvature ``bfc_naive.bfc_edge``
+  (``rewiring.sdrf_no_cuda``; no self-loops)
 * ``None``                               -> no rewiring: the input's ``edge_index`` comes back unchanged
 
 Every flavour removes edges (``remove_edges=True``), as the reference's dispatcher does.

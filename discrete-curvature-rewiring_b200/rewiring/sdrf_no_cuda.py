@@ -6,6 +6,10 @@ on the networkx graph (:40-45).  Here the loop runs inside the same persistent s
 (csrc/dcr_sdrf.cu, ``LOOP_CLASSICAL``): degrees and common-neighbour counts are maintained incrementally, the three
 curvatures ('1d', 'augmented', 'haantjes') are integer functions of them, ``min`` / ``max`` over ``G.edges`` keep the
 reference's first-in-iteration-order tie-break, and the candidate improvements come in closed form.
+
+``curv_type='bfc_paper'`` (an extension: the reference raises ``Method … not available.``) runs the same loop with
+``curvature.bfc_naive.bfc_edge``, the paper-flavour Balanced Forman curvature, as ``compute_curvature_edge`` — the SDRF of
+the paper.  Values, improvements and the removal comparison are fp64; inputs with self-loops raise ``NotImplementedError``.
 """
 import torch
 
@@ -20,7 +24,7 @@ def sdrf_no_cuda(data, curv_type, loops, remove_edges, removal_bound, tau, *, un
     """
     Perform SDRF graph rewiring using the given classical discrete curvature type.
     :param data: data to be rewired (undirected by default in this work).
-    :param curv_type: type of discrete curvature used for the rewiring ('1d', 'augmented' or 'haantjes').
+    :param curv_type: type of discrete curvature used for the rewiring ('1d', 'augmented', 'haantjes' or 'bfc_paper').
     :param loops: number of edge addition/deletion iterations.
     :param remove_edges: whether to delete highly curved edges each iteration to compensate for the addition.
     :param removal_bound: curvature lower bound of deleting edges (delete edges only with higher curvature).

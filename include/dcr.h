@@ -46,6 +46,7 @@ extern "C" {
 #define DCR_SDRF_MODE_1D 2           /* sdrf_no_cuda(curv_type='1d')             rewiring/sdrf_no_cuda.py:9-68          */
 #define DCR_SDRF_MODE_AUGMENTED 3    /* sdrf_no_cuda(curv_type='augmented')      curvature/classical_curvatures.py:17-21 */
 #define DCR_SDRF_MODE_HAANTJES 4     /* sdrf_no_cuda(curv_type='haantjes')       curvature/classical_curvatures.py:22-26 */
+#define DCR_SDRF_MODE_BFC_PAPER 5    /* sdrf_no_cuda's loop with bfc_naive.bfc_edge as the curvature (curvature/bfc_naive.py:7-40) */
 
 const char* dcr_last_error(void);
 int dcr_version(void);
@@ -279,7 +280,11 @@ int dcr_sdrf_create(int n, const int32_t* rowptr_host, const int32_t* order_host
  * to_networkx(data, to_undirected=True)); in_* are ignored.  dcr_sdrf_run's log record then holds the (x, y) of
  * min(G.edges) (x <= y), the sorted (k, l) that was added and the removed edge; removal_bound is compared in fp64.
  * Here a node that lists itself has a LOOP EDGE (u,u) of G.edges with a curvature of its own (degree + 2, the node its
- * own neighbour): it can be the minimum edge (x == y) and the removed edge. */
+ * own neighbour): it can be the minimum edge (x == y) and the removed edge.
+ * BFC_PAPER: the same loop, order and log as 1D / AUGMENTED / HAANTJES with the paper-flavour curvature of
+ * dcr_bfc_paper (fp64, bit-identical to bfc_naive.bfc_edge; 0 where deg_min == 1) as the edge value; improvements and
+ * the draw are fp64.  Self entries have no meaning for bfc_edge: a list that contains its own node is rejected
+ * (status 1). */
 int dcr_sdrf_create_mode(int n, int mode, const int32_t* rowptr_host, const int32_t* order_host,
                          const int32_t* in_rowptr_host, const int32_t* in_order_host, int64_t max_additions,
                          dcr_sdrf** out);
@@ -309,7 +314,8 @@ typedef struct dcr_sdrf_batch_run {      /* one run of dcr_sdrf_run_batch; point
 int64_t dcr_sdrf_batch_workspace_bytes(int count);
 int dcr_sdrf_run_batch(const dcr_sdrf_batch_run* runs, int count, int remove_edges, double guard,
                        void* workspace, int64_t workspace_bytes, void* stream);
-/* Improvements (fp64 of the fp32 differences, candidate order) of the pending iteration after NEED_HOST. */
+/* Improvements (candidate order) of the pending iteration after NEED_HOST: fp64 of the fp32 differences, or the fp64
+ * differences themselves for DCR_SDRF_MODE_BFC_PAPER. */
 int dcr_sdrf_pending_improvements(dcr_sdrf* s, double* out, int64_t capacity, void* stream);
 /* Current number of directed entries (synchronises). */
 int64_t dcr_sdrf_nnz(dcr_sdrf* s);
@@ -321,6 +327,11 @@ int dcr_sdrf_export(dcr_sdrf* s, int32_t* rowptr, int32_t* order_out, int32_t* c
 /* Insertion-order rows INCLUDING the self entries (see dcr_sdrf_create): rowptr_order[n+1] and order_out[rowptr_order[n]]
  * (at most nnz + n entries).  dcr_sdrf_export refuses order_out for a state that has self entries. */
 int dcr_sdrf_export_order(dcr_sdrf* s, int32_t* rowptr_order, int32_t* order_out, void* stream);
+
+/* DCR_SDRF_MODE_BFC_PAPER states only: rowptr[n+1] and the fp64 paper-flavour curvature of every directed entry in
+ * SORTED order per row (the layout of dcr_sdrf_export's colidx_sorted / c32_sorted).  That mode keeps no fp32 curvature
+ * and no supports. */
+int dcr_sdrf_export_c64(dcr_sdrf* s, int32_t* rowptr, double* c64_sorted, void* stream);
 
 #ifdef __cplusplus
 }

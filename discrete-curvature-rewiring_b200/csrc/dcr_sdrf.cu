@@ -83,7 +83,7 @@ struct SdrfDev {
                           //  entry's fp64 paper-flavour value, so every arena edit moves it unchanged; see paper_get)
     int32_t* owner;       // arena: row id of the slot, -1 = free
     int32_t* flag;        // arena: dedupe flags for the refresh
-    int32_t* scalars;     // [0] arena_top, [1] nnz
+    int32_t* scalars;     // [0] arena_top, [1] nnz, [2] add edits applied, [3] max_additions (their limit)
     int32_t* base1; int32_t* base2; int32_t* posI; int32_t* posJ;   // score scratch [row_cap_max]
     uint32_t* imp;        // improvement matrix (fp32 bits; LOOP_PAPER: fp64 bits, two words per cell)
     double* pend;         // compact improvements of a pending iteration
@@ -672,6 +672,76 @@ __device__ __forceinline__ double val_min(double a, double b) { return fmin(a, b
 __device__ __forceinline__ double val_max(double a, double b) { return fmax(a, b); }
 
 // ------------------------------------------------------------------------------------------------------------
+// one edge toggle, shared by the loop (step 4 / 5) and the edit kernel
+// ------------------------------------------------------------------------------------------------------------
+// G.add_edge(k, l) on the arena (the edge must be absent): both rows append in insertion order (directed: the
+// successor row of k and the predecessor row of l); false when the arena is full
+template <int MODE>
+__device__ __forceinline__ bool edge_insert(const SdrfDev& S, int k, int l) {
+    constexpr int L_ROW = (MODE == LOOP_DIRECTED);  // directed: the mirror entry lives in the predecessor rows
+    bool ok = row_insert(S, k, l);
+    ok = ok && row_insert(S, L_ROW * S.n + l, k);
+    if (!ok) return false;
+    if (threadIdx.x == 0) S.scalars[1] += L_ROW ? 1 : 2;
+    __syncthreads();
+    return true;
+}
+// G.remove_edge(k, l) on the arena (the edge must be present)
+template <int MODE>
+__device__ __forceinline__ void edge_delete(const SdrfDev& S, int k, int l, LoopShared* sh) {
+    constexpr int L_ROW = (MODE == LOOP_DIRECTED);
+    row_delete(S, k, l, sh);
+    row_delete(S, L_ROW * S.n + l, k, sh);
+    if (threadIdx.x == 0) S.scalars[1] -= L_ROW ? 1 : 2;
+    __syncthreads();
+}
+// the flavour's support update and dirty rule for toggling {k,l}; call while the edge is PRESENT (after the insertion,
+// before the deletion); delta = +1 for an insertion, -1 for a deletion
+template <int MODE>
+__device__ __forceinline__ void toggle_mark(const SdrfDev& S, const GraphView& g, int k, int l, int delta,
+                                            int* dirty_count, LoopShared* sh) {
+    if constexpr (MODE == LOOP_DIRECTED) directed_mark_dirty(S, k, l, dirty_count);
+    else if constexpr (MODE == LOOP_PAPER) paper_mark_dirty(S, k, l, dirty_count);
+    else toggle_supports<MODE == LOOP_BFC>(S, g, k, l, delta, dirty_count, sh);
+}
+// Refresh the curvature of the first nd dirty pairs (nd <= dirty_cap): dedupe them into slots (S.work, counted in
+// *work_count, which the caller zeroed) and re-evaluate each slot once, one warp per slot.
+template <int MODE>
+__device__ __forceinline__ void refresh_dirty(const SdrfDev& S, const GraphView& g, const GraphView& gin, int nd,
+                                              int* work_count) {
+    const int tid = threadIdx.x, lane = tid & 31, warp = tid >> 5;
+    for (int t = tid; t < nd; t += SDRF_THREADS) {
+        const int a = S.dirty[2 * t], b = S.dirty[2 * t + 1];
+        const int s = edge_slot(g, a, b);
+        if (s >= 0 && atomicExch(&S.flag[s], 1) == 0) S.work[atomicAdd(work_count, 1)] = s;
+    }
+    __syncthreads();
+    const int nwk = *work_count;
+    for (int t = warp; t < nwk; t += SDRF_WARPS) {
+        const int s = S.work[t];
+        const int a = S.owner[s], b = S.col[s];
+        if constexpr (MODE == LOOP_PAPER) {
+            const double c = paper_eval(PaperView{g, -1, -1}, a, b, lane);
+            if (lane == 0) {
+                paper_put(S, s, c);
+                paper_put(S, edge_slot(g, b, a), c);
+                S.flag[s] = 0;
+            }
+            continue;
+        }
+        float c;
+        if constexpr (MODE == LOOP_DIRECTED) c = directed_entry_curvature(g, gin, a, b, lane).c32;
+        else if constexpr (MODE == LOOP_CLASSICAL) c = classical_curvature(S, a, b, s);
+        else c = entry_curvature(S, a, b, s, lane);
+        if (lane == 0) {
+            S.c32[s] = c;
+            if (MODE != LOOP_DIRECTED) S.c32[edge_slot(g, b, a)] = c;   // symmetric A: C[b,a] == C[a,b] bit for bit
+            S.flag[s] = 0;
+        }
+    }
+}
+
+// ------------------------------------------------------------------------------------------------------------
 // the loop
 // ------------------------------------------------------------------------------------------------------------
 // One run of the loop on the calling CTA.  Block-uniform arguments only; nothing here reads blockIdx or gridDim, so the
@@ -697,7 +767,7 @@ __device__ __forceinline__ void sdrf_loop_body(const SdrfDev& S, int loops, int 
     __shared__ std::conditional_t<PAPER, LoopSharedPaper, LoopShared> sh;
     __shared__ DirScoreShared dsh;
     __shared__ int dirty_count, work_count, dred[2];
-    const int tid = threadIdx.x, lane = tid & 31, warp = tid >> 5;
+    const int tid = threadIdx.x;
     GraphView g{S.rstart, S.rlen, S.col};                       // undirected adjacency / successors
     GraphView gin{S.rstart + S.n, S.rlen + S.n, S.col};         // predecessors (directed loop only)
     ScoreScratch sc{S.base1, S.base2, S.posI, S.posJ};
@@ -1009,21 +1079,14 @@ __device__ __forceinline__ void sdrf_loop_body(const SdrfDev& S, int loops, int 
         if (tid == 0) { dirty_count = 0; work_count = 0; }
         __syncthreads();
         const int k = sh.k, l = sh.l;
-        constexpr int L_ROW = (MODE == LOOP_DIRECTED);  // directed: the mirror entry lives in the predecessor rows
         if (k >= 0) {                                   // :69-73
-            bool ok = row_insert(S, k, l);
-            ok = ok && row_insert(S, L_ROW * S.n + l, k);
-            if (!ok) {
+            if (!edge_insert<MODE>(S, k, l)) {
                 if (tid == 0) sh.status = DCR_SDRF_ARENA_FULL;
                 __syncthreads();
                 break;
             }
-            if (tid == 0) S.scalars[1] += L_ROW ? 1 : 2;
-            __syncthreads();
             SDRF_TICK(3);   // insert rows
-            if constexpr (MODE == LOOP_DIRECTED) directed_mark_dirty(S, k, l, &dirty_count);
-            else if constexpr (PAPER) paper_mark_dirty(S, k, l, &dirty_count);
-            else toggle_supports<MODE == LOOP_BFC>(S, g, k, l, +1, &dirty_count, &sh);
+            toggle_mark<MODE>(S, g, k, l, +1, &dirty_count, &sh);
             SDRF_TICK(4);   // supports + dirty (add)
         }
         if (sh.do_remove == 2) {                        // G.remove_edge(0, 0): only the insertion-order rows change (A[0,0] = 0 already)
@@ -1044,13 +1107,8 @@ __device__ __forceinline__ void sdrf_loop_body(const SdrfDev& S, int loops, int 
             __syncthreads();
         } else if (sh.do_remove) {                      // :84-88
             const int xr = sh.xr, yr = sh.yr;
-            if constexpr (MODE == LOOP_DIRECTED) directed_mark_dirty(S, xr, yr, &dirty_count);
-            else if constexpr (PAPER) paper_mark_dirty(S, xr, yr, &dirty_count);
-            else toggle_supports<MODE == LOOP_BFC>(S, g, xr, yr, -1, &dirty_count, &sh);
-            row_delete(S, xr, yr, &sh);
-            row_delete(S, L_ROW * S.n + yr, xr, &sh);
-            if (tid == 0) S.scalars[1] -= L_ROW ? 1 : 2;
-            __syncthreads();
+            toggle_mark<MODE>(S, g, xr, yr, -1, &dirty_count, &sh);
+            edge_delete<MODE>(S, xr, yr, &sh);
         }
         SDRF_TICK(5);   // removal: supports + delete rows
         // ---- 5. refresh the curvature of the dirty edges ----------------------------------------------
@@ -1060,35 +1118,7 @@ __device__ __forceinline__ void sdrf_loop_body(const SdrfDev& S, int loops, int 
             __syncthreads();
             break;
         }
-        for (int t = tid; t < nd; t += SDRF_THREADS) {
-            const int a = S.dirty[2 * t], b = S.dirty[2 * t + 1];
-            const int s = edge_slot(g, a, b);
-            if (s >= 0 && atomicExch(&S.flag[s], 1) == 0) S.work[atomicAdd(&work_count, 1)] = s;
-        }
-        __syncthreads();
-        const int nwk = work_count;
-        for (int t = warp; t < nwk; t += SDRF_WARPS) {
-            const int s = S.work[t];
-            const int a = S.owner[s], b = S.col[s];
-            if constexpr (PAPER) {
-                const double c = paper_eval(PaperView{g, -1, -1}, a, b, lane);
-                if (lane == 0) {
-                    paper_put(S, s, c);
-                    paper_put(S, edge_slot(g, b, a), c);
-                    S.flag[s] = 0;
-                }
-                continue;
-            }
-            float c;
-            if constexpr (MODE == LOOP_DIRECTED) c = directed_entry_curvature(g, gin, a, b, lane).c32;
-            else if constexpr (MODE == LOOP_CLASSICAL) c = classical_curvature(S, a, b, s);
-            else c = entry_curvature(S, a, b, s, lane);
-            if (lane == 0) {
-                S.c32[s] = c;
-                if (MODE != LOOP_DIRECTED) S.c32[edge_slot(g, b, a)] = c;   // symmetric A: C[b,a] == C[a,b] bit for bit
-                S.flag[s] = 0;
-            }
-        }
+        refresh_dirty<MODE>(S, g, gin, nd, &work_count);
         SDRF_TICK(6);   // refresh
         // ---- 6. log ------------------------------------------------------------------------------------
         if (tid == 0) {
@@ -1149,24 +1179,77 @@ sdrf_batch_loop_kernel(const SdrfBatchDesc* __restrict__ descs, int remove_edges
                                 d.n_uniforms, d.forced_choice, guard, d.log, d.result);
 }
 
+// Caller edits (dcr_sdrf_edit): edits[3t .. 3t+2] = (op, u, v), op 1 = G.add_edge(u, v), 0 = G.remove_edge(u, v),
+// applied in order on one CTA.  Each edit is the loop's own toggle (edge_insert / edge_delete, toggle_mark) followed by
+// the refresh of its dirty edges before the next edit: one toggle per refresh keeps the dirty list within dirty_cap.
+// An add of a present edge changes nothing (networkx keeps its position).  The kernel stops BEFORE an edit with
+// u == v or an id outside [0, n) (BAD_EDIT), a remove of an absent edge (REMOVE_NONEDGE) or an add beyond the
+// additions budget (ARENA_FULL; scalars[2] counts the add edits, no-op adds included, scalars[3] is max_additions).
+template <int MODE>
+__global__ void __launch_bounds__(SDRF_THREADS, 1)
+sdrf_edit_kernel(SdrfDev S, const int32_t* __restrict__ edits, long long count, dcr_sdrf_result* __restrict__ result) {
+    __shared__ LoopShared sh;
+    __shared__ int dirty_count, work_count;
+    const GraphView g{S.rstart, S.rlen, S.col};                 // undirected adjacency / successors
+    const GraphView gin{S.rstart + S.n, S.rlen + S.n, S.col};   // predecessors (directed flavour only)
+    int adds = S.scalars[2];                                    // block-uniform copies of the budget words
+    const int add_limit = S.scalars[3];
+    int status = DCR_SDRF_OK, u = -1, v = -1;
+    long long t = 0;
+    for (; t < count; ++t) {
+        const int op = edits[3 * t];
+        u = edits[3 * t + 1];
+        v = edits[3 * t + 2];
+        if ((op != 0 && op != 1) || u == v || u < 0 || u >= S.n || v < 0 || v >= S.n) { status = DCR_SDRF_BAD_EDIT; break; }
+        const bool present = edge_slot(g, u, v) >= 0;
+        if (op == 1 && adds >= add_limit) { status = DCR_SDRF_ARENA_FULL; break; }
+        if (op == 0 && !present) { status = DCR_SDRF_REMOVE_NONEDGE; break; }
+        adds += op;
+        if (op == 1 && present) continue;
+        if (threadIdx.x == 0) { dirty_count = 0; work_count = 0; }
+        __syncthreads();
+        if (op == 1) {
+            if (!edge_insert<MODE>(S, u, v)) { status = DCR_SDRF_ARENA_FULL; break; }   // (not within the budget)
+            toggle_mark<MODE>(S, g, u, v, +1, &dirty_count, &sh);
+        } else {
+            toggle_mark<MODE>(S, g, u, v, -1, &dirty_count, &sh);
+            edge_delete<MODE>(S, u, v, &sh);
+        }
+        if (dirty_count > S.dirty_cap) { status = DCR_SDRF_ARENA_FULL; ++t; break; }   // (not within the budget)
+        refresh_dirty<MODE>(S, g, gin, dirty_count, &work_count);
+        __syncthreads();
+    }
+    if (threadIdx.x == 0) {
+        S.scalars[2] = adds;
+        result->status = status;
+        result->iterations_done = (int)t;
+        result->draws_used = 0;
+        result->stopped = 0;
+        result->pending_n = 0;
+        result->pending_x = status == DCR_SDRF_OK ? -1 : u;
+        result->pending_y = status == DCR_SDRF_OK ? -1 : v;
+        result->reserved = 0;
+    }
+}
+
 // the kernels of the loop flavour that runs DCR_SDRF_MODE_* `mode`
 struct LoopKernels {
     decltype(&sdrf_init_curvature_kernel<LOOP_BFC>) init;
     decltype(&sdrf_loop_kernel<LOOP_BFC>) single;
     decltype(&sdrf_batch_loop_kernel<LOOP_BFC>) batch;
+    decltype(&sdrf_edit_kernel<LOOP_BFC>) edit;
 };
+template <int MODE>
+static LoopKernels loop_kernels_of() {
+    return {sdrf_init_curvature_kernel<MODE>, sdrf_loop_kernel<MODE>, sdrf_batch_loop_kernel<MODE>,
+            sdrf_edit_kernel<MODE>};
+}
 static LoopKernels loop_kernels(int mode) {
     switch (mode) {
-    case DCR_SDRF_MODE_BFC:
-        return {sdrf_init_curvature_kernel<LOOP_BFC>, sdrf_loop_kernel<LOOP_BFC>, sdrf_batch_loop_kernel<LOOP_BFC>};
-    case DCR_SDRF_MODE_BFC_DIRECTED:
-        return {sdrf_init_curvature_kernel<LOOP_DIRECTED>, sdrf_loop_kernel<LOOP_DIRECTED>,
-                sdrf_batch_loop_kernel<LOOP_DIRECTED>};
-    case DCR_SDRF_MODE_BFC_PAPER:
-        return {sdrf_init_curvature_kernel<LOOP_PAPER>, sdrf_loop_kernel<LOOP_PAPER>, sdrf_batch_loop_kernel<LOOP_PAPER>};
-    default:
-        return {sdrf_init_curvature_kernel<LOOP_CLASSICAL>, sdrf_loop_kernel<LOOP_CLASSICAL>,
-                sdrf_batch_loop_kernel<LOOP_CLASSICAL>};
+    case DCR_SDRF_MODE_BFC: return loop_kernels_of<LOOP_BFC>();
+    case DCR_SDRF_MODE_BFC_DIRECTED: return loop_kernels_of<LOOP_DIRECTED>();
+    case DCR_SDRF_MODE_BFC_PAPER: return loop_kernels_of<LOOP_PAPER>();
+    default: return loop_kernels_of<LOOP_CLASSICAL>();
     }
 }
 
@@ -1369,7 +1452,8 @@ static int sdrf_create_impl(int n, int mode, const int32_t* rowptr_host, const i
         SDRF_TRY(cudaMemcpy(D.ord, ord.data(), sum_cap * 4, cudaMemcpyHostToDevice));
         SDRF_TRY(cudaMemcpy(D.owner, owner.data(), sum_cap * 4, cudaMemcpyHostToDevice));
     }
-    int32_t scal[8] = {(int32_t)sum_cap, (int32_t)nnz, 0, 0, 0, 0, 0, 0};
+    // [2] add edits so far, [3] their limit (dcr_sdrf_edit)
+    int32_t scal[8] = {(int32_t)sum_cap, (int32_t)nnz, 0, (int32_t)std::min<int64_t>(max_additions, 0x7fffffff), 0, 0, 0, 0};
     SDRF_TRY(cudaMemcpy(D.scalars, scal, sizeof(scal), cudaMemcpyHostToDevice));
     if (sum_cap > 0) {
         const int ctas = (int)std::min<int64_t>((sum_cap + 7) / 8, (int64_t)sm_count() * 8);
@@ -1408,6 +1492,13 @@ extern "C" int dcr_sdrf_run(dcr_sdrf* s, int loops, int remove_edges, double rem
     loop_kernels(s->mode).single<<<1, SDRF_THREADS, 0, (cudaStream_t)stream>>>(
         s->dev, loops, remove_edges, (float)removal_bound, removal_bound, tau, tau_inf, uniforms, (long long)n_uniforms,
         forced_choice, guard, log, result);
+    DCR_LAUNCH_CHECK();
+    return 0;
+}
+
+extern "C" int dcr_sdrf_edit(dcr_sdrf* s, const int32_t* edits, int64_t count, dcr_sdrf_result* result, void* stream) {
+    if (!s || !result || count < 0 || (count > 0 && !edits)) { set_error("dcr_sdrf_edit: bad arguments"); return 1; }
+    loop_kernels(s->mode).edit<<<1, SDRF_THREADS, 0, (cudaStream_t)stream>>>(s->dev, edits, (long long)count, result);
     DCR_LAUNCH_CHECK();
     return 0;
 }

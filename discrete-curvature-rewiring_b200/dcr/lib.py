@@ -21,7 +21,7 @@ class SdrfBatchRun(C.Structure):
 
 # status codes of include/dcr.h
 SDRF_OK, SDRF_NEED_HOST, SDRF_PROB_NAN, SDRF_PROB_SUM, SDRF_REMOVE_NONEDGE, SDRF_NO_UNIFORM, SDRF_ARENA_FULL, \
-    SDRF_TOO_MANY_CANDIDATES, SDRF_EMPTY_GRAPH = range(9)
+    SDRF_TOO_MANY_CANDIDATES, SDRF_EMPTY_GRAPH, SDRF_BAD_EDIT = range(10)
 SDRF_MODE_BFC, SDRF_MODE_BFC_DIRECTED, SDRF_MODE_1D, SDRF_MODE_AUGMENTED, SDRF_MODE_HAANTJES, SDRF_MODE_BFC_PAPER = range(6)
 SDRF_LOG_INTS = 8
 
@@ -76,6 +76,7 @@ SIGNATURES = {
     "dcr_sdrf_run": (_I, [_P, _I, _I, _D, _D, _P, _L, _I, _D, _P, _P, _P]),
     "dcr_sdrf_batch_workspace_bytes": (_L, [_I]),
     "dcr_sdrf_run_batch": (_I, [_P, _I, _I, _D, _P, _L, _P]),
+    "dcr_sdrf_edit": (_I, [_P, _P, _L, _P, _P]),
     "dcr_sdrf_pending_improvements": (_I, [_P, _P, _L, _P]),
     "dcr_sdrf_nnz": (_L, [_P]),
     "dcr_sdrf_export": (_I, [_P, _P, _P, _P, _P, _P, _P]),

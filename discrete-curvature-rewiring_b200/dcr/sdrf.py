@@ -95,6 +95,16 @@ class SdrfState:
         res = dict(zip(_RESULT_KEYS, self._result.cpu().tolist()))
         return res, log[: res["iterations_done"]]
 
+    def edit(self, edits) -> dict:
+        """Apply ``edits`` (``[m, 3]`` array or tensor of ``(op, u, v)``, op 1 = ``G.add_edge(u, v)``, 0 =
+        ``G.remove_edge(u, v)``) in order with one launch, refreshing the curvature they change (``dcr_sdrf_edit``).
+        Returns the result dict after one device-to-host copy: ``iterations_done`` is the number of edits applied;
+        a status other than ``SDRF_OK`` names the edit it stopped before in ``pending_x`` / ``pending_y``."""
+        e = edit_tensor(edits).to(self.device).contiguous()
+        L.check(self.lib.dcr_sdrf_edit(self.handle, L.ptr(e) if e.numel() else 0, int(e.shape[0]),
+                                       self._result.data_ptr(), L.current_stream()), "dcr_sdrf_edit")
+        return dict(zip(_RESULT_KEYS, self._result.cpu().tolist()))
+
     def pending_improvements(self, n: int) -> np.ndarray:
         out = torch.empty(max(n, 1), dtype=torch.float64, device=self.device)
         L.check(self.lib.dcr_sdrf_pending_improvements(self.handle, out.data_ptr(), int(n), L.current_stream()),
@@ -142,7 +152,23 @@ class SdrfState:
         return out
 
 
-def _raise_for_status(status: int):
+def edit_tensor(edits) -> torch.Tensor:
+    """``edits`` (array or tensor) as the int32 ``[m, 3]`` tensor ``dcr_sdrf_edit`` reads; ``ValueError`` for another
+    shape, a non-integer type or a value int32 cannot hold (the cast would wrap it into another id)."""
+    e = torch.as_tensor(edits)
+    if e.numel() == 0:
+        e = e.reshape(0, 3).to(torch.int32)
+    if e.ndim != 2 or e.shape[1] != 3:
+        raise ValueError(f"edits: an [m, 3] array of (op, u, v), got shape {tuple(e.shape)}")
+    if e.is_floating_point() or e.is_complex() or e.dtype == torch.bool:
+        raise ValueError(f"edits: integer (op, u, v) expected, got {e.dtype}")
+    if e.numel() and e.dtype != torch.int32 and (int(e.min()) < -2**31 or int(e.max()) > 2**31 - 1):
+        raise ValueError("edits: a value does not fit int32")
+    return e.to(torch.int32)
+
+
+def _raise_for_status(status: int, pair=(0, 0)):
+    """Raise what the reference raises for a loop status; ``pair`` is the edge a failed removal or edit named."""
     if status == L.SDRF_PROB_NAN:
         raise ValueError(_MSG_NAN)
     if status == L.SDRF_PROB_SUM:
@@ -150,9 +176,9 @@ def _raise_for_status(status: int):
     if status == L.SDRF_REMOVE_NONEDGE:
         try:
             import networkx as nx
-            raise nx.NetworkXError("The edge 0-0 is not in the graph")
+            raise nx.NetworkXError(f"The edge {pair[0]}-{pair[1]} is not in the graph")
         except ImportError:
-            raise KeyError("The edge 0-0 is not in the graph")
+            raise KeyError(f"The edge {pair[0]}-{pair[1]} is not in the graph")
     if status == L.SDRF_NO_UNIFORM:
         raise L.DcrError("ran out of uniforms (one is consumed per iteration that has candidates)")
     if status == L.SDRF_ARENA_FULL:
@@ -161,6 +187,8 @@ def _raise_for_status(status: int):
         raise ValueError("min() arg is an empty sequence")      # sdrf_no_cuda.py:26 on a graph without edges
     if status == L.SDRF_TOO_MANY_CANDIDATES:
         raise L.DcrError("candidate matrix (deg x + 1)(deg y + 1) exceeds the scratch of the SDRF state")
+    if status == L.SDRF_BAD_EDIT:
+        raise ValueError(f"edit ({pair[0]}, {pair[1]}): a self-loop or a node id out of range")
     raise L.DcrError(f"unexpected SDRF status {status}")
 
 
@@ -226,6 +254,25 @@ def sdrf(edge_index, num_nodes: int, loops: int, remove_edges: bool, removal_bou
     mode, order = _loop_mode(curv_type, is_undirected)
     directed = mode == L.SDRF_MODE_BFC_DIRECTED
     state = _new_state(mode, order(edge_index, num_nodes), loops)
+    try:
+        log = _run_state(state, loops, remove_edges, removal_bound, tau, uniforms, guard)
+        out_rowptr, out_order = state.export()
+    finally:
+        if state_out is not None:
+            state_out.append(state)
+        else:
+            state.close()
+    edge_index_out = (G.from_digraph_order if directed else G.from_networkx_order)(out_rowptr, out_order)
+    if return_log:
+        return edge_index_out, log
+    return edge_index_out
+
+
+def _run_state(state: SdrfState, loops: int, remove_edges: bool, removal_bound: float, tau, uniforms, guard: float):
+    """Up to ``loops`` iterations of the loop on ``state`` with ``sdrf``'s host protocol: launches until the loop is
+    done, re-deciding on the host every draw the kernel hands back (``NEED_HOST``) and raising the reference's
+    exception for a failed one.  ``uniforms=None`` draws from numpy's global legacy generator and leaves it advanced
+    by exactly the draws used, also when this raises.  Returns the int32 ``[iters, 8]`` log."""
     own_stream = uniforms is None
     if own_stream:
         rng_state = np.random.get_state()
@@ -251,20 +298,12 @@ def sdrf(edge_index, num_nodes: int, loops: int, remove_edges: bool, removal_bou
                 forced = host_choice(imp, tau, float(uniforms[draws]))
                 continue
             _raise_for_status(res["status"])
-        out_rowptr, out_order = state.export()
     finally:
         if own_stream:   # advance numpy's global generator by exactly the draws the reference would have made
             np.random.set_state(rng_state)
             if draws:
                 np.random.random_sample(draws)
-        if state_out is not None:
-            state_out.append(state)
-        else:
-            state.close()
-    edge_index_out = (G.from_digraph_order if directed else G.from_networkx_order)(out_rowptr, out_order)
-    if return_log:
-        return edge_index_out, (np.concatenate(logs) if logs else np.zeros((0, L.SDRF_LOG_INTS), dtype=np.int32))
-    return edge_index_out
+    return np.concatenate(logs) if logs else np.zeros((0, L.SDRF_LOG_INTS), dtype=np.int32)
 
 
 def batch_workspace(count: int, device) -> torch.Tensor:

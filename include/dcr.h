@@ -39,6 +39,7 @@ extern "C" {
 #define DCR_SDRF_ARENA_FULL 6     /* adjacency arena exhausted (create with a larger max_additions)               */
 #define DCR_SDRF_TOO_MANY_CANDIDATES 7 /* (deg x+1)(deg y+1) exceeds the candidate scratch of the state          */
 #define DCR_SDRF_EMPTY_GRAPH 8    /* classical loop on a graph without edges (python: min() of an empty sequence)  */
+#define DCR_SDRF_BAD_EDIT 9       /* dcr_sdrf_edit: an edit with u == v, an id outside [0, n) or an op other than 0/1 */
 
 /* loop flavours of dcr_sdrf_create_mode */
 #define DCR_SDRF_MODE_BFC 0          /* sdrf_cuda_bfc(..., is_undirected=True)   rewiring/sdrf_cuda_bfc.py:14-93        */
@@ -314,6 +315,18 @@ typedef struct dcr_sdrf_batch_run {      /* one run of dcr_sdrf_run_batch; point
 int64_t dcr_sdrf_batch_workspace_bytes(int count);
 int dcr_sdrf_run_batch(const dcr_sdrf_batch_run* runs, int count, int remove_edges, double guard,
                        void* workspace, int64_t workspace_bytes, void* stream);
+/* Apply `count` edits (device int32[count][3]: op (1 add / 0 remove), u, v) in order to the state, refreshing the
+ * curvature of every edge they can change.  Writes *result (device): status, iterations_done = edits applied,
+ * pending_x / pending_y = the offending pair when status != OK.  Enqueues only.
+ * Each edit is the networkx operation on the loop's G (A mirrors it), made with the loop's own toggle: an add appends v
+ * to u's row and u to v's row in insertion order (directed mode: u's successor row and v's predecessor row), a remove
+ * deletes in place, an add of a present edge changes nothing.  The call stops BEFORE an edit with u == v, an id outside
+ * [0, n) or another op (DCR_SDRF_BAD_EDIT), a remove of an absent edge (DCR_SDRF_REMOVE_NONEDGE) or an add beyond the
+ * additions budget (DCR_SDRF_ARENA_FULL); the edits before it stay applied.  The budget is the create call's
+ * max_additions: every add edit counts against it (no-op adds too), and the state counts them across calls.  The
+ * iterations of dcr_sdrf_run add edges the state does not count: a caller that also runs the loop keeps
+ * (add edits) + (iterations) <= max_additions itself. */
+int dcr_sdrf_edit(dcr_sdrf* s, const int32_t* edits, int64_t count, dcr_sdrf_result* result, void* stream);
 /* Improvements (candidate order) of the pending iteration after NEED_HOST: fp64 of the fp32 differences, or the fp64
  * differences themselves for DCR_SDRF_MODE_BFC_PAPER. */
 int dcr_sdrf_pending_improvements(dcr_sdrf* s, double* out, int64_t capacity, void* stream);

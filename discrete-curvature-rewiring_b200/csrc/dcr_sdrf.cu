@@ -1185,9 +1185,10 @@ sdrf_batch_loop_kernel(const SdrfBatchDesc* __restrict__ descs, int remove_edges
 // An add of a present edge changes nothing (networkx keeps its position).  The kernel stops BEFORE an edit with
 // u == v or an id outside [0, n) (BAD_EDIT), a remove of an absent edge (REMOVE_NONEDGE) or an add beyond the
 // additions budget (ARENA_FULL; scalars[2] counts the add edits, no-op adds included, scalars[3] is max_additions).
+// Block-uniform arguments only: the single-state kernel and every CTA of the batch kernel run this on their own state.
 template <int MODE>
-__global__ void __launch_bounds__(SDRF_THREADS, 1)
-sdrf_edit_kernel(SdrfDev S, const int32_t* __restrict__ edits, long long count, dcr_sdrf_result* __restrict__ result) {
+__device__ __forceinline__ void sdrf_edit_body(const SdrfDev& S, const int32_t* __restrict__ edits, long long count,
+                                               dcr_sdrf_result* __restrict__ result) {
     __shared__ LoopShared sh;
     __shared__ int dirty_count, work_count;
     const GraphView g{S.rstart, S.rlen, S.col};                 // undirected adjacency / successors
@@ -1232,17 +1233,45 @@ sdrf_edit_kernel(SdrfDev S, const int32_t* __restrict__ edits, long long count, 
     }
 }
 
+template <int MODE>
+__global__ void __launch_bounds__(SDRF_THREADS, 1)
+sdrf_edit_kernel(SdrfDev S, const int32_t* __restrict__ edits, long long count, dcr_sdrf_result* __restrict__ result) {
+    sdrf_edit_body<MODE>(S, edits, count, result);
+}
+
+// Per-state arguments of the batched edit kernel (dcr_sdrf_edit_batch packs one per run into the caller's workspace).
+struct SdrfEditDesc {
+    SdrfDev S;
+    const int32_t* edits;
+    long long count;
+    dcr_sdrf_result* result;
+};
+static_assert(sizeof(SdrfEditDesc) % 8 == 0, "descriptor copied as 8-byte words");
+
+// B independent edit lists, one CTA per state, the descriptor copied to shared memory as in sdrf_batch_loop_kernel.
+template <int MODE>
+__global__ void __launch_bounds__(SDRF_THREADS, 1)
+sdrf_batch_edit_kernel(const SdrfEditDesc* __restrict__ descs) {
+    __shared__ SdrfEditDesc d;
+    constexpr int WORDS = sizeof(SdrfEditDesc) / 8;
+    const unsigned long long* src = reinterpret_cast<const unsigned long long*>(descs + blockIdx.x);
+    if (threadIdx.x < WORDS) reinterpret_cast<unsigned long long*>(&d)[threadIdx.x] = src[threadIdx.x];
+    __syncthreads();
+    sdrf_edit_body<MODE>(d.S, d.edits, d.count, d.result);
+}
+
 // the kernels of the loop flavour that runs DCR_SDRF_MODE_* `mode`
 struct LoopKernels {
     decltype(&sdrf_init_curvature_kernel<LOOP_BFC>) init;
     decltype(&sdrf_loop_kernel<LOOP_BFC>) single;
     decltype(&sdrf_batch_loop_kernel<LOOP_BFC>) batch;
     decltype(&sdrf_edit_kernel<LOOP_BFC>) edit;
+    decltype(&sdrf_batch_edit_kernel<LOOP_BFC>) batch_edit;
 };
 template <int MODE>
 static LoopKernels loop_kernels_of() {
     return {sdrf_init_curvature_kernel<MODE>, sdrf_loop_kernel<MODE>, sdrf_batch_loop_kernel<MODE>,
-            sdrf_edit_kernel<MODE>};
+            sdrf_edit_kernel<MODE>, sdrf_batch_edit_kernel<MODE>};
 }
 static LoopKernels loop_kernels(int mode) {
     switch (mode) {
@@ -1300,6 +1329,32 @@ __global__ void sdrf_export_c64_kernel(SdrfDev S, const int32_t* rowptr, double*
         for (int t = lane; t < d; t += 32) c64[o + t] = paper_get(S, s + t);
     }
 }
+// from_networkx(G).edge_index of the insertion-order rows (G.from_networkx_order): row w lists its neighbours < w
+// ascending, which is the prefix of its sorted arena row, then its neighbours >= w (its self entry included) in insertion
+// order.  directed: the successor rows as they are (G.from_digraph_order).  One warp per row; `rowptr` comes from
+// sdrf_export_rowptr_kernel(with_self = 1).  Nothing is written at or beyond `capacity`.
+__global__ void sdrf_export_edge_index_kernel(SdrfDev S, const int32_t* rowptr, int64_t* src, int64_t* dst,
+                                              long long capacity, int directed) {
+    const int lane = threadIdx.x & 31;
+    const int warps = (gridDim.x * blockDim.x) >> 5;
+    for (int w = (blockIdx.x * blockDim.x + threadIdx.x) >> 5; w < S.n; w += warps) {
+        const int s = S.rstart[w], len = S.rlen[w], olen = len + S.selfl[w];
+        const int lo = directed ? 0 : lower_bound(S.col, s, len, w);
+        long long o = rowptr[w];
+        for (int t = lane; t < lo; t += 32)
+            if (o + t < capacity) { src[o + t] = w; dst[o + t] = S.col[s + t]; }
+        o += lo;
+        for (int base = 0; base < olen; base += 32) {
+            const int t = base + lane;
+            const int x = t < olen ? S.ord[s + t] : -1;
+            const bool keep = t < olen && (directed || x >= w);
+            const unsigned m = __ballot_sync(FULL, keep);
+            const long long p = o + __popc(m & ((1u << lane) - 1u));
+            if (keep && p < capacity) { src[p] = w; dst[p] = x; }
+            o += __popc(m);
+        }
+    }
+}
 __global__ void sdrf_copy_pending_kernel(const double* pend, double* out, long long n) {
     for (long long t = blockIdx.x * (long long)blockDim.x + threadIdx.x; t < n; t += (long long)gridDim.x * blockDim.x)
         out[t] = pend[t];
@@ -1312,6 +1367,7 @@ using namespace dcr;
 struct dcr_sdrf {
     SdrfDev dev;
     void* slab;           // one allocation backing every array
+    size_t slab_bytes;
     int mode;             // DCR_SDRF_MODE_*
     int64_t n_self;       // nodes that list themselves (self-loops of G)
 };
@@ -1322,6 +1378,25 @@ static T* carve(char*& p, size_t count) {
     p += (count * sizeof(T) + 255) / 256 * 256;
     return out;
 }
+
+// Points D's arrays into the slab at `p` (D's sizes set).  The persistent state, rstart … scalars, is carved first and
+// the scratch after it, so the state is the byte prefix [slab, D.base1) of the slab: that prefix is all dcr_sdrf_fork
+// copies.  A new array that must survive between launches goes before base1.
+static void carve_slab(SdrfDev& D, char* p, int rows, bool paper) {
+    D.rstart = carve<int32_t>(p, rows); D.rlen = carve<int32_t>(p, rows); D.rcap = carve<int32_t>(p, rows);
+    D.selfl = carve<int32_t>(p, rows);
+    D.col = carve<int32_t>(p, D.cap_total); D.ord = carve<int32_t>(p, D.cap_total);
+    D.supp = carve<int32_t>(p, D.cap_total); D.c32 = carve<float>(p, D.cap_total);
+    D.owner = carve<int32_t>(p, D.cap_total); D.flag = carve<int32_t>(p, D.cap_total);
+    D.scalars = carve<int32_t>(p, 8);
+    // ---- scratch of one launch (not copied by dcr_sdrf_fork)
+    D.base1 = carve<int32_t>(p, D.row_cap_max); D.base2 = carve<int32_t>(p, D.row_cap_max);
+    D.posI = carve<int32_t>(p, D.row_cap_max); D.posJ = carve<int32_t>(p, D.row_cap_max);
+    D.imp = carve<uint32_t>(p, (paper ? 2 : 1) * D.imp_cap); D.pend = carve<double>(p, D.imp_cap);
+    D.dirty = carve<int32_t>(p, (size_t)2 * D.dirty_cap); D.work = carve<int32_t>(p, D.dirty_cap);
+    D.wlist = carve<int32_t>(p, D.row_cap_max);
+}
+static size_t persistent_bytes(const dcr_sdrf* s) { return (size_t)((char*)s->dev.base1 - (char*)s->slab); }
 
 // rows [0,n): rowptr/order (neighbours, or successors in the directed mode); rows [n,2n): in_rowptr/in_order
 // (predecessors, directed mode only)
@@ -1420,18 +1495,8 @@ static int sdrf_create_impl(int n, int mode, const int32_t* rowptr_host, const i
     add(D.row_cap_max, 4);                                   // wlist
     cudaError_t e = cudaMalloc(&s->slab, bytes);
     if (e != cudaSuccess) { delete s; return cuda_fail(e, "cudaMalloc(sdrf slab)", __FILE__, __LINE__); }
-    char* p = (char*)s->slab;
-    D.rstart = carve<int32_t>(p, rows); D.rlen = carve<int32_t>(p, rows); D.rcap = carve<int32_t>(p, rows);
-    D.selfl = carve<int32_t>(p, rows);
-    D.col = carve<int32_t>(p, cap_total); D.ord = carve<int32_t>(p, cap_total);
-    D.supp = carve<int32_t>(p, cap_total); D.c32 = carve<float>(p, cap_total);
-    D.owner = carve<int32_t>(p, cap_total); D.flag = carve<int32_t>(p, cap_total);
-    D.scalars = carve<int32_t>(p, 8);
-    D.base1 = carve<int32_t>(p, D.row_cap_max); D.base2 = carve<int32_t>(p, D.row_cap_max);
-    D.posI = carve<int32_t>(p, D.row_cap_max); D.posJ = carve<int32_t>(p, D.row_cap_max);
-    D.imp = carve<uint32_t>(p, (paper ? 2 : 1) * D.imp_cap); D.pend = carve<double>(p, D.imp_cap);
-    D.dirty = carve<int32_t>(p, (size_t)2 * D.dirty_cap); D.work = carve<int32_t>(p, D.dirty_cap);
-    D.wlist = carve<int32_t>(p, D.row_cap_max);
+    s->slab_bytes = bytes;
+    carve_slab(D, (char*)s->slab, rows, paper);
 
     auto fail = [&](cudaError_t err, const char* what) {
         cudaFree(s->slab);
@@ -1484,6 +1549,33 @@ extern "C" void dcr_sdrf_destroy(dcr_sdrf* s) {
     delete s;
 }
 
+// Every copy gets a slab of the source's size (same sizes, so the same carve) and one device-to-device copy of the
+// persistent prefix on `stream`; the scratch is not copied.  All slabs are allocated before any copy is enqueued, so a
+// failure leaves nothing behind.
+extern "C" int dcr_sdrf_fork(dcr_sdrf* s, int count, dcr_sdrf** out_host, void* stream) {
+    if (!s || count < 1 || !out_host) { set_error("dcr_sdrf_fork: bad arguments"); return 1; }
+    const bool directed = s->mode == DCR_SDRF_MODE_BFC_DIRECTED;
+    const bool paper = s->mode == DCR_SDRF_MODE_BFC_PAPER;
+    std::vector<dcr_sdrf*> copies;
+    auto release = [&]() {
+        for (dcr_sdrf* c : copies) { cudaFree(c->slab); delete c; }
+    };
+    for (int b = 0; b < count; ++b) {
+        dcr_sdrf* c = new dcr_sdrf(*s);
+        const cudaError_t e = cudaMalloc(&c->slab, s->slab_bytes);
+        if (e != cudaSuccess) { delete c; release(); return cuda_fail(e, "cudaMalloc(sdrf fork slab)", __FILE__, __LINE__); }
+        copies.push_back(c);
+        carve_slab(c->dev, (char*)c->slab, directed ? 2 * s->dev.n : s->dev.n, paper);
+    }
+    const size_t bytes = persistent_bytes(s);
+    for (dcr_sdrf* c : copies) {
+        const cudaError_t e = cudaMemcpyAsync(c->slab, s->slab, bytes, cudaMemcpyDeviceToDevice, (cudaStream_t)stream);
+        if (e != cudaSuccess) { release(); return cuda_fail(e, "cudaMemcpyAsync(sdrf fork)", __FILE__, __LINE__); }
+    }
+    for (int b = 0; b < count; ++b) out_host[b] = copies[b];
+    return 0;
+}
+
 extern "C" int dcr_sdrf_run(dcr_sdrf* s, int loops, int remove_edges, double removal_bound, double tau,
                             const double* uniforms, int64_t n_uniforms, int forced_choice, double guard, int32_t* log,
                             dcr_sdrf_result* result, void* stream) {
@@ -1499,6 +1591,49 @@ extern "C" int dcr_sdrf_run(dcr_sdrf* s, int loops, int remove_edges, double rem
 extern "C" int dcr_sdrf_edit(dcr_sdrf* s, const int32_t* edits, int64_t count, dcr_sdrf_result* result, void* stream) {
     if (!s || !result || count < 0 || (count > 0 && !edits)) { set_error("dcr_sdrf_edit: bad arguments"); return 1; }
     loop_kernels(s->mode).edit<<<1, SDRF_THREADS, 0, (cudaStream_t)stream>>>(s->dev, edits, (long long)count, result);
+    DCR_LAUNCH_CHECK();
+    return 0;
+}
+
+extern "C" int64_t dcr_sdrf_edit_batch_workspace_bytes(int count) {
+    return count < 1 ? 0 : (int64_t)count * (int64_t)sizeof(SdrfEditDesc);
+}
+
+extern "C" int dcr_sdrf_edit_batch(const dcr_sdrf_edit_run* runs, int count, void* workspace, int64_t workspace_bytes,
+                                   void* stream) {
+    if (count < 1 || !runs) { set_error("dcr_sdrf_edit_batch: count must be >= 1"); return 1; }
+    std::vector<SdrfEditDesc> descs(count);
+    std::vector<const dcr_sdrf*> seen(count);
+    for (int b = 0; b < count; ++b) {
+        const dcr_sdrf_edit_run& r = runs[b];
+        if (!r.state) { set_error("dcr_sdrf_edit_batch: run %d has no state", b); return 1; }
+        if (!r.result || r.count < 0 || (r.count > 0 && !r.edits)) {
+            set_error("dcr_sdrf_edit_batch: run %d: bad arguments", b);
+            return 1;
+        }
+        if (r.state->mode != runs[0].state->mode) {
+            set_error("dcr_sdrf_edit_batch: run %d has loop mode %d, run 0 has %d (one mode per call)", b, r.state->mode,
+                      runs[0].state->mode);
+            return 1;
+        }
+        descs[b] = {r.state->dev, r.edits, (long long)r.count, r.result};
+        seen[b] = r.state;
+    }
+    std::sort(seen.begin(), seen.end());
+    if (std::adjacent_find(seen.begin(), seen.end()) != seen.end()) {
+        set_error("dcr_sdrf_edit_batch: the same state appears twice (runs of one call must own their states)");
+        return 1;
+    }
+    if (!workspace || workspace_bytes < dcr_sdrf_edit_batch_workspace_bytes(count)) {
+        set_error("dcr_sdrf_edit_batch: workspace of dcr_sdrf_edit_batch_workspace_bytes(%d) = %lld bytes required", count,
+                  (long long)dcr_sdrf_edit_batch_workspace_bytes(count));
+        return 1;
+    }
+    if ((uintptr_t)workspace % alignof(SdrfEditDesc)) { set_error("dcr_sdrf_edit_batch: workspace must be 8-byte aligned"); return 1; }
+    cudaStream_t st = (cudaStream_t)stream;
+    // pageable source: the copy is staged before cudaMemcpyAsync returns, so `descs` may go out of scope
+    DCR_CUDA(cudaMemcpyAsync(workspace, descs.data(), sizeof(SdrfEditDesc) * count, cudaMemcpyHostToDevice, st));
+    loop_kernels(runs[0].state->mode).batch_edit<<<count, SDRF_THREADS, 0, st>>>((const SdrfEditDesc*)workspace);
     DCR_LAUNCH_CHECK();
     return 0;
 }
@@ -1596,6 +1731,22 @@ extern "C" int dcr_sdrf_export_order(dcr_sdrf* s, int32_t* rowptr_order, int32_t
     DCR_LAUNCH_CHECK();
     const int ctas = std::max(1, std::min((s->dev.n + 7) / 8, sm_count() * 8));
     sdrf_export_order_kernel<<<ctas, 256, 0, st>>>(s->dev, rowptr_order, order_out);
+    DCR_LAUNCH_CHECK();
+    return 0;
+}
+
+extern "C" int dcr_sdrf_export_edge_index(dcr_sdrf* s, int32_t* rowptr_order, int64_t* src, int64_t* dst,
+                                          int64_t capacity, void* stream) {
+    if (!s || !rowptr_order || capacity < 0 || (capacity > 0 && (!src || !dst))) {
+        set_error("dcr_sdrf_export_edge_index: bad arguments");
+        return 1;
+    }
+    cudaStream_t st = (cudaStream_t)stream;
+    sdrf_export_rowptr_kernel<<<1, SDRF_THREADS, 0, st>>>(s->dev, rowptr_order, 1);
+    DCR_LAUNCH_CHECK();
+    const int ctas = std::max(1, std::min((s->dev.n + 7) / 8, sm_count() * 8));
+    sdrf_export_edge_index_kernel<<<ctas, 256, 0, st>>>(s->dev, rowptr_order, src, dst, (long long)capacity,
+                                                        s->mode == DCR_SDRF_MODE_BFC_DIRECTED);
     DCR_LAUNCH_CHECK();
     return 0;
 }

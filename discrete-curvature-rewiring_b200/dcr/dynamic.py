@@ -8,12 +8,14 @@ an edit can change is recomputed.  ``rewire`` continues SDRF from the current gr
 """
 from __future__ import annotations
 
+import copy
+
 import numpy as np
 import torch
 
-from . import graph as G
 from . import lib as L
-from .sdrf import CLASSICAL_MODES, _loop_mode, _new_state, _raise_for_status, _run_state
+from .sdrf import (CLASSICAL_MODES, _batch_return, _batch_uniforms, _loop_mode, _new_state, _per_run, _raise_for_status,
+                   _run_batch_states, _run_state, edit_batch_states)
 
 _INT32_MAX = 2**31 - 1
 
@@ -117,6 +119,16 @@ class DynamicCurvature:
     def __exit__(self, *exc):
         self.close()
 
+    def fork(self, count: int = 1) -> list:
+        """``count`` independent copies of this object (graph, insertion order, curvature, budget) made on the device
+        with one ``dcr_sdrf_fork``; each is closed on its own."""
+        out = []
+        for st in self._state.fork(count):
+            dc = copy.copy(self)
+            dc._state = st
+            out.append(dc)
+        return out
+
     @property
     def remaining(self) -> int:
         """Additions left in the budget."""
@@ -129,6 +141,12 @@ class DynamicCurvature:
         batch before it, the edits before it stay applied and the object stays usable: ``networkx.NetworkXError`` for
         removing a non-edge, ``ValueError`` for a self-loop or an id outside ``[0, n)``, ``DcrError`` for an add beyond
         the budget."""
+        e, stop, dev = self._prepare_edits(ops)
+        return self._finish_edits(e, stop, self._state.edit(dev))
+
+    def _prepare_edits(self, ops):
+        """``(e, stop, dev)``: ``ops`` checked (:func:`edit_array`), the index of the first add beyond the budget (or
+        ``m``) and the edits before it as the device takes them."""
         e = edit_array(ops)
         is_add = e[:, 0] == 1
         over = np.flatnonzero(is_add & (np.cumsum(is_add) > self.remaining))
@@ -138,9 +156,13 @@ class DynamicCurvature:
         dev = e[:stop].copy()
         ids = dev[:, 1:]
         ids[(ids < 0) | (ids > _INT32_MAX)] = -1        # an id int32 cannot hold: out of range for the device as well
-        res = self._state.edit(dev)
+        return e, stop, dev
+
+    def _finish_edits(self, e, stop: int, res: dict) -> int:
+        """Count the add edits the device applied (``res``) and raise for the edit it stopped before, or for the first
+        add beyond the budget; returns the number applied."""
         applied = res["iterations_done"]
-        self._edit_adds += int(np.count_nonzero(is_add[:applied]))
+        self._edit_adds += int(np.count_nonzero(e[:applied, 0] == 1))
         if res["status"] != L.SDRF_OK:                  # it stopped before edit `applied`: name that edit as given
             _raise_for_status(res["status"], tuple(int(x) for x in e[applied, 1:]))
         if stop < e.shape[0]:
@@ -167,9 +189,9 @@ class DynamicCurvature:
         return self._state.export()
 
     def edge_index(self) -> np.ndarray:
-        """int64 ``[2, nnz]`` in the column order ``sdrf()`` returns (``from_networkx(G).edge_index``)."""
-        rp, od = self._state.export()
-        return (G.from_digraph_order if self.directed else G.from_networkx_order)(rp, od)
+        """int64 ``[2, nnz]`` in the column order ``sdrf()`` returns (``from_networkx(G).edge_index``), exported on the
+        device."""
+        return self._state.edge_index().cpu().numpy()
 
     def curvature(self) -> np.ndarray:
         """One value per column of :meth:`edge_index`: fp32 ``C[i,j]`` for ``'bfc'``, the integer curvature for
@@ -201,3 +223,65 @@ class DynamicCurvature:
         self._loop_adds += int(np.count_nonzero(log[:, 3] >= 0))
         ei = self.edge_index()
         return (ei, log) if return_log else ei
+
+    def rewire_batch(self, loops, remove_edges: bool, removal_bound, tau, *, uniforms, guard: float = 1e-9,
+                     return_log: bool = False, return_exceptions: bool = False):
+        """B continuations of SDRF from the current graph in one launch, one CTA per run, on B forks of this object.
+        Run ``r`` computes exactly what ``self.fork()[0].rewire(loops[r], remove_edges, removal_bound[r], tau[r],
+        uniforms=uniforms[r])`` computes; ``self`` is left unchanged.
+
+        ``uniforms``: a ``[B, loops]`` array or a list of B 1-d arrays; it fixes B.  ``loops``, ``removal_bound``,
+        ``tau``: scalars or length-B sequences.  Raises ``ValueError`` before any launch when a run's ``loops`` exceeds
+        :attr:`remaining`.  Returns and raises what ``sdrf_batch`` does: a list of B ``edge_index`` arrays (and with
+        ``return_log`` a list of B logs); a failed run raises after the batch (the lowest-index one) or, with
+        ``return_exceptions``, leaves its exception in its slot."""
+        uni = _batch_uniforms(uniforms, "rewire_batch")
+        count = len(uni)
+        iters = [max(int(v), 0) for v in _per_run("loops", loops, count)]
+        bounds = [float(v) for v in _per_run("removal_bound", removal_bound, count)]
+        taus = _per_run("tau", tau, count)
+        over = [r for r in range(count) if iters[r] > self.remaining]
+        if over:
+            raise ValueError(f"rewire_batch: run {over[0]}: {iters[over[0]]} iterations exceed the remaining additions "
+                             f"budget ({self.remaining})")
+        forks = self._state.fork(count)
+        try:
+            logs, done, errors = _run_batch_states(forks, iters, bounds, taus, uni, remove_edges, guard)
+            outs, out_logs = [], []
+            for r in range(count):
+                out_logs.append(logs[r][: done[r]].cpu().numpy())
+                outs.append(errors[r] if errors[r] is not None else forks[r].edge_index().cpu().numpy())
+        finally:
+            for f in forks:
+                f.close()
+        return _batch_return(outs, out_logs, errors, return_log, return_exceptions)
+
+
+def edit_batch(objects, ops_list, *, return_exceptions: bool = False) -> list:
+    """Apply ``ops_list[b]`` to ``objects[b]`` for every b in ONE launch, one CTA per object, and return the number of
+    edits each applied.  Every object ends exactly as ``objects[b].edit(ops_list[b])`` would leave it (same budget rule,
+    same stop).  A failed object raises after the batch (the lowest-index one, with the type and message ``edit``
+    raises) or, with ``return_exceptions``, leaves its exception in its slot; the others are applied either way.
+    Objects of different modes, or one object twice, raise ``ValueError`` before any launch."""
+    objects, ops_list = list(objects), list(ops_list)
+    if not objects:
+        raise ValueError("edit_batch: an empty batch")
+    if len(ops_list) != len(objects):
+        raise ValueError(f"edit_batch: {len(ops_list)} edit lists for {len(objects)} objects")
+    if len({id(o) for o in objects}) != len(objects):
+        raise ValueError("edit_batch: the same object appears twice (each edit list needs its own object)")
+    if any(o.mode != objects[0].mode for o in objects):
+        raise ValueError("edit_batch: objects of different modes (one mode per call)")
+    if any(o._state is None for o in objects):
+        raise ValueError("edit_batch: a closed object")
+    prepared = [o._prepare_edits(ops) for o, ops in zip(objects, ops_list)]
+    results = edit_batch_states([o._state for o in objects], [dev for _, _, dev in prepared])
+    counts, errors = [], []
+    for o, (e, stop, _), res in zip(objects, prepared, results):
+        try:
+            counts.append(o._finish_edits(e, stop, res))
+            errors.append(None)
+        except Exception as ex:      # this object stopped; the others are applied
+            counts.append(ex)
+            errors.append(ex)
+    return _batch_return(counts, None, errors, False, return_exceptions)

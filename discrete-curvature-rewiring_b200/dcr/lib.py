@@ -19,6 +19,11 @@ class SdrfBatchRun(C.Structure):
                 ("n_uniforms", C.c_int64), ("log", C.c_void_p), ("result", C.c_void_p)]
 
 
+class SdrfEditRun(C.Structure):
+    """``dcr_sdrf_edit_run``: one state of ``dcr_sdrf_edit_batch`` (``edits`` and ``result`` are device pointers)."""
+    _fields_ = [("state", C.c_void_p), ("edits", C.c_void_p), ("count", C.c_int64), ("result", C.c_void_p)]
+
+
 # status codes of include/dcr.h
 SDRF_OK, SDRF_NEED_HOST, SDRF_PROB_NAN, SDRF_PROB_SUM, SDRF_REMOVE_NONEDGE, SDRF_NO_UNIFORM, SDRF_ARENA_FULL, \
     SDRF_TOO_MANY_CANDIDATES, SDRF_EMPTY_GRAPH, SDRF_BAD_EDIT = range(10)
@@ -77,11 +82,15 @@ SIGNATURES = {
     "dcr_sdrf_batch_workspace_bytes": (_L, [_I]),
     "dcr_sdrf_run_batch": (_I, [_P, _I, _I, _D, _P, _L, _P]),
     "dcr_sdrf_edit": (_I, [_P, _P, _L, _P, _P]),
+    "dcr_sdrf_edit_batch_workspace_bytes": (_L, [_I]),
+    "dcr_sdrf_edit_batch": (_I, [_P, _I, _P, _L, _P]),
+    "dcr_sdrf_fork": (_I, [_P, _I, C.POINTER(_P), _P]),
     "dcr_sdrf_pending_improvements": (_I, [_P, _P, _L, _P]),
     "dcr_sdrf_nnz": (_L, [_P]),
     "dcr_sdrf_export": (_I, [_P, _P, _P, _P, _P, _P, _P]),
     "dcr_sdrf_export_order": (_I, [_P, _P, _P, _P]),
     "dcr_sdrf_export_c64": (_I, [_P, _P, _P, _P]),
+    "dcr_sdrf_export_edge_index": (_I, [_P, _P, _P, _P, _L, _P]),
 }
 
 _lib = None

@@ -71,6 +71,24 @@ class SdrfState:
         self.device = torch.device("cuda", torch.cuda.current_device())
         self._result = torch.zeros(8, dtype=torch.int32, device=self.device)
 
+    @classmethod
+    def _from_handle(cls, handle: C.c_void_p, like: "SdrfState") -> "SdrfState":
+        """A state that owns ``handle``, a copy of ``like`` made by ``dcr_sdrf_fork``."""
+        self = cls.__new__(cls)
+        self.lib, self.mode, self.n, self.n_self, self.device = like.lib, like.mode, like.n, like.n_self, like.device
+        self._keep = None
+        self.handle = handle
+        self._result = torch.zeros(8, dtype=torch.int32, device=self.device)
+        return self
+
+    def fork(self, count: int) -> list:
+        """``count`` independent copies of this state (graph, insertion order, curvature, budget) after one
+        ``dcr_sdrf_fork``: device-to-device copies enqueued on the current stream, no host set-up."""
+        count = int(count)
+        handles = (C.c_void_p * max(count, 1))()
+        L.check(self.lib.dcr_sdrf_fork(self.handle, count, handles, L.current_stream()), "dcr_sdrf_fork")
+        return [SdrfState._from_handle(C.c_void_p(h), self) for h in handles[:count]]
+
     def close(self):
         if getattr(self, "handle", None):
             self.lib.dcr_sdrf_destroy(self.handle)
@@ -150,6 +168,16 @@ class SdrfState:
         if with_curvature:
             out += (col[:nnz].cpu().numpy(), c32[:nnz].cpu().numpy(), tri[:nnz].cpu().numpy())
         return out
+
+    def edge_index(self) -> torch.Tensor:
+        """The current graph as the int64 ``[2, E]`` device tensor ``from_networkx(G).edge_index`` gives, in the column
+        order ``sdrf()`` returns (``dcr_sdrf_export_edge_index``)."""
+        cap = self.nnz() + self.n_self
+        rowptr = torch.empty(self.n + 1, dtype=torch.int32, device=self.device)
+        out = torch.empty((2, max(cap, 1)), dtype=torch.int64, device=self.device)
+        L.check(self.lib.dcr_sdrf_export_edge_index(self.handle, rowptr.data_ptr(), out[0].data_ptr(), out[1].data_ptr(),
+                                                    cap, L.current_stream()), "dcr_sdrf_export_edge_index")
+        return out[:, : int(rowptr[-1])]
 
 
 def edit_tensor(edits) -> torch.Tensor:
@@ -330,6 +358,79 @@ def run_batch(states, loops, removal_bounds, taus, uniforms, forced, logs, remov
     return [dict(zip(_RESULT_KEYS, r)) for r in results[:b].cpu().tolist()]
 
 
+def edit_batch_states(states, edits) -> list:
+    """One ``dcr_sdrf_edit_batch`` launch: ``states[b]`` applies ``edits[b]`` (an ``[m, 3]`` array of ``(op, u, v)``, see
+    ``SdrfState.edit``).  Returns the B result dicts of ``SdrfState.edit`` after ONE device-to-host copy."""
+    b = len(states)
+    dev = states[0].device
+    host = [edit_tensor(e).cpu() for e in edits]
+    counts = [int(e.shape[0]) for e in host]
+    offsets = np.concatenate([[0], np.cumsum(counts)]).tolist()
+    flat = torch.cat(host).to(dev)            # every edit list in one host-to-device copy
+    results = torch.zeros((b, 8), dtype=torch.int32, device=dev)
+    nbytes = int(L.load().dcr_sdrf_edit_batch_workspace_bytes(b))
+    workspace = torch.empty(max(nbytes // 8, 1), dtype=torch.int64, device=dev)
+    runs = (L.SdrfEditRun * b)()
+    for i, s in enumerate(states):
+        ptr = flat.data_ptr() + 3 * 4 * offsets[i] if counts[i] else 0
+        runs[i] = L.SdrfEditRun(s.handle, ptr, counts[i], results[i].data_ptr())
+    L.check(L.load().dcr_sdrf_edit_batch(runs, b, workspace.data_ptr(), workspace.numel() * workspace.element_size(),
+                                         L.current_stream()), "dcr_sdrf_edit_batch")
+    return [dict(zip(_RESULT_KEYS, r)) for r in results.cpu().tolist()]
+
+
+def _batch_uniforms(uniforms, caller: str) -> list:
+    """``uniforms`` of a batch (a ``[B, loops]`` array or a list of B 1-d arrays) as B fp64 arrays; B >= 1.  ``caller``
+    names the public function in the errors."""
+    if isinstance(uniforms, np.ndarray) and uniforms.ndim != 2:
+        raise ValueError("uniforms: a [B, loops] array or a list of B 1-d arrays")
+    uni = [np.ascontiguousarray(u, dtype=np.float64) for u in uniforms]
+    if len(uni) < 1:
+        raise ValueError(f"{caller}: an empty batch")
+    if any(u.ndim != 1 for u in uni):
+        raise ValueError("uniforms: a [B, loops] array or a list of B 1-d arrays")
+    return uni
+
+
+def _run_batch_states(states, iters, bounds, taus, uni, remove_edges: bool, guard: float):
+    """Run ``r`` continues ``states[r]`` for up to ``iters[r]`` iterations with the uniforms ``uni[r]``, all runs in
+    one ``dcr_sdrf_run_batch`` launch; runs that need a host-side decision re-enter together in the next launch, and a
+    failing run does not stop the others.  Returns ``(logs, done, errors)``: the device logs, the iterations each run
+    completed and, per run, ``None`` or the exception ``sdrf`` raises for it."""
+    count = len(states)
+    dev = states[0].device
+    padded, supplied = zip(*(_pad_uniforms(u, iters[r]) for r, u in enumerate(uni)))
+    u_dev = [torch.from_numpy(u).to(dev) for u in padded]
+    logs = [torch.empty((max(iters[r], 1), L.SDRF_LOG_INTS), dtype=torch.int32, device=dev) for r in range(count)]
+    results = torch.zeros((count, 8), dtype=torch.int32, device=dev)
+    workspace = batch_workspace(count, dev)
+    done, draws, forced = [0] * count, [0] * count, [-1] * count
+    errors = [None] * count
+    active = [r for r in range(count) if iters[r] > 0]
+    while active:
+        res = run_batch([states[r] for r in active], [iters[r] - done[r] for r in active],
+                        [bounds[r] for r in active], [taus[r] for r in active],
+                        [u_dev[r][draws[r]:supplied[r]] if supplied[r] > draws[r] else u_dev[r][:0] for r in active],
+                        [forced[r] for r in active], [logs[r][done[r]:] for r in active], remove_edges, guard,
+                        results, workspace)
+        again = []
+        for r, rr in zip(active, res):
+            forced[r] = -1
+            done[r] += rr["iterations_done"]
+            draws[r] += rr["draws_used"]
+            try:
+                if rr["status"] == L.SDRF_NEED_HOST:
+                    imp = states[r].pending_improvements(rr["pending_n"])
+                    forced[r] = host_choice(imp, taus[r], float(padded[r][draws[r]]))
+                    again.append(r)
+                elif rr["status"] != L.SDRF_OK:
+                    _raise_for_status(rr["status"])
+            except Exception as e:      # this run is over; the others go on
+                errors[r] = e
+        active = again
+    return logs, done, errors
+
+
 def _per_run(name: str, value, count: int) -> list:
     is_seq = isinstance(value, (list, tuple)) or (isinstance(value, (np.ndarray, torch.Tensor)) and value.ndim > 0)
     if not is_seq:
@@ -357,14 +458,8 @@ def sdrf_batch(edge_indices, num_nodes, loops, remove_edges: bool, removal_bound
     raises after the batch — the lowest-index one, with the type and message ``sdrf`` raises — or, with
     ``return_exceptions``, leaves its exception in its ``edge_index`` slot (its log slot holds the iterations it
     completed)."""
-    if isinstance(uniforms, np.ndarray) and uniforms.ndim != 2:
-        raise ValueError("uniforms: a [B, loops] array or a list of B 1-d arrays")
-    uni = [np.ascontiguousarray(u, dtype=np.float64) for u in uniforms]
+    uni = _batch_uniforms(uniforms, "sdrf_batch")
     count = len(uni)
-    if count < 1:
-        raise ValueError("sdrf_batch: an empty batch")
-    if any(u.ndim != 1 for u in uni):
-        raise ValueError("uniforms: a [B, loops] array or a list of B 1-d arrays")
     shared_input = not isinstance(edge_indices, (list, tuple))
     inputs = [edge_indices] * count if shared_input else _per_run("edge_indices", edge_indices, count)
     nodes = [int(v) for v in _per_run("num_nodes", num_nodes, count)]
@@ -383,36 +478,7 @@ def sdrf_batch(edge_indices, num_nodes, loops, remove_edges: bool, removal_bound
             if key not in orders:
                 orders[key] = order(inputs[r], nodes[r])
             states.append(_new_state(mode, orders[key], iters[r]))
-        dev = states[0].device
-        padded, supplied = zip(*(_pad_uniforms(u, iters[r]) for r, u in enumerate(uni)))
-        u_dev = [torch.from_numpy(u).to(dev) for u in padded]
-        logs = [torch.empty((max(iters[r], 1), L.SDRF_LOG_INTS), dtype=torch.int32, device=dev) for r in range(count)]
-        results = torch.zeros((count, 8), dtype=torch.int32, device=dev)
-        workspace = batch_workspace(count, dev)
-        done, draws, forced = [0] * count, [0] * count, [-1] * count
-        errors = [None] * count
-        active = [r for r in range(count) if iters[r] > 0]
-        while active:
-            res = run_batch([states[r] for r in active], [iters[r] - done[r] for r in active],
-                            [bounds[r] for r in active], [taus[r] for r in active],
-                            [u_dev[r][draws[r]:supplied[r]] if supplied[r] > draws[r] else u_dev[r][:0] for r in active],
-                            [forced[r] for r in active], [logs[r][done[r]:] for r in active], remove_edges, guard,
-                            results, workspace)
-            again = []
-            for r, rr in zip(active, res):
-                forced[r] = -1
-                done[r] += rr["iterations_done"]
-                draws[r] += rr["draws_used"]
-                try:
-                    if rr["status"] == L.SDRF_NEED_HOST:
-                        imp = states[r].pending_improvements(rr["pending_n"])
-                        forced[r] = host_choice(imp, taus[r], float(padded[r][draws[r]]))
-                        again.append(r)
-                    elif rr["status"] != L.SDRF_OK:
-                        _raise_for_status(rr["status"])
-                except Exception as e:      # this run is over; the others go on
-                    errors[r] = e
-            active = again
+        logs, done, errors = _run_batch_states(states, iters, bounds, taus, uni, remove_edges, guard)
         outs, out_logs = [], []
         for r in range(count):
             out_logs.append(logs[r][: done[r]].cpu().numpy())
@@ -424,6 +490,12 @@ def sdrf_batch(edge_indices, num_nodes, loops, remove_edges: bool, removal_bound
     finally:
         for s in states:
             s.close()
+    return _batch_return(outs, out_logs, errors, return_log, return_exceptions)
+
+
+def _batch_return(outs, out_logs, errors, return_log: bool, return_exceptions: bool):
+    """A batch's return value: the lowest-index failure is raised unless ``return_exceptions`` (then it stays in its
+    run's slot of ``outs``)."""
     if not return_exceptions:
         first = next((e for e in errors if e is not None), None)
         if first is not None:

@@ -327,6 +327,28 @@ int dcr_sdrf_run_batch(const dcr_sdrf_batch_run* runs, int count, int remove_edg
  * iterations of dcr_sdrf_run add edges the state does not count: a caller that also runs the loop keeps
  * (add edits) + (iterations) <= max_additions itself. */
 int dcr_sdrf_edit(dcr_sdrf* s, const int32_t* edits, int64_t count, dcr_sdrf_result* result, void* stream);
+/* Batched edits: `count` independent edit lists in ONE launch, one persistent CTA per state.  Each record carries what
+ * dcr_sdrf_edit takes; `runs` is a host array packed into `workspace` (device memory of at least
+ * dcr_sdrf_edit_batch_workspace_bytes(count) bytes, 8-byte aligned) with one host-to-device copy on `stream`, then one
+ * launch.  Status 1 before any launch for count < 1, a null state, the same state twice, states of different
+ * DCR_SDRF_MODE_* or a short workspace.  Every run then behaves exactly as its own dcr_sdrf_edit call would, including
+ * where it stops and what it writes into its result. */
+typedef struct dcr_sdrf_edit_run {       /* one state of dcr_sdrf_edit_batch; edits / result are device pointers */
+    dcr_sdrf* state;
+    const int32_t* edits;                /* int32[count][3], as in dcr_sdrf_edit                         */
+    int64_t count;
+    dcr_sdrf_result* result;
+} dcr_sdrf_edit_run;
+int64_t dcr_sdrf_edit_batch_workspace_bytes(int count);
+int dcr_sdrf_edit_batch(const dcr_sdrf_edit_run* runs, int count, void* workspace, int64_t workspace_bytes,
+                        void* stream);
+/* `count` independent copies of s: graph, insertion order, curvature, supports and the budget words (add edits so far
+ * and max_additions: a copy has the budget the source has left, and its arena is the source's size).  out_host: host
+ * array of `count` handles, each released with dcr_sdrf_destroy.  Allocates, then enqueues the copies on `stream` after
+ * the work already on it; no host synchronise.  Status 1 for count < 1 or a null state; on any failure nothing is
+ * allocated and no handle is written.  The pending improvements of a run that stopped with DCR_SDRF_NEED_HOST are not
+ * copied: fork a state only between runs that ended otherwise. */
+int dcr_sdrf_fork(dcr_sdrf* s, int count, dcr_sdrf** out_host, void* stream);
 /* Improvements (candidate order) of the pending iteration after NEED_HOST: fp64 of the fp32 differences, or the fp64
  * differences themselves for DCR_SDRF_MODE_BFC_PAPER. */
 int dcr_sdrf_pending_improvements(dcr_sdrf* s, double* out, int64_t capacity, void* stream);
@@ -340,6 +362,14 @@ int dcr_sdrf_export(dcr_sdrf* s, int32_t* rowptr, int32_t* order_out, int32_t* c
 /* Insertion-order rows INCLUDING the self entries (see dcr_sdrf_create): rowptr_order[n+1] and order_out[rowptr_order[n]]
  * (at most nnz + n entries).  dcr_sdrf_export refuses order_out for a state that has self entries. */
 int dcr_sdrf_export_order(dcr_sdrf* s, int32_t* rowptr_order, int32_t* order_out, void* stream);
+
+/* The edge_index that from_networkx(G) gives for the current graph, on the device: column t is (src[t], dst[t]) for
+ * t < rowptr_order[n], in the column order sdrf() returns (row w: neighbours < w ascending, then neighbours >= w, its
+ * self entry included, in insertion order; BFC_DIRECTED: the successor rows in insertion order).  rowptr_order[n+1] as in
+ * dcr_sdrf_export_order.  At most nnz + (nodes that listed themselves at create) columns; nothing is written at or
+ * beyond `capacity`.  Enqueues only. */
+int dcr_sdrf_export_edge_index(dcr_sdrf* s, int32_t* rowptr_order, int64_t* src, int64_t* dst, int64_t capacity,
+                               void* stream);
 
 /* DCR_SDRF_MODE_BFC_PAPER states only: rowptr[n+1] and the fp64 paper-flavour curvature of every directed entry in
  * SORTED order per row (the layout of dcr_sdrf_export's colidx_sorted / c32_sorted).  That mode keeps no fp32 curvature

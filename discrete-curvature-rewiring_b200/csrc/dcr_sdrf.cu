@@ -742,6 +742,57 @@ __device__ __forceinline__ void refresh_dirty(const SdrfDev& S, const GraphView&
 }
 
 // ------------------------------------------------------------------------------------------------------------
+// candidate scoring of one pair (x, y), shared by the loop (step 2) and sdrf_score_kernel
+// ------------------------------------------------------------------------------------------------------------
+// The candidate list of one side in networkx order (sdrf_cuda_bfc.py:45-49): the insertion-order row of `row` (x's
+// neighbours / successors, y's neighbours / predecessors; a node that lists itself appears in it) and then the node
+// itself.  n = row length + self entry + 1.
+struct CandList {
+    const int32_t* ord;
+    int o, n, self;
+    __device__ __forceinline__ int operator()(int t) const { return t < n - 1 ? ord[o + t] : self; }
+};
+__device__ __forceinline__ int cand_count(const SdrfDev& S, int row) { return S.rlen[row] + S.selfl[row] + 1; }
+
+// Scores every cell (I, J) of nbI x nbJ for the pair (x, y).  BFC / directed: put(I, J, D) with D the curvature of
+// (x, y) after adding (i, j), MASKED_D for a masked cell; classical: put(I, J, improvement) in closed form, MASKED_D
+// for a masked cell; paper: the fp64 bits of the improvement (IMP_MASKED64 when masked) into imp64[I * n_j + J],
+// against cxy_d = bfc(x, y).  Reads the state and writes only its scratch rows (sc; the paper flavour: S.base1 / base2),
+// imp64 / put and the shared structs.  Every thread calls.
+// after_prepare() runs between the BFC flavour's two scoring phases (the loop's phase timer).
+template <int MODE, class Put, class Sh, class Hook>
+__device__ __forceinline__ void score_pair(const SdrfDev& S, const GraphView& g, const GraphView& gin, int x, int y,
+                                           const CandList& nbI, const CandList& nbJ, const ScoreScratch& sc, Put put,
+                                           unsigned long long* imp64, double cxy_d, Sh* sh, DirScoreShared* dsh,
+                                           int* dred, Hook after_prepare) {
+    const int n_i = nbI.n, n_j = nbJ.n;
+    if constexpr (MODE == LOOP_BFC) {
+        score_prepare(g, S.supp, x, y, nbI, n_i, nbJ, n_j, sc, &sh->score);
+        after_prepare();
+        // x (y) sits at the end of its list — and, with a self-loop, once more inside it: then every row is checked
+        score_cells(g, S.supp, x, y, nbI, n_i, nbJ, n_j, sc, &sh->score, put, S.selfl[x] ? -1 : n_i - 1,
+                    S.selfl[y] ? -1 : n_j - 1);
+    } else if constexpr (MODE == LOOP_DIRECTED) {
+        directed_score_prepare(g, gin, x, y, nbI, n_i, nbJ, n_j, sc, dsh, dred);
+        directed_score_cells(g, gin, x, y, nbI, n_i, nbJ, n_j, sc, dsh, put);
+    } else if constexpr (MODE == LOOP_PAPER) {
+        paper_score(S, g, x, y, nbI, n_i, nbJ, n_j, cxy_d, imp64, sh);
+    } else {
+        // sdrf_no_cuda.py:41-46 in closed form: adding (i,j) changes curvature(x,y) only when it touches x or y.
+        // i == x (then j in N(y)\N(x)): deg x + 1 and one more triangle; j == y mirrored; every other
+        // candidate leaves both degrees and the common neighbours alone.
+        const float special = S.ctype == 0 ? -1.0f : (S.ctype == 1 ? 2.0f : 1.0f);
+        const long long cells = (long long)n_i * n_j;
+        for (long long c = threadIdx.x; c < cells; c += SDRF_THREADS) {
+            const int I = (int)(c / n_j), J = (int)(c - (long long)I * n_j);
+            const int i = nbI(I), j = nbJ(J);
+            const bool masked = (i == j) || edge_slot(g, i, j) >= 0;       // :34
+            put(I, J, masked ? MASKED_D : ((i == x || j == y) ? special : 0.0f));
+        }
+    }
+}
+
+// ------------------------------------------------------------------------------------------------------------
 // the loop
 // ------------------------------------------------------------------------------------------------------------
 // One run of the loop on the calling CTA.  Block-uniform arguments only; nothing here reads blockIdx or gridDim, so the
@@ -894,38 +945,19 @@ __device__ __forceinline__ void sdrf_loop_body(const SdrfDev& S, int loops, int 
         }
         SDRF_TICK(0);   // argmin/argmax
         // ---- 2. candidate matrix in networkx order (:45-54) and improvements (:57-62) ------------------
-        const int ox = S.rstart[x], oy = S.rstart[(MODE == LOOP_DIRECTED ? S.n : 0) + y];
-        auto nbI = [=](int I) { return I < n_i - 1 ? S.ord[ox + I] : x; };
-        auto nbJ = [=](int J) { return J < n_j - 1 ? S.ord[oy + J] : y; };
+        const CandList nbI{S.ord, S.rstart[x], n_i, x};
+        const CandList nbJ{S.ord, S.rstart[(MODE == LOOP_DIRECTED ? S.n : 0) + y], n_j, y};
         {
             const float cxy = sh.cxy;
             uint32_t* imp = S.imp;
-            auto put = [=](int I, int J, float d) {
-                imp[(long long)I * n_j + J] = (d == MASKED_D) ? IMP_MASKED : __float_as_uint(__fsub_rn(d, cxy));
+            auto put = [=](int I, int J, float d) {    // (the classical flavour puts the improvement itself)
+                imp[(long long)I * n_j + J] = (d == MASKED_D) ? IMP_MASKED
+                                              : __float_as_uint(MODE == LOOP_CLASSICAL ? d : __fsub_rn(d, cxy));
             };
-            if constexpr (MODE == LOOP_BFC) {
-                score_prepare(g, S.supp, x, y, nbI, n_i, nbJ, n_j, sc, &sh.score);
-                SDRF_TICK(7);   // (profile build: scoring = prepare [7] + cells [1])
-                // x (y) sits at the end of its list — and, with a self-loop, once more inside it: then every row is checked
-                score_cells(g, S.supp, x, y, nbI, n_i, nbJ, n_j, sc, &sh.score, put, S.selfl[x] ? -1 : n_i - 1,
-                            S.selfl[y] ? -1 : n_j - 1);
-            } else if constexpr (MODE == LOOP_DIRECTED) {
-                directed_score_prepare(g, gin, x, y, nbI, n_i, nbJ, n_j, sc, &dsh, dred);
-                directed_score_cells(g, gin, x, y, nbI, n_i, nbJ, n_j, sc, &dsh, put);
-            } else if constexpr (PAPER) {
-                paper_score(S, g, x, y, nbI, n_i, nbJ, n_j, sh.cxy_d, reinterpret_cast<unsigned long long*>(S.imp), &sh);
-            } else {
-                // sdrf_no_cuda.py:41-46 in closed form: adding (i,j) changes curvature(x,y) only when it touches x or y.
-                // i == x (then j in N(y)\N(x)): deg x + 1 and one more triangle; j == y mirrored; every other
-                // candidate leaves both degrees and the common neighbours alone.
-                const float special = S.ctype == 0 ? -1.0f : (S.ctype == 1 ? 2.0f : 1.0f);
-                for (long long c = tid; c < cells; c += SDRF_THREADS) {
-                    const int I = (int)(c / n_j), J = (int)(c - (long long)I * n_j);
-                    const int i = nbI(I), j = nbJ(J);
-                    const bool masked = (i == j) || edge_slot(g, i, j) >= 0;       // :34
-                    imp[c] = masked ? IMP_MASKED : __float_as_uint((i == x || j == y) ? special : 0.0f);
-                }
-            }
+            double cxy_d = 0.0;
+            if constexpr (PAPER) cxy_d = sh.cxy_d;
+            score_pair<MODE>(S, g, gin, x, y, nbI, nbJ, sc, put, reinterpret_cast<unsigned long long*>(S.imp), cxy_d,
+                             &sh, &dsh, dred, [&] { SDRF_TICK(7); });   // (profile build: scoring = prepare [7] + cells [1])
         }
         __syncthreads();
         SDRF_TICK(1);   // scoring
@@ -1260,6 +1292,118 @@ sdrf_batch_edit_kernel(const SdrfEditDesc* __restrict__ descs) {
     sdrf_edit_body<MODE>(d.S, d.edits, d.count, d.result);
 }
 
+// ------------------------------------------------------------------------------------------------------------
+// caller queries: the candidate scores of many pairs (dcr_sdrf_score_sizes, dcr_sdrf_score)
+// ------------------------------------------------------------------------------------------------------------
+// The pairs the loop itself can score: BFC and directed any 0 <= x, y < n (its (0,0) fallback scores a non-edge and
+// x == y); classical an edge in either orientation or the loop edge (u, u) of a node that lists itself; paper an edge.
+template <int MODE>
+__device__ __forceinline__ bool score_query_ok(const SdrfDev& S, const GraphView& g, int x, int y) {
+    if (x < 0 || x >= S.n || y < 0 || y >= S.n) return false;
+    if constexpr (MODE == LOOP_BFC || MODE == LOOP_DIRECTED) return true;
+    if (x == y) return MODE == LOOP_CLASSICAL && S.selfl[x];
+    return edge_slot(g, x, y) >= 0;
+}
+// DCR_SDRF_OK and (n_i, n_j) of a query the score kernel takes, else its status
+template <int MODE>
+__device__ __forceinline__ int score_query_sizes(const SdrfDev& S, const GraphView& g, int x, int y, int& n_i, int& n_j) {
+    n_i = n_j = 0;
+    if (!score_query_ok<MODE>(S, g, x, y)) return DCR_SDRF_BAD_QUERY;
+    const int a = cand_count(S, x), b = cand_count(S, (MODE == LOOP_DIRECTED ? S.n : 0) + y);
+    if (a > S.row_cap_max || b > S.row_cap_max) return DCR_SDRF_TOO_MANY_CANDIDATES;   // (rows grown past the budget)
+    n_i = a;
+    n_j = b;
+    return DCR_SDRF_OK;
+}
+
+template <int MODE>
+__global__ void sdrf_score_sizes_kernel(SdrfDev S, const int32_t* __restrict__ pairs, int count,
+                                        int32_t* __restrict__ sizes, int32_t* __restrict__ status) {
+    const GraphView g{S.rstart, S.rlen, S.col};
+    for (int q = blockIdx.x * blockDim.x + threadIdx.x; q < count; q += gridDim.x * blockDim.x) {
+        int n_i, n_j;
+        status[q] = score_query_sizes<MODE>(S, g, pairs[2 * q], pairs[2 * q + 1], n_i, n_j);
+        sizes[2 * q] = n_i;
+        sizes[2 * q + 1] = n_j;
+    }
+}
+
+// Persistent grid: CTA b scores the queries b, b + gridDim.x, ... with the loop's own scoring step (score_pair) on its
+// slice of the caller's workspace (four scratch rows of `stride` ints).  Query q writes its candidate ids (nbI, then
+// nbJ) at cand + cand_offsets[q], its n_i x n_j fp64 cells at imp + cell_offsets[q] (IMP_MASKED64 = masked) and one
+// best record.  The state is only read: S arrives with its scratch pointers cleared (dcr_sdrf_score) and this copy's
+// score scratch points into the workspace.
+template <int MODE>
+__global__ void __launch_bounds__(SDRF_THREADS, 1)
+sdrf_score_kernel(SdrfDev S, const int32_t* __restrict__ pairs, int count, const int64_t* __restrict__ cell_offsets,
+                  const int64_t* __restrict__ cand_offsets, int32_t* __restrict__ cand, unsigned long long* imp,
+                  dcr_sdrf_score_best* __restrict__ best, int32_t* __restrict__ workspace, int stride) {
+    constexpr bool PAPER = MODE == LOOP_PAPER;
+    __shared__ std::conditional_t<PAPER, LoopSharedPaper, LoopShared> sh;
+    __shared__ DirScoreShared dsh;
+    __shared__ int dred[2];
+    const int tid = threadIdx.x;
+    const GraphView g{S.rstart, S.rlen, S.col};
+    const GraphView gin{S.rstart + S.n, S.rlen + S.n, S.col};
+    int32_t* ws = workspace + (long long)blockIdx.x * 4 * stride;   // this CTA's scratch: the copy S points at it
+    S.base1 = ws;
+    S.base2 = ws + stride;
+    S.posI = ws + 2 * stride;
+    S.posJ = ws + 3 * stride;
+    const ScoreScratch sc{S.base1, S.base2, S.posI, S.posJ};
+    for (int q = blockIdx.x; q < count; q += gridDim.x) {
+        const int x = pairs[2 * q], y = pairs[2 * q + 1];
+        dcr_sdrf_score_best* rec = best + q;
+        int n_i, n_j;
+        if (score_query_sizes<MODE>(S, g, x, y, n_i, n_j) != DCR_SDRF_OK) {   // (the sizes pass reported it)
+            if (tid == 0) *rec = {-1, -1, -1, -1, __longlong_as_double(-1ll)};
+            continue;
+        }
+        const CandList nbI{S.ord, S.rstart[x], n_i, x};
+        const CandList nbJ{S.ord, S.rstart[(MODE == LOOP_DIRECTED ? S.n : 0) + y], n_j, y};
+        int32_t* cq = cand + cand_offsets[q];
+        for (int t = tid; t < n_i + n_j; t += SDRF_THREADS) cq[t] = t < n_i ? nbI(t) : nbJ(t - n_i);
+        // C[x,y] of the state; 0 for a non-edge (the loop's (0,0) fallback, the reference's dense C)
+        const int sxy = edge_slot(g, x, y);
+        const float cxy = (!PAPER && sxy >= 0) ? S.c32[sxy] : 0.0f;
+        double cxy_d = 0.0;
+        if constexpr (PAPER) cxy_d = paper_get(S, sxy);               // (a paper query is an edge)
+        unsigned long long* out = imp + cell_offsets[q];
+        auto put = [=](int I, int J, float d) {    // the value the loop draws from, as fp64
+            out[(long long)I * n_j + J] =
+                d == MASKED_D ? IMP_MASKED64
+                              : (unsigned long long)__double_as_longlong(MODE == LOOP_CLASSICAL ? d : __fsub_rn(d, cxy));
+        };
+        score_pair<MODE>(S, g, gin, x, y, nbI, nbJ, sc, put, out, cxy_d, &sh, &dsh, dred, [] {});
+        __syncthreads();
+        // the best record: the first maximum in cell order (the loop's tau = inf selection) and its rank among the
+        // unmasked cells; thread t owns the contiguous cell range [t*L, (t+1)*L) as in the loop
+        const long long cells = (long long)n_i * n_j;
+        const long long L = (cells + SDRF_THREADS - 1) / SDRF_THREADS;
+        const long long f_lo = min(cells, (long long)tid * L), f_hi = min(cells, f_lo + L);
+        long long my_cnt = 0;
+        BestT<double> b{(double)INFINITY, ~0ull};
+        for (long long f = f_lo; f < f_hi; ++f) {
+            const unsigned long long bits = out[f];
+            if (bits == IMP_MASKED64) continue;
+            ++my_cnt;
+            b = best_of(b, BestT<double>{-__longlong_as_double((long long)bits), (unsigned long long)f});
+        }
+        long long n_cand;
+        const long long my_off = block_exscan_ll(my_cnt, &n_cand, &sh.red);
+        b = block_best(b, &sh.red);
+        const long long fstar = (long long)b.key;
+        if (n_cand == 0) {
+            if (tid == 0) *rec = {0, -1, -1, -1, __longlong_as_double(-1ll)};
+        } else if (fstar >= f_lo && fstar < f_hi) {
+            long long c = my_off;
+            for (long long f = f_lo; f < fstar; ++f) c += out[f] != IMP_MASKED64;
+            *rec = {n_cand, c, nbI((int)(fstar / n_j)), nbJ((int)(fstar % n_j)), __longlong_as_double((long long)out[fstar])};
+        }
+        __syncthreads();
+    }
+}
+
 // the kernels of the loop flavour that runs DCR_SDRF_MODE_* `mode`
 struct LoopKernels {
     decltype(&sdrf_init_curvature_kernel<LOOP_BFC>) init;
@@ -1267,11 +1411,14 @@ struct LoopKernels {
     decltype(&sdrf_batch_loop_kernel<LOOP_BFC>) batch;
     decltype(&sdrf_edit_kernel<LOOP_BFC>) edit;
     decltype(&sdrf_batch_edit_kernel<LOOP_BFC>) batch_edit;
+    decltype(&sdrf_score_sizes_kernel<LOOP_BFC>) score_sizes;
+    decltype(&sdrf_score_kernel<LOOP_BFC>) score;
 };
 template <int MODE>
 static LoopKernels loop_kernels_of() {
     return {sdrf_init_curvature_kernel<MODE>, sdrf_loop_kernel<MODE>, sdrf_batch_loop_kernel<MODE>,
-            sdrf_edit_kernel<MODE>, sdrf_batch_edit_kernel<MODE>};
+            sdrf_edit_kernel<MODE>, sdrf_batch_edit_kernel<MODE>, sdrf_score_sizes_kernel<MODE>,
+            sdrf_score_kernel<MODE>};
 }
 static LoopKernels loop_kernels(int mode) {
     switch (mode) {
@@ -1686,6 +1833,48 @@ extern "C" int dcr_sdrf_run_batch(const dcr_sdrf_batch_run* runs, int count, int
     DCR_CUDA(cudaMemcpyAsync(workspace, descs.data(), sizeof(SdrfBatchDesc) * count, cudaMemcpyHostToDevice, st));
     loop_kernels(runs[0].state->mode).batch<<<count, SDRF_THREADS, 0, st>>>((const SdrfBatchDesc*)workspace,
                                                                              remove_edges, guard);
+    DCR_LAUNCH_CHECK();
+    return 0;
+}
+
+// ints per scratch row of one CTA of sdrf_score_kernel (every candidate list is at most row_cap_max long)
+static int score_stride(const dcr_sdrf* s) { return (s->dev.row_cap_max + 63) / 64 * 64; }
+
+extern "C" int64_t dcr_sdrf_score_workspace_bytes(dcr_sdrf* s, int count) {
+    if (!s || count < 1) return 0;
+    return (int64_t)std::min(count, sm_count()) * 4 * score_stride(s) * (int64_t)sizeof(int32_t);
+}
+
+extern "C" int dcr_sdrf_score_sizes(dcr_sdrf* s, const int32_t* pairs, int count, int32_t* sizes, int32_t* status,
+                                    void* stream) {
+    if (!s || count < 1 || !pairs || !sizes || !status) { set_error("dcr_sdrf_score_sizes: bad arguments"); return 1; }
+    const int ctas = std::max(1, std::min((count + 255) / 256, sm_count() * 8));
+    loop_kernels(s->mode).score_sizes<<<ctas, 256, 0, (cudaStream_t)stream>>>(s->dev, pairs, count, sizes, status);
+    DCR_LAUNCH_CHECK();
+    return 0;
+}
+
+extern "C" int dcr_sdrf_score(dcr_sdrf* s, const int32_t* pairs, int count, const int64_t* cell_offsets,
+                              const int64_t* cand_offsets, int32_t* cand, double* imp, dcr_sdrf_score_best* best,
+                              void* workspace, int64_t workspace_bytes, void* stream) {
+    if (!s || count < 1 || !pairs || !cell_offsets || !cand_offsets || !cand || !imp || !best) {
+        set_error("dcr_sdrf_score: bad arguments");
+        return 1;
+    }
+    if (!workspace || workspace_bytes < dcr_sdrf_score_workspace_bytes(s, count)) {
+        set_error("dcr_sdrf_score: workspace of dcr_sdrf_score_workspace_bytes(state, %d) = %lld bytes required", count,
+                  (long long)dcr_sdrf_score_workspace_bytes(s, count));
+        return 1;
+    }
+    if ((uintptr_t)workspace % 4) { set_error("dcr_sdrf_score: workspace must be 4-byte aligned"); return 1; }
+    // the kernel reads the state only: its copy has no scratch, so a write to the state's own scratch cannot happen
+    SdrfDev D = s->dev;
+    D.base1 = D.base2 = D.posI = D.posJ = D.dirty = D.work = D.wlist = nullptr;
+    D.imp = nullptr;
+    D.pend = nullptr;
+    loop_kernels(s->mode).score<<<std::min(count, sm_count()), SDRF_THREADS, 0, (cudaStream_t)stream>>>(
+        D, pairs, count, cell_offsets, cand_offsets, cand, reinterpret_cast<unsigned long long*>(imp), best,
+        (int32_t*)workspace, score_stride(s));
     DCR_LAUNCH_CHECK();
     return 0;
 }

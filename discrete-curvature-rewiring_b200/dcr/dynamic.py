@@ -18,6 +18,7 @@ from .sdrf import (CLASSICAL_MODES, _batch_return, _batch_uniforms, _loop_mode, 
                    _run_batch_states, _run_state, edit_batch_states)
 
 _INT32_MAX = 2**31 - 1
+_MASKED64 = np.uint64(0xFFFFFFFFFFFFFFFF)      # a masked cell of dcr_sdrf_score
 
 
 def align_to_columns(rowptr: np.ndarray, col: np.ndarray, values: np.ndarray, edge_index: np.ndarray,
@@ -204,6 +205,64 @@ class DynamicCurvature:
             val = val.astype(np.int64)                          # small integers, exact in the fp32 store
             loop_values = classical_loop_values(np.diff(rp.astype(np.int64)), self.curv_type)
         return align_to_columns(rp, col, val, ei, loop_values)
+
+    # ---- candidate scoring ----------------------------------------------------------------------------------------
+    def _score(self, pairs, max_cells: int):
+        """``dcr.sdrf.SdrfState.score`` of ``pairs``, ``None`` for no pairs.  Ids outside ``[0, n)`` raise here, the pairs
+        the mode's loop cannot score on the device; both before the scoring launch."""
+        device = self._state.device
+        p = pair_array(pairs)
+        if not np.issubdtype(p.dtype, np.integer):
+            raise ValueError(f"pairs: integer (x, y) expected, got {p.dtype}")
+        out_of_range = np.flatnonzero(((p < 0) | (p >= self.n)).any(axis=1))
+        if out_of_range.size:       # (checked here: the device takes int32 ids)
+            q = int(out_of_range[0])
+            raise ValueError(f"pairs[{q}] = ({int(p[q, 0])}, {int(p[q, 1])}): node ids must lie in [0, {self.n})")
+        if p.shape[0] == 0:
+            return None
+        return self._state.score(torch.from_numpy(p.astype(np.int32)).to(device), int(max_cells))
+
+    def improvements(self, pairs, *, max_cells: int = 1 << 27) -> list:
+        """For every pair ``(x, y)`` of the ``[Q, 2]`` array ``pairs``: ``(candidates, improvements)``, the int64 ``[m, 2]``
+        candidate edges ``(i, j)`` and the fp64 ``[m]`` improvement of the curvature of ``(x, y)`` if ``(i, j)`` is
+        added — exactly the candidates and the ``improvements`` array ``sdrf()`` draws from when its loop picks ``(x, y)``,
+        in its order (``i`` from ``x``'s list, ``j`` from ``y``'s; the classical and paper loops log the chosen pair
+        sorted).  The values: fp32 ``D - C[x,y]`` for ``'bfc'``, the integer improvement for ``'1d'`` / ``'augmented'`` /
+        ``'haantjes'``, the fp64 difference for ``'bfc_paper'``.
+        Valid pairs are those the loop can pick: ``'bfc'`` any nodes (a non-edge and ``x == y`` included, with
+        ``C[x,y] = 0``; directed: ``x``'s successors times ``y``'s predecessors); the classical modes an edge in either
+        orientation or ``(u, u)`` of a node with a self-loop; ``'bfc_paper'`` an edge.  Another pair raises ``ValueError``
+        naming its index, and so do queries whose candidate cells exceed ``max_cells`` (8 bytes of device output each);
+        both before the scoring launch.  One launch for all pairs, one CTA per pair; the object is left unchanged and no
+        budget is charged."""
+        out = self._score(pairs, max_cells)
+        if out is None:
+            return []
+        sizes = out["sizes"].cpu().numpy().astype(np.int64)
+        cand_off = out["cand_offsets"].cpu().numpy()
+        cell_off = out["cell_offsets"].cpu().numpy()
+        cand = out["cand"].cpu().numpy().astype(np.int64)
+        imp = out["imp"].cpu().numpy()
+        res = []
+        for q, (n_i, n_j) in enumerate(sizes.tolist()):
+            rows = cand[cand_off[q]: cand_off[q] + n_i]
+            cols = cand[cand_off[q] + n_i: cand_off[q + 1]]
+            cells = imp[cell_off[q]: cell_off[q + 1]]
+            flat = np.flatnonzero(cells.view(np.uint64) != _MASKED64)
+            res.append((np.stack([rows[flat // n_j], cols[flat % n_j]], axis=1), cells[flat]))
+        return res
+
+    def best_additions(self, pairs, *, max_cells: int = 1 << 27):
+        """The greedy (``tau = inf``) choice of the loop for every pair of ``pairs`` (see :meth:`improvements`):
+        ``(additions [Q, 2] int64, improvement [Q] fp64, n_candidates [Q] int64)``, the first candidate of maximal
+        improvement in the loop's order; ``(-1, -1)`` and NaN for a pair without candidates.  Only the Q best records are
+        copied to the host."""
+        out = self._score(pairs, max_cells)
+        if out is None:
+            return np.zeros((0, 2), dtype=np.int64), np.zeros(0), np.zeros(0, dtype=np.int64)
+        rec = out["best"].cpu().numpy()
+        ij = np.ascontiguousarray(rec[:, 2]).view(np.int32).reshape(-1, 2).astype(np.int64)
+        return ij, np.ascontiguousarray(rec[:, 3]).view(np.float64), rec[:, 0].copy()
 
     # ---- SDRF ---------------------------------------------------------------------------------------------------
     def rewire(self, loops: int, remove_edges: bool, removal_bound: float, tau, *, uniforms=None,

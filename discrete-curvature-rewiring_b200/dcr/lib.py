@@ -26,7 +26,7 @@ class SdrfEditRun(C.Structure):
 
 # status codes of include/dcr.h
 SDRF_OK, SDRF_NEED_HOST, SDRF_PROB_NAN, SDRF_PROB_SUM, SDRF_REMOVE_NONEDGE, SDRF_NO_UNIFORM, SDRF_ARENA_FULL, \
-    SDRF_TOO_MANY_CANDIDATES, SDRF_EMPTY_GRAPH, SDRF_BAD_EDIT = range(10)
+    SDRF_TOO_MANY_CANDIDATES, SDRF_EMPTY_GRAPH, SDRF_BAD_EDIT, SDRF_BAD_QUERY = range(11)
 SDRF_MODE_BFC, SDRF_MODE_BFC_DIRECTED, SDRF_MODE_1D, SDRF_MODE_AUGMENTED, SDRF_MODE_HAANTJES, SDRF_MODE_BFC_PAPER = range(6)
 SDRF_LOG_INTS = 8
 
@@ -91,6 +91,9 @@ SIGNATURES = {
     "dcr_sdrf_export_order": (_I, [_P, _P, _P, _P]),
     "dcr_sdrf_export_c64": (_I, [_P, _P, _P, _P]),
     "dcr_sdrf_export_edge_index": (_I, [_P, _P, _P, _P, _L, _P]),
+    "dcr_sdrf_score_sizes": (_I, [_P, _P, _I, _P, _P, _P]),
+    "dcr_sdrf_score_workspace_bytes": (_L, [_P, _I]),
+    "dcr_sdrf_score": (_I, [_P, _P, _I, _P, _P, _P, _P, _P, _P, _L, _P]),
 }
 
 _lib = None

@@ -20,6 +20,15 @@ _MSG_NAN = "probabilities contain NaN"
 _MSG_SUM = "probabilities do not sum to 1"
 # the fields of dcr_sdrf_result that the host reads, in record order
 _RESULT_KEYS = ("status", "iterations_done", "draws_used", "stopped", "pending_n", "pending_x", "pending_y")
+# the pairs each loop mode scores (dcr_sdrf_score_sizes), for the message of a rejected query
+_QUERY_RULE = {
+    L.SDRF_MODE_BFC: "node ids must lie in [0, n)",
+    L.SDRF_MODE_BFC_DIRECTED: "node ids must lie in [0, n)",
+    L.SDRF_MODE_1D: "not an edge of the graph (nor (u, u) of a node with a self-loop)",
+    L.SDRF_MODE_AUGMENTED: "not an edge of the graph (nor (u, u) of a node with a self-loop)",
+    L.SDRF_MODE_HAANTJES: "not an edge of the graph (nor (u, u) of a node with a self-loop)",
+    L.SDRF_MODE_BFC_PAPER: "not an edge of the graph",
+}
 
 
 def host_choice(improvements: np.ndarray, tau, u: float) -> int:
@@ -122,6 +131,46 @@ class SdrfState:
         L.check(self.lib.dcr_sdrf_edit(self.handle, L.ptr(e) if e.numel() else 0, int(e.shape[0]),
                                        self._result.data_ptr(), L.current_stream()), "dcr_sdrf_edit")
         return dict(zip(_RESULT_KEYS, self._result.cpu().tolist()))
+
+    def score(self, pairs: torch.Tensor, max_cells: int | None = None) -> dict:
+        """Candidate scores of the Q >= 1 pairs ``(x, y)`` of the device int32 ``[Q, 2]`` tensor ``pairs``
+        (``dcr_sdrf_score_sizes``, one read of the totals, ``dcr_sdrf_score``).  Returns device tensors:
+        ``sizes`` int32 ``[Q, 2]`` ``(n_i, n_j)``; ``cand_offsets`` / ``cell_offsets`` int64 ``[Q + 1]``; ``cand`` int32
+        (query q: its ``n_i`` row ids, then its ``n_j`` column ids); ``imp`` fp64 cells, row-major per query, a masked cell
+        with all bits set; ``best`` int64 ``[Q, 4]``, the ``dcr_sdrf_score_best`` records.  Raises ``ValueError`` for the
+        first pair this mode's loop cannot score, or when the cells exceed ``max_cells``, before the scoring launch."""
+        q = int(pairs.shape[0])
+        dev = self.device
+        sizes = torch.empty((q, 2), dtype=torch.int32, device=dev)
+        status = torch.empty(q, dtype=torch.int32, device=dev)
+        L.check(self.lib.dcr_sdrf_score_sizes(self.handle, pairs.data_ptr(), q, sizes.data_ptr(), status.data_ptr(),
+                                              L.current_stream()), "dcr_sdrf_score_sizes")
+        s64 = sizes.to(torch.int64)
+        cell_offsets = torch.zeros(q + 1, dtype=torch.int64, device=dev)
+        cand_offsets = torch.zeros(q + 1, dtype=torch.int64, device=dev)
+        torch.cumsum(s64[:, 0] * s64[:, 1], 0, out=cell_offsets[1:])
+        torch.cumsum(s64.sum(1), 0, out=cand_offsets[1:])
+        bad = status != L.SDRF_OK
+        first_bad = torch.where(bad.any(), torch.argmax(bad.to(torch.int32)), -1)
+        cells, cands, first_bad = torch.stack([cell_offsets[-1], cand_offsets[-1], first_bad]).cpu().tolist()
+        if first_bad >= 0:
+            st, (x, y) = int(status[first_bad]), pairs[first_bad].tolist()
+            if st != L.SDRF_BAD_QUERY:
+                _raise_for_status(st)
+            raise ValueError(f"pairs[{first_bad}] = ({x}, {y}): {_QUERY_RULE[self.mode]}")
+        if max_cells is not None and cells > max_cells:
+            raise ValueError(f"the {q} queries have {cells} candidate cells, more than max_cells = {max_cells} "
+                             f"({8 * cells + 4 * cands} bytes of output)")
+        cand = torch.empty(max(cands, 1), dtype=torch.int32, device=dev)
+        imp = torch.empty(max(cells, 1), dtype=torch.float64, device=dev)
+        best = torch.empty((q, 4), dtype=torch.int64, device=dev)
+        nbytes = int(self.lib.dcr_sdrf_score_workspace_bytes(self.handle, q))
+        workspace = torch.empty(max(nbytes // 4, 1), dtype=torch.int32, device=dev)
+        L.check(self.lib.dcr_sdrf_score(self.handle, pairs.data_ptr(), q, cell_offsets.data_ptr(), cand_offsets.data_ptr(),
+                                        cand.data_ptr(), imp.data_ptr(), best.data_ptr(), workspace.data_ptr(), nbytes,
+                                        L.current_stream()), "dcr_sdrf_score")
+        return {"sizes": sizes, "cand_offsets": cand_offsets, "cell_offsets": cell_offsets, "cand": cand[:cands],
+                "imp": imp[:cells], "best": best}
 
     def pending_improvements(self, n: int) -> np.ndarray:
         out = torch.empty(max(n, 1), dtype=torch.float64, device=self.device)

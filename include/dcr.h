@@ -40,6 +40,7 @@ extern "C" {
 #define DCR_SDRF_TOO_MANY_CANDIDATES 7 /* (deg x+1)(deg y+1) exceeds the candidate scratch of the state          */
 #define DCR_SDRF_EMPTY_GRAPH 8    /* classical loop on a graph without edges (python: min() of an empty sequence)  */
 #define DCR_SDRF_BAD_EDIT 9       /* dcr_sdrf_edit: an edit with u == v, an id outside [0, n) or an op other than 0/1 */
+#define DCR_SDRF_BAD_QUERY 10     /* dcr_sdrf_score_sizes: a pair the loop of this mode cannot score                */
 
 /* loop flavours of dcr_sdrf_create_mode */
 #define DCR_SDRF_MODE_BFC 0          /* sdrf_cuda_bfc(..., is_undirected=True)   rewiring/sdrf_cuda_bfc.py:14-93        */
@@ -375,6 +376,35 @@ int dcr_sdrf_export_edge_index(dcr_sdrf* s, int32_t* rowptr_order, int64_t* src,
  * SORTED order per row (the layout of dcr_sdrf_export's colidx_sorted / c32_sorted).  That mode keeps no fp32 curvature
  * and no supports. */
 int dcr_sdrf_export_c64(dcr_sdrf* s, int32_t* rowptr, double* c64_sorted, void* stream);
+
+/* Candidate scoring of many pairs (x, y) on a loop state: "if (i, j) is added, how much does the curvature of (x, y)
+ * improve?" for every (i, j) of the candidate lists the loop would build for (x, y).  Valid pairs are those the loop
+ * itself can score: BFC and BFC_DIRECTED any 0 <= x, y < n (a non-edge and x == y included; C[x,y] = 0 there);
+ * 1D / AUGMENTED / HAANTJES an edge in either orientation, or (u, u) for a node that lists itself; BFC_PAPER an edge.
+ * x's list gives the rows (its insertion-order row, then x; BFC_DIRECTED: its successors), y's the columns (BFC_DIRECTED:
+ * its predecessors).  Both calls only enqueue, allocate nothing and never write the state; status 1 for count < 1, a
+ * null state or pointer, or a short workspace.
+ * dcr_sdrf_score_sizes: per query, sizes[2q] = n_i and sizes[2q+1] = n_j (0 for a rejected query) and status[q] =
+ * DCR_SDRF_OK, DCR_SDRF_BAD_QUERY or DCR_SDRF_TOO_MANY_CANDIDATES (a row longer than the state's scratch rows, after
+ * loop iterations beyond max_additions).  pairs: device int32[count][2]; sizes, status: device int32.
+ * dcr_sdrf_score: a persistent grid of min(count, #SMs) CTAs, one query per CTA at a time.  Query q writes its candidate
+ * ids (the n_i row ids, then the n_j column ids) at cand + cand_offsets[q], its n_i x n_j cells row-major at
+ * imp + cell_offsets[q] and best[q].  A cell is the value the loop draws from, as fp64: fp32(D - C[x,y]) for BFC and
+ * BFC_DIRECTED, the integer improvement for the classical modes, the fp64 difference for BFC_PAPER; a masked cell
+ * (i == j or (i, j) an edge) has all bits set (a NaN).  workspace: device memory of at least
+ * dcr_sdrf_score_workspace_bytes(s, count) bytes, 4-byte aligned.  A query rejected by the sizes pass writes only best[q]
+ * (n_candidates = -1). */
+typedef struct dcr_sdrf_score_best {
+    int64_t n_candidates;    /* unmasked cells                                                                      */
+    int64_t choice;          /* index among the unmasked cells of the first maximum (the loop's tau = inf choice)    */
+    int32_t i, j;            /* the candidate at that cell                                                          */
+    double improvement;      /* its improvement; choice = i = j = -1 and a NaN when there is no candidate           */
+} dcr_sdrf_score_best;
+int dcr_sdrf_score_sizes(dcr_sdrf* s, const int32_t* pairs, int count, int32_t* sizes, int32_t* status, void* stream);
+int64_t dcr_sdrf_score_workspace_bytes(dcr_sdrf* s, int count);
+int dcr_sdrf_score(dcr_sdrf* s, const int32_t* pairs, int count, const int64_t* cell_offsets,
+                   const int64_t* cand_offsets, int32_t* cand, double* imp, dcr_sdrf_score_best* best, void* workspace,
+                   int64_t workspace_bytes, void* stream);
 
 #ifdef __cplusplus
 }

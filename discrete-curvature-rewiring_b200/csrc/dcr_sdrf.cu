@@ -17,7 +17,9 @@
 // (iteration t+1 needs the graph of iteration t), hence one CTA per run; independent runs go side by side, one CTA
 // each, in one launch of the batch kernel (dcr_sdrf_run_batch).
 #include <algorithm>
+#include <atomic>
 #include <cmath>
+#include <cstdio>
 #include <type_traits>
 #include <vector>
 
@@ -629,40 +631,121 @@ __device__ void paper_score(const SdrfDev& S, const GraphView& g, int x, int y, 
 // ------------------------------------------------------------------------------------------------------------
 // initialisation kernels over arena slots (multi-CTA)
 // ------------------------------------------------------------------------------------------------------------
+// One warp per arena slot s.  The single-state kernels and the batched ones of dcr_sdrf_create_batch call the same
+// per-entry bodies, so a value is computed by the same code on either path.
+__device__ __forceinline__ void init_support_entry(const SdrfDev& S, int s, int lane) {
+    const int a = S.owner[s];
+    if (a < 0) return;
+    const int c = warp_intersect_count(GraphView{S.rstart, S.rlen, S.col}, a, S.col[s], lane);
+    if (lane == 0) S.supp[s] = c;
+}
+template <int MODE>
+__device__ __forceinline__ void init_curvature_entry(const SdrfDev& S, int s, int lane) {
+    const int a = S.owner[s];
+    if (a < 0) return;
+    if constexpr (MODE == LOOP_PAPER) {
+        const double c = paper_eval(PaperView{{S.rstart, S.rlen, S.col}, -1, -1}, a, S.col[s], lane);
+        if (lane == 0) paper_put(S, s, c);
+        return;
+    }
+    float c;
+    if constexpr (MODE == LOOP_DIRECTED) {
+        if (a >= S.n) return;                   // predecessor rows carry no curvature
+        const GraphView gout{S.rstart, S.rlen, S.col}, gin{S.rstart + S.n, S.rlen + S.n, S.col};
+        c = directed_entry_curvature(gout, gin, a, S.col[s], lane).c32;
+    } else if constexpr (MODE == LOOP_CLASSICAL) {
+        c = classical_curvature(S, a, S.col[s], s);
+    } else {
+        c = entry_curvature(S, a, S.col[s], s, lane);
+    }
+    if (lane == 0) S.c32[s] = c;
+}
 __global__ void sdrf_init_support_kernel(SdrfDev S, int top) {
     const int lane = threadIdx.x & 31;
     const int warps = (gridDim.x * blockDim.x) >> 5;
-    GraphView g{S.rstart, S.rlen, S.col};
-    for (int s = (blockIdx.x * blockDim.x + threadIdx.x) >> 5; s < top; s += warps) {
-        const int a = S.owner[s];
-        if (a < 0) continue;
-        const int c = warp_intersect_count(g, a, S.col[s], lane);
-        if (lane == 0) S.supp[s] = c;
-    }
+    for (int s = (blockIdx.x * blockDim.x + threadIdx.x) >> 5; s < top; s += warps) init_support_entry(S, s, lane);
 }
 template <int MODE>
 __global__ void sdrf_init_curvature_kernel(SdrfDev S, int top) {
     const int lane = threadIdx.x & 31;
     const int warps = (gridDim.x * blockDim.x) >> 5;
-    for (int s = (blockIdx.x * blockDim.x + threadIdx.x) >> 5; s < top; s += warps) {
-        const int a = S.owner[s];
-        if (a < 0) continue;
-        if constexpr (MODE == LOOP_PAPER) {
-            const double c = paper_eval(PaperView{{S.rstart, S.rlen, S.col}, -1, -1}, a, S.col[s], lane);
-            if (lane == 0) paper_put(S, s, c);
-            continue;
-        }
-        float c;
-        if constexpr (MODE == LOOP_DIRECTED) {
-            if (a >= S.n) continue;                 // predecessor rows carry no curvature
-            const GraphView gout{S.rstart, S.rlen, S.col}, gin{S.rstart + S.n, S.rlen + S.n, S.col};
-            c = directed_entry_curvature(gout, gin, a, S.col[s], lane).c32;
-        } else if constexpr (MODE == LOOP_CLASSICAL) {
-            c = classical_curvature(S, a, S.col[s], s);
+    for (int s = (blockIdx.x * blockDim.x + threadIdx.x) >> 5; s < top; s += warps) init_curvature_entry<MODE>(S, s, lane);
+}
+
+// ------------------------------------------------------------------------------------------------------------
+// set-up of many states in one pass (dcr_sdrf_create_batch)
+// ------------------------------------------------------------------------------------------------------------
+// Per-state record of the batched set-up; `stage` points at the state's part of the packed staging buffer:
+// rstart, rlen, rcap, selfl [rows each], col, ord, owner [used each], scalars [8], all int32.
+struct SdrfInitDesc {
+    SdrfDev S;
+    const int32_t* stage;
+    int rows, used;       // used: arena slots filled at set-up (sum of the row capacities)
+};
+static_assert(sizeof(SdrfInitDesc) % 8 == 0, "descriptor table packed as 8-byte words");
+
+// the state whose range [off[b], off[b+1]) holds t (off: count+1 non-decreasing offsets, off[0] = 0 <= t < off[count])
+__device__ __forceinline__ int state_of(const long long* __restrict__ off, int count, long long t) {
+    int lo = 0, hi = count - 1;
+    while (lo < hi) {
+        const int mid = (lo + hi + 1) >> 1;
+        if (off[mid] <= t) lo = mid; else hi = mid - 1;
+    }
+    return lo;
+}
+
+// Fills every state's persistent arrays from the staging buffer and clears the rest of its arena, as
+// sdrf_create_impl's copies and memsets do: unit t of state b is arena slot t (t < cap_total) or row t - cap_total.
+// off[b] = sum over earlier states of cap_total + rows.
+__global__ void sdrf_batch_setup_kernel(const SdrfInitDesc* __restrict__ descs, const long long* __restrict__ off,
+                                        int count) {
+    const long long total = off[count];
+    for (long long t = blockIdx.x * (long long)blockDim.x + threadIdx.x; t < total;
+         t += (long long)gridDim.x * blockDim.x) {
+        const int b = state_of(off, count, t);
+        const SdrfInitDesc& d = descs[b];
+        const SdrfDev& S = d.S;
+        const long long i = t - off[b];
+        const int32_t* st = d.stage;
+        if (i < S.cap_total) {
+            const int s = (int)i;
+            const int32_t* cols = st + 4 * d.rows;
+            if (s < d.used) {
+                S.col[s] = cols[s];
+                S.ord[s] = cols[d.used + s];
+            }
+            S.owner[s] = s < d.used ? cols[2 * d.used + s] : -1;
+            S.flag[s] = 0;
+            S.supp[s] = 0;
+            S.c32[s] = 0.0f;
+            if (s < 8) S.scalars[s] = cols[3 * d.used + s];
         } else {
-            c = entry_curvature(S, a, S.col[s], s, lane);
+            const int r = (int)(i - S.cap_total);
+            S.rstart[r] = st[r];
+            S.rlen[r] = st[d.rows + r];
+            S.rcap[r] = st[2 * d.rows + r];
+            S.selfl[r] = st[3 * d.rows + r];
         }
-        if (lane == 0) S.c32[s] = c;
+    }
+}
+// one warp per filled arena slot of every state (off[b] = sum over earlier states of `used`)
+__global__ void sdrf_batch_init_support_kernel(const SdrfInitDesc* __restrict__ descs, const long long* __restrict__ off,
+                                               int count) {
+    const int lane = threadIdx.x & 31;
+    const long long warps = ((long long)gridDim.x * blockDim.x) >> 5;
+    for (long long w = (blockIdx.x * (long long)blockDim.x + threadIdx.x) >> 5; w < off[count]; w += warps) {
+        const int b = state_of(off, count, w);
+        init_support_entry(descs[b].S, (int)(w - off[b]), lane);
+    }
+}
+template <int MODE>
+__global__ void sdrf_batch_init_curvature_kernel(const SdrfInitDesc* __restrict__ descs,
+                                                 const long long* __restrict__ off, int count) {
+    const int lane = threadIdx.x & 31;
+    const long long warps = ((long long)gridDim.x * blockDim.x) >> 5;
+    for (long long w = (blockIdx.x * (long long)blockDim.x + threadIdx.x) >> 5; w < off[count]; w += warps) {
+        const int b = state_of(off, count, w);
+        init_curvature_entry<MODE>(descs[b].S, (int)(w - off[b]), lane);
     }
 }
 
@@ -1413,12 +1496,13 @@ struct LoopKernels {
     decltype(&sdrf_batch_edit_kernel<LOOP_BFC>) batch_edit;
     decltype(&sdrf_score_sizes_kernel<LOOP_BFC>) score_sizes;
     decltype(&sdrf_score_kernel<LOOP_BFC>) score;
+    decltype(&sdrf_batch_init_curvature_kernel<LOOP_BFC>) batch_init;
 };
 template <int MODE>
 static LoopKernels loop_kernels_of() {
     return {sdrf_init_curvature_kernel<MODE>, sdrf_loop_kernel<MODE>, sdrf_batch_loop_kernel<MODE>,
             sdrf_edit_kernel<MODE>, sdrf_batch_edit_kernel<MODE>, sdrf_score_sizes_kernel<MODE>,
-            sdrf_score_kernel<MODE>};
+            sdrf_score_kernel<MODE>, sdrf_batch_init_curvature_kernel<MODE>};
 }
 static LoopKernels loop_kernels(int mode) {
     switch (mode) {
@@ -1433,6 +1517,9 @@ static LoopKernels loop_kernels(int mode) {
 // export
 // ------------------------------------------------------------------------------------------------------------
 // with_self: row lengths of the INSERTION-ORDER rows (a node that lists itself has one entry more)
+__device__ __forceinline__ int export_row_len(const SdrfDev& S, int v, int with_self) {
+    return S.rlen[v] + (with_self ? S.selfl[v] : 0);
+}
 __global__ void sdrf_export_rowptr_kernel(SdrfDev S, int32_t* rowptr, int with_self) {
     __shared__ Reduce red;
     // single CTA: chunked exclusive scan of rlen
@@ -1440,10 +1527,10 @@ __global__ void sdrf_export_rowptr_kernel(SdrfDev S, int32_t* rowptr, int with_s
     const int L = (n + SDRF_THREADS - 1) / SDRF_THREADS;
     const int lo = min(n, (int)threadIdx.x * L), hi = min(n, lo + L);
     long long s = 0;
-    for (int v = lo; v < hi; ++v) s += S.rlen[v] + (with_self ? S.selfl[v] : 0);
+    for (int v = lo; v < hi; ++v) s += export_row_len(S, v, with_self);
     long long total;
     long long off = block_exscan_ll(s, &total, &red);
-    for (int v = lo; v < hi; ++v) { rowptr[v] = (int32_t)off; off += S.rlen[v] + (with_self ? S.selfl[v] : 0); }
+    for (int v = lo; v < hi; ++v) { rowptr[v] = (int32_t)off; off += export_row_len(S, v, with_self); }
     if (threadIdx.x == 0) rowptr[n] = (int32_t)total;
 }
 __global__ void sdrf_export_order_kernel(SdrfDev S, const int32_t* rowptr, int32_t* order_out) {
@@ -1480,26 +1567,78 @@ __global__ void sdrf_export_c64_kernel(SdrfDev S, const int32_t* rowptr, double*
 // ascending, which is the prefix of its sorted arena row, then its neighbours >= w (its self entry included) in insertion
 // order.  directed: the successor rows as they are (G.from_digraph_order).  One warp per row; `rowptr` comes from
 // sdrf_export_rowptr_kernel(with_self = 1).  Nothing is written at or beyond `capacity`.
+// Row w of one state, written from column o on with the node ids shifted by `shift` (the batched export's node offset).
+__device__ __forceinline__ void export_edge_row(const SdrfDev& S, int w, long long o, long long shift, int64_t* src,
+                                                int64_t* dst, long long capacity, int directed, int lane) {
+    const int s = S.rstart[w], len = S.rlen[w], olen = len + S.selfl[w];
+    const int lo = directed ? 0 : lower_bound(S.col, s, len, w);
+    for (int t = lane; t < lo; t += 32)
+        if (o + t < capacity) { src[o + t] = w + shift; dst[o + t] = S.col[s + t] + shift; }
+    o += lo;
+    for (int base = 0; base < olen; base += 32) {
+        const int t = base + lane;
+        const int x = t < olen ? S.ord[s + t] : -1;
+        const bool keep = t < olen && (directed || x >= w);
+        const unsigned m = __ballot_sync(FULL, keep);
+        const long long p = o + __popc(m & ((1u << lane) - 1u));
+        if (keep && p < capacity) { src[p] = w + shift; dst[p] = x + shift; }
+        o += __popc(m);
+    }
+}
 __global__ void sdrf_export_edge_index_kernel(SdrfDev S, const int32_t* rowptr, int64_t* src, int64_t* dst,
                                               long long capacity, int directed) {
     const int lane = threadIdx.x & 31;
     const int warps = (gridDim.x * blockDim.x) >> 5;
-    for (int w = (blockIdx.x * blockDim.x + threadIdx.x) >> 5; w < S.n; w += warps) {
-        const int s = S.rstart[w], len = S.rlen[w], olen = len + S.selfl[w];
-        const int lo = directed ? 0 : lower_bound(S.col, s, len, w);
-        long long o = rowptr[w];
-        for (int t = lane; t < lo; t += 32)
-            if (o + t < capacity) { src[o + t] = w; dst[o + t] = S.col[s + t]; }
-        o += lo;
-        for (int base = 0; base < olen; base += 32) {
-            const int t = base + lane;
-            const int x = t < olen ? S.ord[s + t] : -1;
-            const bool keep = t < olen && (directed || x >= w);
-            const unsigned m = __ballot_sync(FULL, keep);
-            const long long p = o + __popc(m & ((1u << lane) - 1u));
-            if (keep && p < capacity) { src[p] = w; dst[p] = x; }
-            o += __popc(m);
-        }
+    for (int w = (blockIdx.x * blockDim.x + threadIdx.x) >> 5; w < S.n; w += warps)
+        export_edge_row(S, w, rowptr[w], 0, src, dst, capacity, directed, lane);
+}
+
+// ---- the batched export (dcr_sdrf_export_edge_index_batch): all states' rows in three launches
+struct SdrfExportDesc {
+    SdrfDev S;
+    long long node_offset;    // added to every node id of the state
+};
+static_assert(sizeof(SdrfExportDesc) % 8 == 0, "descriptor table packed as 8-byte words");
+
+// 1. counts[r] = export_row_len of global row r (row_off[b] = sum over earlier states of n)
+__global__ void sdrf_batch_export_counts_kernel(const SdrfExportDesc* __restrict__ descs,
+                                                const long long* __restrict__ row_off, int count,
+                                                long long* __restrict__ counts) {
+    for (long long r = blockIdx.x * (long long)blockDim.x + threadIdx.x; r < row_off[count];
+         r += (long long)gridDim.x * blockDim.x) {
+        const int b = state_of(row_off, count, r);
+        counts[r] = export_row_len(descs[b].S, (int)(r - row_off[b]), 1);
+    }
+}
+// 2. single CTA: counts[0 .. R) becomes its exclusive prefix (in place), edge_ptr[b] = the first column of state b and
+//    edge_ptr[count] = the total
+__global__ void __launch_bounds__(SDRF_THREADS, 1)
+sdrf_batch_export_scan_kernel(const long long* __restrict__ row_off, int count, long long* counts,
+                              int64_t* __restrict__ edge_ptr) {
+    __shared__ Reduce red;
+    const long long R = row_off[count];
+    const long long L = (R + SDRF_THREADS - 1) / SDRF_THREADS;
+    const long long lo = min(R, (long long)threadIdx.x * L), hi = min(R, lo + L);
+    long long s = 0;
+    for (long long r = lo; r < hi; ++r) s += counts[r];
+    long long total;
+    long long off = block_exscan_ll(s, &total, &red);
+    for (long long r = lo; r < hi; ++r) { const long long c = counts[r]; counts[r] = off; off += c; }
+    __syncthreads();
+    for (int b = threadIdx.x; b < count; b += SDRF_THREADS) edge_ptr[b] = row_off[b] < R ? counts[row_off[b]] : total;
+    if (threadIdx.x == 0) edge_ptr[count] = total;
+}
+// 3. one warp per global row, from column rowptr[r]
+__global__ void sdrf_batch_export_rows_kernel(const SdrfExportDesc* __restrict__ descs,
+                                              const long long* __restrict__ row_off, int count,
+                                              const long long* __restrict__ rowptr, int64_t* src, int64_t* dst,
+                                              long long capacity, int directed) {
+    const int lane = threadIdx.x & 31;
+    const long long warps = ((long long)gridDim.x * blockDim.x) >> 5;
+    for (long long r = (blockIdx.x * (long long)blockDim.x + threadIdx.x) >> 5; r < row_off[count]; r += warps) {
+        const int b = state_of(row_off, count, r);
+        const SdrfExportDesc& d = descs[b];
+        export_edge_row(d.S, (int)(r - row_off[b]), rowptr[r], d.node_offset, src, dst, capacity, directed, lane);
     }
 }
 __global__ void sdrf_copy_pending_kernel(const double* pend, double* out, long long n) {
@@ -1511,12 +1650,20 @@ __global__ void sdrf_copy_pending_kernel(const double* pend, double* out, long l
 
 using namespace dcr;
 
+// Slabs of the states of one dcr_sdrf_create_batch call live in one allocation; each state holds a reference and the
+// last dcr_sdrf_destroy frees it.
+struct SdrfPool {
+    void* base;
+    std::atomic<int> refs;
+};
+
 struct dcr_sdrf {
     SdrfDev dev;
-    void* slab;           // one allocation backing every array
+    void* slab;           // one allocation backing every array (a pooled state: its part of the pool)
     size_t slab_bytes;
     int mode;             // DCR_SDRF_MODE_*
     int64_t n_self;       // nodes that list themselves (self-loops of G)
+    SdrfPool* pool;       // null: the state owns `slab`
 };
 
 template <class T>
@@ -1545,21 +1692,27 @@ static void carve_slab(SdrfDev& D, char* p, int rows, bool paper) {
 }
 static size_t persistent_bytes(const dcr_sdrf* s) { return (size_t)((char*)s->dev.base1 - (char*)s->slab); }
 
-// rows [0,n): rowptr/order (neighbours, or successors in the directed mode); rows [n,2n): in_rowptr/in_order
-// (predecessors, directed mode only)
-static int sdrf_create_impl(int n, int mode, const int32_t* rowptr_host, const int32_t* order_host,
-                            const int32_t* in_rowptr_host, const int32_t* in_order_host, int64_t max_additions,
-                            dcr_sdrf** out) {
-    if (n <= 0 || !rowptr_host || !out) { set_error("dcr_sdrf_create: bad arguments"); return 1; }
-    if (mode < DCR_SDRF_MODE_BFC || mode > DCR_SDRF_MODE_BFC_PAPER) { set_error("dcr_sdrf_create: unknown mode"); return 1; }
+// The host image and the sizes of one state, from its insertion-order rows: the validation and sizing shared by
+// dcr_sdrf_create_mode and dcr_sdrf_create_batch.
+struct SdrfPlan {
+    SdrfDev D;            // the sizes (n, ctype, cap_total, row_cap_max, imp_cap, dirty_cap); no pointers yet
+    int rows;
+    int64_t sum_cap;      // arena slots filled at set-up
+    int64_t n_self;
+    size_t bytes;         // slab size
+    std::vector<int32_t> rstart, rlen, rcap, selfl, col, ord, owner;
+    int32_t scal[8];
+};
+
+// rows [0,n): the neighbour (directed: successor) lists, rows [n,2n): the predecessor lists (directed mode only);
+// row_len(r) / row_src(r) give row r, nnz / in_nnz the entries of the two halves.  `who` starts every error message.
+template <class RowLen, class RowSrc>
+static int sdrf_plan(const char* who, int n, int mode, int64_t nnz, int64_t in_nnz, RowLen row_len, RowSrc row_src,
+                     int64_t max_additions, SdrfPlan& P) {
     const bool directed = mode == DCR_SDRF_MODE_BFC_DIRECTED;
     const bool paper = mode == DCR_SDRF_MODE_BFC_PAPER;
-    if (directed && !in_rowptr_host) { set_error("dcr_sdrf_create: the directed mode needs the predecessor lists"); return 1; }
     const int rows = directed ? 2 * n : n;
-    int64_t nnz = rowptr_host[n];             // (entries of the insertion-order lists; self entries are subtracted below)
-    if (directed && in_rowptr_host[n] != nnz) { set_error("dcr_sdrf_create: successor / predecessor lists disagree"); return 1; }
-    auto row_len = [&](int r) { return r < n ? rowptr_host[r + 1] - rowptr_host[r] : in_rowptr_host[r - n + 1] - in_rowptr_host[r - n]; };
-    auto row_src = [&](int r) { return r < n ? order_host + rowptr_host[r] : in_order_host + in_rowptr_host[r - n]; };
+    if (directed && in_nnz != nnz) { set_error("%s: successor / predecessor lists disagree", who); return 1; }
     std::vector<int32_t> rstart(rows), rlen(rows), rcap(rows), selfl(rows, 0);
     int64_t sum_cap = 0, n_self = 0;
     int d1 = 0, d2 = 0;   // the two largest row lengths
@@ -1570,8 +1723,8 @@ static int sdrf_create_impl(int n, int mode, const int32_t* rowptr_host, const i
             const int me = v < n ? v : v - n;
             int hits = 0;
             for (int t = 0; t < len; ++t) hits += src[t] == me;
-            if (hits > 1) { set_error("dcr_sdrf_create: node %d lists itself more than once", me); return 1; }
-            if (hits && paper) { set_error("dcr_sdrf_create: node %d lists itself (the paper-flavour loop takes no self-loops)", me); return 1; }
+            if (hits > 1) { set_error("%s: node %d lists itself more than once", who, me); return 1; }
+            if (hits && paper) { set_error("%s: node %d lists itself (the paper-flavour loop takes no self-loops)", who, me); return 1; }
             selfl[v] = hits;
             if (v < n) n_self += hits;                 // (counted once per node: the successor / neighbour rows)
             len -= hits;
@@ -1584,7 +1737,7 @@ static int sdrf_create_impl(int n, int mode, const int32_t* rowptr_host, const i
         if (len > d1) { d2 = d1; d1 = len; } else if (len > d2) d2 = len;
     }
     const int64_t cap_total = 5 * sum_cap + 8 * max_additions + 1024;
-    if (cap_total > 0x7ffffff0LL) { set_error("dcr_sdrf_create: graph too large for a 32-bit arena"); return 1; }
+    if (cap_total > 0x7ffffff0LL) { set_error("%s: graph too large for a 32-bit arena", who); return 1; }
     std::vector<int32_t> col(sum_cap, 0), ord(sum_cap, 0), owner(sum_cap, -1);
     nnz -= n_self;                            // (directed: successor entries; the predecessor rows mirror them)
     for (int v = 0; v < rows; ++v) {
@@ -1593,7 +1746,7 @@ static int sdrf_create_impl(int n, int mode, const int32_t* rowptr_host, const i
         const int self = v < n ? v : v - n;
         int filled = 0;
         for (int t = 0; t < len + selfl[v]; ++t) {
-            if (src[t] < 0 || src[t] >= n || (src[t] == self && !selfl[v])) { set_error("dcr_sdrf_create: bad neighbour id"); return 1; }
+            if (src[t] < 0 || src[t] >= n || (src[t] == self && !selfl[v])) { set_error("%s: bad neighbour id", who); return 1; }
             ord[rstart[v] + t] = src[t];
             if (src[t] == self) continue;
             col[rstart[v] + filled] = src[t];
@@ -1602,25 +1755,23 @@ static int sdrf_create_impl(int n, int mode, const int32_t* rowptr_host, const i
         }
         std::sort(col.begin() + rstart[v], col.begin() + rstart[v] + len);
         for (int t = 1; t < len; ++t)
-            if (col[rstart[v] + t] == col[rstart[v] + t - 1]) { set_error("dcr_sdrf_create: duplicate neighbour"); return 1; }
+            if (col[rstart[v] + t] == col[rstart[v] + t - 1]) { set_error("%s: duplicate neighbour", who); return 1; }
     }
     if (directed) {   // the predecessor rows must be the transpose of the successor rows
         for (int v = 0; v < n; ++v)
-            if (selfl[v] != selfl[n + v]) { set_error("dcr_sdrf_create: successor / predecessor lists disagree"); return 1; }
+            if (selfl[v] != selfl[n + v]) { set_error("%s: successor / predecessor lists disagree", who); return 1; }
         for (int v = 0; v < n; ++v)
             for (int t = 0; t < rlen[v]; ++t) {
                 const int w = col[rstart[v] + t];
                 const int32_t* b = col.data() + rstart[n + w];
                 if (!std::binary_search(b, b + rlen[n + w], v)) {
-                    set_error("dcr_sdrf_create: successor / predecessor lists disagree");
+                    set_error("%s: successor / predecessor lists disagree", who);
                     return 1;
                 }
             }
     }
-    dcr_sdrf* s = new dcr_sdrf();
-    s->mode = mode;
-    s->n_self = n_self;
-    SdrfDev& D = s->dev;
+    SdrfDev& D = P.D;
+    D = SdrfDev{};
     D.n = n;
     D.ctype = (mode >= DCR_SDRF_MODE_1D && mode <= DCR_SDRF_MODE_HAANTJES) ? mode - DCR_SDRF_MODE_1D : 0;
     D.cap_total = (int)cap_total;
@@ -1640,9 +1791,43 @@ static int sdrf_create_impl(int n, int mode, const int32_t* rowptr_host, const i
     add(D.imp_cap, paper ? 8 : 4); add(D.imp_cap, 8);        // imp, pend
     add((size_t)2 * D.dirty_cap, 4); add(D.dirty_cap, 4);    // dirty, work
     add(D.row_cap_max, 4);                                   // wlist
-    cudaError_t e = cudaMalloc(&s->slab, bytes);
+    P.rows = rows;
+    P.sum_cap = sum_cap;
+    P.n_self = n_self;
+    P.bytes = bytes;
+    P.rstart = std::move(rstart); P.rlen = std::move(rlen); P.rcap = std::move(rcap); P.selfl = std::move(selfl);
+    P.col = std::move(col); P.ord = std::move(ord); P.owner = std::move(owner);
+    // [0] arena top, [1] nnz, [2] add edits so far, [3] their limit (dcr_sdrf_edit)
+    const int32_t scal[8] = {(int32_t)sum_cap, (int32_t)nnz, 0, (int32_t)std::min<int64_t>(max_additions, 0x7fffffff), 0, 0, 0, 0};
+    std::copy(scal, scal + 8, P.scal);
+    return 0;
+}
+
+static int sdrf_create_impl(int n, int mode, const int32_t* rowptr_host, const int32_t* order_host,
+                            const int32_t* in_rowptr_host, const int32_t* in_order_host, int64_t max_additions,
+                            dcr_sdrf** out) {
+    if (n <= 0 || !rowptr_host || !out) { set_error("dcr_sdrf_create: bad arguments"); return 1; }
+    if (mode < DCR_SDRF_MODE_BFC || mode > DCR_SDRF_MODE_BFC_PAPER) { set_error("dcr_sdrf_create: unknown mode"); return 1; }
+    const bool directed = mode == DCR_SDRF_MODE_BFC_DIRECTED;
+    const bool paper = mode == DCR_SDRF_MODE_BFC_PAPER;
+    if (directed && !in_rowptr_host) { set_error("dcr_sdrf_create: the directed mode needs the predecessor lists"); return 1; }
+    auto row_len = [&](int r) { return r < n ? rowptr_host[r + 1] - rowptr_host[r] : in_rowptr_host[r - n + 1] - in_rowptr_host[r - n]; };
+    auto row_src = [&](int r) { return r < n ? order_host + rowptr_host[r] : in_order_host + in_rowptr_host[r - n]; };
+    SdrfPlan P;
+    if (sdrf_plan("dcr_sdrf_create", n, mode, rowptr_host[n], directed ? in_rowptr_host[n] : 0, row_len, row_src,
+                  max_additions, P))
+        return 1;
+    const int rows = P.rows;
+    const int64_t sum_cap = P.sum_cap, cap_total = P.D.cap_total;
+    dcr_sdrf* s = new dcr_sdrf();
+    s->mode = mode;
+    s->n_self = P.n_self;
+    s->pool = nullptr;
+    SdrfDev& D = s->dev;
+    D = P.D;
+    cudaError_t e = cudaMalloc(&s->slab, P.bytes);
     if (e != cudaSuccess) { delete s; return cuda_fail(e, "cudaMalloc(sdrf slab)", __FILE__, __LINE__); }
-    s->slab_bytes = bytes;
+    s->slab_bytes = P.bytes;
     carve_slab(D, (char*)s->slab, rows, paper);
 
     auto fail = [&](cudaError_t err, const char* what) {
@@ -1651,22 +1836,20 @@ static int sdrf_create_impl(int n, int mode, const int32_t* rowptr_host, const i
         return cuda_fail(err, what, __FILE__, __LINE__);
     };
 #define SDRF_TRY(call) do { cudaError_t e2 = (call); if (e2 != cudaSuccess) return fail(e2, #call); } while (0)
-    SDRF_TRY(cudaMemcpy(D.rstart, rstart.data(), rows * 4, cudaMemcpyHostToDevice));
-    SDRF_TRY(cudaMemcpy(D.rlen, rlen.data(), rows * 4, cudaMemcpyHostToDevice));
-    SDRF_TRY(cudaMemcpy(D.rcap, rcap.data(), rows * 4, cudaMemcpyHostToDevice));
-    SDRF_TRY(cudaMemcpy(D.selfl, selfl.data(), rows * 4, cudaMemcpyHostToDevice));
+    SDRF_TRY(cudaMemcpy(D.rstart, P.rstart.data(), rows * 4, cudaMemcpyHostToDevice));
+    SDRF_TRY(cudaMemcpy(D.rlen, P.rlen.data(), rows * 4, cudaMemcpyHostToDevice));
+    SDRF_TRY(cudaMemcpy(D.rcap, P.rcap.data(), rows * 4, cudaMemcpyHostToDevice));
+    SDRF_TRY(cudaMemcpy(D.selfl, P.selfl.data(), rows * 4, cudaMemcpyHostToDevice));
     SDRF_TRY(cudaMemset(D.owner, 0xff, cap_total * 4));
     SDRF_TRY(cudaMemset(D.flag, 0, cap_total * 4));
     SDRF_TRY(cudaMemset(D.supp, 0, cap_total * 4));
     SDRF_TRY(cudaMemset(D.c32, 0, cap_total * 4));
     if (sum_cap > 0) {
-        SDRF_TRY(cudaMemcpy(D.col, col.data(), sum_cap * 4, cudaMemcpyHostToDevice));
-        SDRF_TRY(cudaMemcpy(D.ord, ord.data(), sum_cap * 4, cudaMemcpyHostToDevice));
-        SDRF_TRY(cudaMemcpy(D.owner, owner.data(), sum_cap * 4, cudaMemcpyHostToDevice));
+        SDRF_TRY(cudaMemcpy(D.col, P.col.data(), sum_cap * 4, cudaMemcpyHostToDevice));
+        SDRF_TRY(cudaMemcpy(D.ord, P.ord.data(), sum_cap * 4, cudaMemcpyHostToDevice));
+        SDRF_TRY(cudaMemcpy(D.owner, P.owner.data(), sum_cap * 4, cudaMemcpyHostToDevice));
     }
-    // [2] add edits so far, [3] their limit (dcr_sdrf_edit)
-    int32_t scal[8] = {(int32_t)sum_cap, (int32_t)nnz, 0, (int32_t)std::min<int64_t>(max_additions, 0x7fffffff), 0, 0, 0, 0};
-    SDRF_TRY(cudaMemcpy(D.scalars, scal, sizeof(scal), cudaMemcpyHostToDevice));
+    SDRF_TRY(cudaMemcpy(D.scalars, P.scal, sizeof(P.scal), cudaMemcpyHostToDevice));
     if (sum_cap > 0) {
         const int ctas = (int)std::min<int64_t>((sum_cap + 7) / 8, (int64_t)sm_count() * 8);
         if (!directed && !paper) sdrf_init_support_kernel<<<ctas, 256>>>(D, (int)sum_cap);   // (paper: no supports)
@@ -1676,6 +1859,132 @@ static int sdrf_create_impl(int n, int mode, const int32_t* rowptr_host, const i
     SDRF_TRY(cudaDeviceSynchronize());
 #undef SDRF_TRY
     *out = s;
+    return 0;
+}
+
+// Every state's slab is carved out of one pool allocation at a 256-byte aligned offset.  The host images of all states go
+// to the device in one copy of a packed staging buffer (a stream-ordered allocation freed after the set-up), whose tail
+// holds the device tables; three launches then fill the slabs, the supports and the curvature of every state.
+extern "C" int dcr_sdrf_create_batch(int count, int mode, const int32_t* num_nodes, const int64_t* rowptr_host,
+                                     const int32_t* order_host, const int64_t* in_rowptr_host,
+                                     const int32_t* in_order_host, const int64_t* max_additions, dcr_sdrf** out_host) {
+    if (count < 1 || !num_nodes || !rowptr_host || !max_additions || !out_host) {
+        set_error("dcr_sdrf_create_batch: bad arguments (count must be >= 1)");
+        return 1;
+    }
+    if (mode < DCR_SDRF_MODE_BFC || mode > DCR_SDRF_MODE_BFC_PAPER) { set_error("dcr_sdrf_create_batch: unknown mode"); return 1; }
+    const bool directed = mode == DCR_SDRF_MODE_BFC_DIRECTED;
+    const bool paper = mode == DCR_SDRF_MODE_BFC_PAPER;
+    if (directed && !in_rowptr_host) { set_error("dcr_sdrf_create_batch: the directed mode needs the predecessor lists"); return 1; }
+    // node offsets; the row offsets must start at 0 and never decrease
+    std::vector<int64_t> node_off(count + 1, 0);
+    for (int g = 0; g < count; ++g) {
+        if (num_nodes[g] <= 0) { set_error("dcr_sdrf_create_batch: graph %d has %d nodes", g, num_nodes[g]); return 1; }
+        if (max_additions[g] < 0) { set_error("dcr_sdrf_create_batch: graph %d: max_additions < 0", g); return 1; }
+        node_off[g + 1] = node_off[g] + num_nodes[g];
+    }
+    const int64_t N = node_off[count];
+    for (int half = 0; half < (directed ? 2 : 1); ++half) {
+        const int64_t* rp = half ? in_rowptr_host : rowptr_host;
+        if (rp[0] != 0) { set_error("dcr_sdrf_create_batch: row offsets must start at 0"); return 1; }
+        for (int64_t v = 0; v < N; ++v)
+            if (rp[v + 1] < rp[v] || rp[v + 1] - rp[v] > 0x7fffffff) {
+                const int64_t g = std::upper_bound(node_off.begin(), node_off.end(), v) - node_off.begin() - 1;
+                set_error("dcr_sdrf_create_batch: graph %lld: the row offsets decrease at node %lld", (long long)g,
+                          (long long)(v - node_off[g]));
+                return 1;
+            }
+    }
+    if ((rowptr_host[N] > 0 && !order_host) || (directed && in_rowptr_host[N] > 0 && !in_order_host)) {
+        set_error("dcr_sdrf_create_batch: bad arguments (no neighbour lists)");
+        return 1;
+    }
+    std::vector<SdrfPlan> plans(count);
+    for (int g = 0; g < count; ++g) {
+        const int n = num_nodes[g];
+        const int64_t* rp = rowptr_host + node_off[g];
+        const int64_t* irp = directed ? in_rowptr_host + node_off[g] : nullptr;
+        auto row_len = [&](int r) { return (int)(r < n ? rp[r + 1] - rp[r] : irp[r - n + 1] - irp[r - n]); };
+        auto row_src = [&](int r) { return r < n ? order_host + rp[r] : in_order_host + irp[r - n]; };
+        char who[64];
+        snprintf(who, sizeof(who), "dcr_sdrf_create_batch: graph %d", g);
+        if (sdrf_plan(who, n, mode, rp[n] - rp[0], directed ? irp[n] - irp[0] : 0, row_len, row_src, max_additions[g],
+                      plans[g]))
+            return 1;
+    }
+    // pool offsets (every slab size is a multiple of 256), staging offsets (int32 words) and the device tables
+    std::vector<size_t> slab_off(count + 1, 0);
+    std::vector<int64_t> stage_off(count + 1, 0);
+    std::vector<long long> unit_off(count + 1, 0), entry_off(count + 1, 0);
+    for (int g = 0; g < count; ++g) {
+        const SdrfPlan& P = plans[g];
+        slab_off[g + 1] = slab_off[g] + P.bytes;
+        stage_off[g + 1] = stage_off[g] + 4 * (int64_t)P.rows + 3 * P.sum_cap + 8;
+        unit_off[g + 1] = unit_off[g] + P.D.cap_total + P.rows;
+        entry_off[g + 1] = entry_off[g] + P.sum_cap;
+    }
+    const size_t words = (size_t)(stage_off[count] + 1) / 2 * 2;                 // (8-byte aligned tables after it)
+    const size_t table_bytes = sizeof(SdrfInitDesc) * count + 2 * sizeof(long long) * (count + 1);
+    const size_t stage_bytes = 4 * words + table_bytes;
+    void* pool_base = nullptr;
+    cudaError_t e = cudaMalloc(&pool_base, slab_off[count]);
+    if (e != cudaSuccess) return cuda_fail(e, "cudaMalloc(sdrf pool)", __FILE__, __LINE__);
+    std::vector<char> host(stage_bytes);
+    int32_t* hw = reinterpret_cast<int32_t*>(host.data());
+    SdrfInitDesc* hdesc = reinterpret_cast<SdrfInitDesc*>(host.data() + 4 * words);
+    long long* hunit = reinterpret_cast<long long*>(hdesc + count);
+    long long* hentry = hunit + count + 1;
+    void* stage = nullptr;
+    e = cudaMallocAsync(&stage, stage_bytes, 0);
+    if (e != cudaSuccess) { cudaFree(pool_base); return cuda_fail(e, "cudaMallocAsync(sdrf staging)", __FILE__, __LINE__); }
+    const int32_t* dstage = reinterpret_cast<const int32_t*>(stage);
+    for (int g = 0; g < count; ++g) {
+        const SdrfPlan& P = plans[g];
+        int32_t* w = hw + stage_off[g];
+        for (const std::vector<int32_t>* a : {&P.rstart, &P.rlen, &P.rcap, &P.selfl, &P.col, &P.ord, &P.owner}) {
+            std::copy(a->begin(), a->end(), w);
+            w += a->size();
+        }
+        std::copy(P.scal, P.scal + 8, w);
+        SdrfInitDesc& d = hdesc[g];
+        d.S = P.D;
+        carve_slab(d.S, (char*)pool_base + slab_off[g], P.rows, paper);
+        d.stage = dstage + stage_off[g];
+        d.rows = P.rows;
+        d.used = (int)P.sum_cap;
+    }
+    std::copy(unit_off.begin(), unit_off.end(), hunit);
+    std::copy(entry_off.begin(), entry_off.end(), hentry);
+    const SdrfInitDesc* ddesc = reinterpret_cast<const SdrfInitDesc*>((char*)stage + 4 * words);
+    const long long* dunit = reinterpret_cast<const long long*>(ddesc + count);
+    const long long* dentry = dunit + count + 1;
+    e = cudaMemcpyAsync(stage, host.data(), stage_bytes, cudaMemcpyHostToDevice, 0);
+    if (e == cudaSuccess) {
+        const int ctas = (int)std::max<int64_t>(1, std::min<int64_t>((unit_off[count] + 255) / 256, (int64_t)sm_count() * 8));
+        sdrf_batch_setup_kernel<<<ctas, 256>>>(ddesc, dunit, count);
+        if (entry_off[count] > 0) {
+            const int ictas = (int)std::min<int64_t>((entry_off[count] + 7) / 8, (int64_t)sm_count() * 8);
+            if (!directed && !paper) sdrf_batch_init_support_kernel<<<ictas, 256>>>(ddesc, dentry, count);
+            loop_kernels(mode).batch_init<<<ictas, 256>>>(ddesc, dentry, count);
+        }
+        e = cudaGetLastError();
+    }
+    const cudaError_t ef = cudaFreeAsync(stage, 0);
+    if (e == cudaSuccess) e = ef;
+    const cudaError_t es = cudaDeviceSynchronize();
+    if (e == cudaSuccess) e = es;
+    if (e != cudaSuccess) { cudaFree(pool_base); return cuda_fail(e, "dcr_sdrf_create_batch: set-up", __FILE__, __LINE__); }
+    SdrfPool* pool = new SdrfPool{pool_base, {count}};
+    for (int g = 0; g < count; ++g) {
+        dcr_sdrf* s = new dcr_sdrf();
+        s->dev = hdesc[g].S;
+        s->slab = (char*)pool_base + slab_off[g];
+        s->slab_bytes = plans[g].bytes;
+        s->mode = mode;
+        s->n_self = plans[g].n_self;
+        s->pool = pool;
+        out_host[g] = s;
+    }
     return 0;
 }
 
@@ -1692,7 +2001,11 @@ extern "C" int dcr_sdrf_create_mode(int n, int mode, const int32_t* rowptr_host,
 
 extern "C" void dcr_sdrf_destroy(dcr_sdrf* s) {
     if (!s) return;
-    cudaFree(s->slab);
+    if (!s->pool) cudaFree(s->slab);
+    else if (s->pool->refs.fetch_sub(1) == 1) {
+        cudaFree(s->pool->base);
+        delete s->pool;
+    }
     delete s;
 }
 
@@ -1709,6 +2022,7 @@ extern "C" int dcr_sdrf_fork(dcr_sdrf* s, int count, dcr_sdrf** out_host, void* 
     };
     for (int b = 0; b < count; ++b) {
         dcr_sdrf* c = new dcr_sdrf(*s);
+        c->pool = nullptr;                      // (a copy owns its slab, also when the source is pooled)
         const cudaError_t e = cudaMalloc(&c->slab, s->slab_bytes);
         if (e != cudaSuccess) { delete c; release(); return cuda_fail(e, "cudaMalloc(sdrf fork slab)", __FILE__, __LINE__); }
         copies.push_back(c);
@@ -1936,6 +2250,69 @@ extern "C" int dcr_sdrf_export_edge_index(dcr_sdrf* s, int32_t* rowptr_order, in
     const int ctas = std::max(1, std::min((s->dev.n + 7) / 8, sm_count() * 8));
     sdrf_export_edge_index_kernel<<<ctas, 256, 0, st>>>(s->dev, rowptr_order, src, dst, (long long)capacity,
                                                         s->mode == DCR_SDRF_MODE_BFC_DIRECTED);
+    DCR_LAUNCH_CHECK();
+    return 0;
+}
+
+extern "C" int64_t dcr_sdrf_export_edge_index_batch_workspace_bytes(dcr_sdrf* const* states, int count) {
+    if (count < 1 || !states) return 0;
+    int64_t rows = 0;
+    for (int b = 0; b < count; ++b) {
+        if (!states[b]) return 0;
+        rows += states[b]->dev.n;
+    }
+    return (int64_t)sizeof(SdrfExportDesc) * count + (int64_t)sizeof(long long) * (count + 1 + rows);
+}
+
+extern "C" int dcr_sdrf_export_edge_index_batch(dcr_sdrf* const* states, int count, const int64_t* node_offsets,
+                                                int64_t* src, int64_t* dst, int64_t capacity, int64_t* edge_ptr,
+                                                void* workspace, int64_t workspace_bytes, void* stream) {
+    if (count < 1 || !states || !node_offsets || !edge_ptr || capacity < 0 || (capacity > 0 && (!src || !dst))) {
+        set_error("dcr_sdrf_export_edge_index_batch: bad arguments (count must be >= 1)");
+        return 1;
+    }
+    // host tables: one descriptor per state, then the row offsets (count + 1); the device copy is followed by the
+    // per-row counts, which the scan turns into the global column offsets
+    std::vector<char> host(sizeof(SdrfExportDesc) * count + sizeof(long long) * (count + 1));
+    SdrfExportDesc* desc = reinterpret_cast<SdrfExportDesc*>(host.data());
+    long long* row_off = reinterpret_cast<long long*>(desc + count);
+    row_off[0] = 0;
+    for (int b = 0; b < count; ++b) {
+        if (!states[b]) { set_error("dcr_sdrf_export_edge_index_batch: state %d is null", b); return 1; }
+        if (states[b]->mode != states[0]->mode) {
+            set_error("dcr_sdrf_export_edge_index_batch: state %d has loop mode %d, state 0 has %d (one mode per call)", b,
+                      states[b]->mode, states[0]->mode);
+            return 1;
+        }
+        if (node_offsets[b] < 0 || (b > 0 && node_offsets[b] < node_offsets[b - 1] + states[b - 1]->dev.n)) {
+            set_error("dcr_sdrf_export_edge_index_batch: node_offsets[%d] = %lld overlaps the nodes of the state before "
+                      "it or is negative", b, (long long)node_offsets[b]);
+            return 1;
+        }
+        desc[b] = {states[b]->dev, (long long)node_offsets[b]};
+        row_off[b + 1] = row_off[b] + states[b]->dev.n;
+    }
+    if (!workspace || workspace_bytes < dcr_sdrf_export_edge_index_batch_workspace_bytes(states, count)) {
+        set_error("dcr_sdrf_export_edge_index_batch: workspace of dcr_sdrf_export_edge_index_batch_workspace_bytes = %lld "
+                  "bytes required", (long long)dcr_sdrf_export_edge_index_batch_workspace_bytes(states, count));
+        return 1;
+    }
+    if ((uintptr_t)workspace % 8) { set_error("dcr_sdrf_export_edge_index_batch: workspace must be 8-byte aligned"); return 1; }
+    cudaStream_t st = (cudaStream_t)stream;
+    const SdrfExportDesc* ddesc = (const SdrfExportDesc*)workspace;
+    const long long* drow_off = (const long long*)(ddesc + count);
+    long long* rowptr = (long long*)(drow_off + count + 1);
+    const long long rows = row_off[count];
+    // pageable source: the copy is staged before cudaMemcpyAsync returns, so `host` may go out of scope
+    DCR_CUDA(cudaMemcpyAsync(workspace, host.data(), host.size(), cudaMemcpyHostToDevice, st));
+    const int ctas = (int)std::max<long long>(1, std::min<long long>((rows + 255) / 256, (long long)sm_count() * 8));
+    sdrf_batch_export_counts_kernel<<<ctas, 256, 0, st>>>(ddesc, drow_off, count, rowptr);
+    DCR_LAUNCH_CHECK();
+    sdrf_batch_export_scan_kernel<<<1, SDRF_THREADS, 0, st>>>(drow_off, count, rowptr, edge_ptr);
+    DCR_LAUNCH_CHECK();
+    const int wctas = (int)std::max<long long>(1, std::min<long long>((rows + 7) / 8, (long long)sm_count() * 8));
+    sdrf_batch_export_rows_kernel<<<wctas, 256, 0, st>>>(ddesc, drow_off, count, rowptr, src, dst, (long long)capacity,
+                                                         states[0]->mode == DCR_SDRF_MODE_BFC_DIRECTED);
     DCR_LAUNCH_CHECK();
     return 0;
 }

@@ -77,6 +77,7 @@ SIGNATURES = {
     "dcr_post_delta_directed": (_I, [_P, _P, _P, _P, _I, _I, _I, _P, _I, _P, _I, _P, _P, _L, _P]),
     "dcr_sdrf_create": (_I, [_I, _P, _P, _L, C.POINTER(_P)]),
     "dcr_sdrf_create_mode": (_I, [_I, _I, _P, _P, _P, _P, _L, C.POINTER(_P)]),
+    "dcr_sdrf_create_batch": (_I, [_I, _I, _P, _P, _P, _P, _P, _P, C.POINTER(_P)]),
     "dcr_sdrf_destroy": (None, [_P]),
     "dcr_sdrf_run": (_I, [_P, _I, _I, _D, _D, _P, _L, _I, _D, _P, _P, _P]),
     "dcr_sdrf_batch_workspace_bytes": (_L, [_I]),
@@ -91,6 +92,8 @@ SIGNATURES = {
     "dcr_sdrf_export_order": (_I, [_P, _P, _P, _P]),
     "dcr_sdrf_export_c64": (_I, [_P, _P, _P, _P]),
     "dcr_sdrf_export_edge_index": (_I, [_P, _P, _P, _P, _L, _P]),
+    "dcr_sdrf_export_edge_index_batch_workspace_bytes": (_L, [_P, _I]),
+    "dcr_sdrf_export_edge_index_batch": (_I, [_P, _I, _P, _P, _P, _L, _P, _P, _L, _P]),
     "dcr_sdrf_score_sizes": (_I, [_P, _P, _I, _P, _P, _P]),
     "dcr_sdrf_score_workspace_bytes": (_L, [_P, _I]),
     "dcr_sdrf_score": (_I, [_P, _P, _I, _P, _P, _P, _P, _P, _P, _L, _P]),

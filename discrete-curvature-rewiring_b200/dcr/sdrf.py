@@ -83,12 +83,50 @@ class SdrfState:
     @classmethod
     def _from_handle(cls, handle: C.c_void_p, like: "SdrfState") -> "SdrfState":
         """A state that owns ``handle``, a copy of ``like`` made by ``dcr_sdrf_fork``."""
+        return cls._adopt(handle, like.lib, like.mode, like.n, like.n_self, like.device)
+
+    @classmethod
+    def _adopt(cls, handle: C.c_void_p, lib, mode: int, n: int, n_self: int, device) -> "SdrfState":
         self = cls.__new__(cls)
-        self.lib, self.mode, self.n, self.n_self, self.device = like.lib, like.mode, like.n, like.n_self, like.device
+        self.lib, self.mode, self.n, self.n_self, self.device = lib, mode, n, n_self, device
         self._keep = None
         self.handle = handle
         self._result = torch.zeros(8, dtype=torch.int32, device=self.device)
         return self
+
+    @classmethod
+    def create_batch(cls, mode: int, num_nodes, rowptr: np.ndarray, order: np.ndarray, max_additions,
+                     in_rowptr: np.ndarray | None = None, in_order: np.ndarray | None = None) -> list:
+        """B states from one concatenated input with one ``dcr_sdrf_create_batch``: graph ``g`` has ``num_nodes[g]``
+        rows of the int64 offsets ``rowptr`` (over all graphs' nodes, from 0) into ``order``, which lists LOCAL ids in
+        insertion order (the directed mode: also the predecessor lists ``in_rowptr`` / ``in_order``), and the budget
+        ``max_additions[g]``.  State ``g`` equals ``SdrfState`` of graph ``g`` alone; all share one device pool."""
+        L.require_cuda()
+        lib = L.load()
+        nn = np.ascontiguousarray(num_nodes, dtype=np.int32)
+        count = int(nn.size)
+        rp = np.ascontiguousarray(rowptr, dtype=np.int64)
+        od = np.ascontiguousarray(order, dtype=np.int32)
+        ma = np.ascontiguousarray(max_additions, dtype=np.int64)
+        if mode == L.SDRF_MODE_BFC_DIRECTED:
+            irp = np.ascontiguousarray(in_rowptr, dtype=np.int64)
+            iod = np.ascontiguousarray(in_order, dtype=np.int32)
+        else:
+            irp = iod = None
+        handles = (C.c_void_p * max(count, 1))()
+        L.check(lib.dcr_sdrf_create_batch(count, int(mode), nn.ctypes.data, rp.ctypes.data, od.ctypes.data if od.size else 0,
+                                          irp.ctypes.data if irp is not None else 0,
+                                          iod.ctypes.data if iod is not None and iod.size else 0, ma.ctypes.data, handles),
+                "dcr_sdrf_create_batch")
+        # nodes that list themselves, per graph (the neighbour / successor rows)
+        graph_of_node = np.repeat(np.arange(count), nn)
+        local = np.arange(nn.sum(), dtype=np.int64) - np.repeat(np.cumsum(nn, dtype=np.int64) - nn, nn)
+        counts = np.diff(rp)
+        is_self = od == np.repeat(local, counts)
+        n_self = np.bincount(np.repeat(graph_of_node, counts)[is_self], minlength=count)
+        device = torch.device("cuda", torch.cuda.current_device())
+        return [cls._adopt(C.c_void_p(h), lib, int(mode), int(nn[g]), int(n_self[g]), device)
+                for g, h in enumerate(handles[:count])]
 
     def fork(self, count: int) -> list:
         """``count`` independent copies of this state (graph, insertion order, curvature, budget) after one
@@ -227,6 +265,25 @@ class SdrfState:
         L.check(self.lib.dcr_sdrf_export_edge_index(self.handle, rowptr.data_ptr(), out[0].data_ptr(), out[1].data_ptr(),
                                                     cap, L.current_stream()), "dcr_sdrf_export_edge_index")
         return out[:, : int(rowptr[-1])]
+
+
+def export_edge_index_batch(states, node_offsets, capacity: int):
+    """``SdrfState.edge_index`` of every state into one output with ``dcr_sdrf_export_edge_index_batch``: state ``b``'s
+    columns follow state ``b-1``'s with node ids shifted by ``node_offsets[b]``.  Returns the device int64 ``[2, capacity]``
+    output and the device int64 ``edge_ptr[B + 1]``; the columns are ``[:, :edge_ptr[B]]`` (``capacity`` bounds it)."""
+    count = len(states)
+    lib = L.load()
+    dev = states[0].device
+    handles = (C.c_void_p * count)(*[s.handle.value for s in states])
+    offs = np.ascontiguousarray(node_offsets, dtype=np.int64)
+    out = torch.empty((2, max(int(capacity), 1)), dtype=torch.int64, device=dev)
+    edge_ptr = torch.empty(count + 1, dtype=torch.int64, device=dev)
+    nbytes = int(lib.dcr_sdrf_export_edge_index_batch_workspace_bytes(handles, count))
+    workspace = torch.empty(max(nbytes // 8, 1), dtype=torch.int64, device=dev)
+    L.check(lib.dcr_sdrf_export_edge_index_batch(handles, count, offs.ctypes.data, out[0].data_ptr(), out[1].data_ptr(),
+                                                 int(capacity), edge_ptr.data_ptr(), workspace.data_ptr(), nbytes,
+                                                 L.current_stream()), "dcr_sdrf_export_edge_index_batch")
+    return out, edge_ptr
 
 
 def edit_tensor(edits) -> torch.Tensor:
@@ -550,3 +607,140 @@ def _batch_return(outs, out_logs, errors, return_log: bool, return_exceptions: b
         if first is not None:
             raise first
     return (outs, out_logs) if return_log else outs
+
+
+# log fields that hold node ids (dcr.h: {x, y, n_candidates, k, l, choice, removed_x, removed_y}; -1 = none)
+_LOG_NODE_FIELDS = [0, 1, 3, 4, 6, 7]
+
+
+def dataset_ptr(ptr, count: int) -> np.ndarray:
+    """``ptr`` of a batched dataset (PyG ``Batch.ptr``: graph ``g`` owns the nodes ``ptr[g] .. ptr[g+1] - 1``) as int64
+    numpy, checked against ``count`` graphs; ``ValueError`` naming the graph for a non-monotone ``ptr`` or an empty
+    graph."""
+    p = ptr.detach().cpu().numpy() if hasattr(ptr, "detach") else np.asarray(ptr)
+    if p.ndim != 1 or p.size < 2 or p.dtype.kind not in "iu":
+        raise ValueError("ptr: a 1-d integer array of B + 1 node offsets")
+    p = p.astype(np.int64)
+    if p.size - 1 != count:
+        raise ValueError(f"ptr describes {p.size - 1} graphs, the batch has {count} runs")
+    if p[0] != 0:
+        raise ValueError(f"ptr[0] = {p[0]}: the node offsets start at 0")
+    d = np.diff(p)
+    if (d < 0).any():
+        g = int(np.flatnonzero(d < 0)[0])
+        raise ValueError(f"graph {g}: ptr is not monotone (ptr[{g}] = {p[g]} > ptr[{g + 1}] = {p[g + 1]})")
+    if (d == 0).any():
+        g = int(np.flatnonzero(d == 0)[0])
+        raise ValueError(f"graph {g} has no nodes (ptr[{g}] = ptr[{g + 1}] = {p[g]})")
+    if d.max() > 2**31 - 1:
+        g = int(np.argmax(d))
+        raise ValueError(f"graph {g} has {d[g]} nodes, more than int32 ids can name")
+    return p
+
+
+def _column_graphs(ei: np.ndarray, p: np.ndarray) -> np.ndarray:
+    """The graph of every column of the global ``edge_index`` ``ei``; ``ValueError`` naming the column and graph for an
+    endpoint outside ``[0, ptr[B])`` or a column joining two graphs."""
+    total = int(p[-1])
+    outside = (ei < 0) | (ei >= total)
+    if outside.any():
+        t = int(np.flatnonzero(outside.any(0))[0])
+        u, v = (int(x) for x in ei[:, t])
+        inside = v if outside[0, t] else u
+        where = (f"; its other endpoint lies in graph {int(np.searchsorted(p, inside, side='right')) - 1}"
+                 if not outside[:, t].all() else "")
+        raise ValueError(f"edge_index column {t} = ({u}, {v}) has a node outside [0, {total}){where}")
+    gu = np.searchsorted(p, ei[0], side="right") - 1
+    gv = np.searchsorted(p, ei[1], side="right") - 1
+    if (gu != gv).any():
+        t = int(np.flatnonzero(gu != gv)[0])
+        raise ValueError(f"edge_index column {t} = ({ei[0, t]}, {ei[1, t]}) joins graph {gu[t]} and graph {gv[t]}")
+    return gu
+
+
+def _dataset_order(order, mode: int, ei: np.ndarray, p: np.ndarray, gid: np.ndarray) -> list:
+    """``order`` (``_loop_mode``) computed ONCE on the disjoint union of the graphs, as ``create_batch`` takes it: int64
+    row offsets over all nodes and LOCAL ids.  The order functions rank a column only against columns of the same source
+    (or pair), all of one graph, and keep their relative order, so the union's rows are each graph's own rows.  A mode's
+    input error names the graph it comes from."""
+    try:
+        lists = order(ei, int(p[-1]))
+    except NotImplementedError as e:
+        if mode == L.SDRF_MODE_BFC_PAPER:
+            t = int(np.flatnonzero(ei[0] == ei[1])[0])             # a self-loop
+        else:                                                      # a repeated directed pair
+            _, first = np.unique(ei[0] * int(p[-1]) + ei[1], return_index=True)
+            repeat = np.ones(ei.shape[1], dtype=bool)
+            repeat[first] = False
+            t = int(np.flatnonzero(repeat)[0])
+        raise NotImplementedError(f"graph {gid[t]}: {e}") from None
+    node_base = np.repeat(p[:-1], np.diff(p))                     # first node of the graph of every node
+    out = []
+    for rowptr, od in zip(lists[0::2], lists[1::2]):
+        rowptr = np.asarray(rowptr, dtype=np.int64)
+        out += [rowptr, (od - np.repeat(node_base, np.diff(rowptr))).astype(np.int32)]
+    return out
+
+
+def sdrf_dataset(edge_index, ptr, loops, remove_edges: bool, removal_bound, tau, *, uniforms, guard: float = 1e-9,
+                 return_log: bool = False, is_undirected: bool = True, curv_type: str = "bfc",
+                 return_exceptions: bool = False):
+    """SDRF on every graph of a batched dataset (PyG layout: ``edge_index`` in global node ids, graph ``g`` owns the
+    nodes ``ptr[g] .. ptr[g+1] - 1``), one CTA per graph in one launch.  Graph ``g``'s result is what
+    ``sdrf(ei_g - ptr[g], ptr[g+1] - ptr[g], loops[g], remove_edges, removal_bound[g], tau[g], uniforms=uniforms[g],
+    guard=guard, is_undirected=is_undirected, curv_type=curv_type)`` computes on its columns ``ei_g`` alone, shifted back
+    by ``ptr[g]`` (in the edge_index and in the node ids of the log).
+
+    ``loops``, ``removal_bound``, ``tau``: scalars or per-graph sequences; ``uniforms``: a ``[B, loops]`` array or a list
+    of B 1-d arrays.  The insertion order is computed once on the whole input, all states are set up by one
+    ``dcr_sdrf_create_batch`` and exported by one ``dcr_sdrf_export_edge_index_batch``.
+
+    Returns ``(edge_index, edge_ptr)``: the device int64 ``[2, E']`` rewired dataset, graph ``g`` in the columns
+    ``edge_ptr[g] .. edge_ptr[g+1] - 1`` of the device int64 ``edge_ptr[B + 1]``; with ``return_log`` also the list of
+    B logs.  A failing graph does not stop the others; the lowest-index failure is raised afterwards with ``sdrf``'s
+    type and message, or, with ``return_exceptions``, the graph is left empty in ``edge_ptr`` and the list of B
+    exceptions (``None`` for a graph that succeeded) is appended to the return value.  The input is checked before
+    anything is allocated: ``ValueError`` naming the graph for a column between two graphs or outside ``[0, ptr[B])``,
+    a non-monotone ``ptr`` or a graph without nodes."""
+    uni = _batch_uniforms(uniforms, "sdrf_dataset")
+    count = len(uni)
+    p = dataset_ptr(ptr, count)
+    ei = G._as_numpy_edge_index(edge_index)
+    gid = _column_graphs(ei, p)
+    iters = [max(int(v), 0) for v in _per_run("loops", loops, count)]
+    bounds = [float(v) for v in _per_run("removal_bound", removal_bound, count)]
+    taus = _per_run("tau", tau, count)
+    mode, order = _loop_mode(curv_type, is_undirected)
+    lists = _dataset_order(order, mode, ei, p, gid)
+    L.require_cuda()
+    states = SdrfState.create_batch(mode, np.diff(p), lists[0], lists[1], iters, *lists[2:])
+    try:
+        logs, done, errors = _run_batch_states(states, iters, bounds, taus, uni, remove_edges, guard)
+        first = next((e for e in errors if e is not None), None)
+        if first is not None and not return_exceptions:
+            raise first
+        ok = [g for g in range(count) if errors[g] is None]
+        dev = states[0].device
+        if ok:
+            entries = lists[0][p[1:]] - lists[0][p[:-1]]          # insertion-order entries at set-up, per graph
+            cap = sum(int(entries[g]) + 2 * done[g] for g in ok)   # an iteration adds at most two
+            out, ok_ptr = export_edge_index_batch([states[g] for g in ok], p[ok], cap)
+        else:
+            out, ok_ptr = torch.zeros((2, 0), dtype=torch.int64, device=dev), torch.zeros(1, dtype=torch.int64, device=dev)
+        # a failed graph repeats the offset before it
+        idx = torch.from_numpy(np.concatenate([[0], np.cumsum([e is None for e in errors])])).to(dev)
+        edge_ptr = ok_ptr[idx]
+        edge_index_out = out[:, : int(edge_ptr[-1])]
+        result = [edge_index_out, edge_ptr]
+        if return_log:
+            flat = torch.cat([logs[g][: done[g]] for g in range(count)]).cpu().numpy()
+            node = flat[:, _LOG_NODE_FIELDS]
+            shift = np.repeat(p[:-1], done)[:, None]
+            flat[:, _LOG_NODE_FIELDS] = np.where(node >= 0, node + shift, node)
+            result.append(np.split(flat, np.cumsum(done)[:-1]))
+        if return_exceptions:
+            result.append(errors)
+        return tuple(result)
+    finally:
+        for s in states:
+            s.close()

@@ -12,7 +12,8 @@
 Every flavour removes edges (``remove_edges=True``), as the reference's dispatcher does.
 
 ``rewire_batch`` runs many such rewirings — one per seed, per graph or per hyper-parameter setting — in one kernel launch
-(``dcr.sdrf.sdrf_batch``, one CTA per run).
+(``dcr.sdrf.sdrf_batch``, one CTA per run).  ``rewire_dataset`` rewires every graph of a dataset in the PyG batch layout
+(``edge_index`` + ``ptr``) and returns it in that layout (``dcr.sdrf.sdrf_dataset``).
 """
 import numpy as np
 import torch
@@ -61,3 +62,47 @@ def rewire_batch(datasets, curv_type, max_iterations, removal_bound, tau, *, see
     outs = _sdrf.sdrf_batch(inputs, nodes, max_iterations, True, removal_bound, tau, uniforms=uniforms,
                             curv_type=curv_type, return_exceptions=return_exceptions)
     return [o if isinstance(o, BaseException) else torch.from_numpy(o).to(torch.long) for o in outs]
+
+
+def _dataset_layout(data):
+    """``(edge_index, ptr)`` of a ``Batch``-like object (its own) or of a sequence of ``Data`` (concatenated, graph ``g``
+    owning ``max(num_nodes, max id + 1)`` nodes, the node count ``rewire`` uses)."""
+    if not isinstance(data, (list, tuple)):
+        return torch.as_tensor(data.edge_index), torch.as_tensor(data.ptr)
+    if not data:
+        raise ValueError("rewire_dataset: an empty dataset")
+    eis = [torch.as_tensor(d.edge_index, dtype=torch.long).cpu().reshape(2, -1) for d in data]
+    sizes = [max(int(d.num_nodes), int(e.max()) + 1 if e.numel() else 0) for d, e in zip(data, eis)]
+    ptr = torch.from_numpy(np.concatenate([[0], np.cumsum(sizes)])).to(torch.long)
+    return torch.cat([e + int(o) for e, o in zip(eis, ptr[:-1])], dim=1), ptr
+
+
+def rewire_dataset(data, curv_type, max_iterations, removal_bound, tau, *, seeds=None, uniforms=None,
+                   return_exceptions=False):
+    """``rewire`` on every graph of a dataset in one launch (``dcr.sdrf.sdrf_dataset``).  ``data``: a ``Batch``-like object
+    with ``edge_index`` (global node ids) and ``ptr``, or a list of ``Data``, which is concatenated.  ``max_iterations``,
+    ``removal_bound``, ``tau``: scalars or per-graph sequences.  Exactly one of ``seeds`` / ``uniforms``, as in
+    ``rewire_batch``: graph ``g`` equals ``np.random.seed(seeds[g]); rewire(data_g, ...)`` with its node ids shifted by
+    ``ptr[g]``.
+
+    Returns ``(edge_index, edge_ptr)``: graph ``g`` in the columns ``edge_ptr[g] .. edge_ptr[g+1] - 1``; with
+    ``return_exceptions`` also the list of B exceptions (``None`` where a graph succeeded; a failed graph is empty).
+    ``curv_type=None`` returns the input's ``edge_index`` and the offsets of its per-graph columns (a ``Batch`` lists
+    each graph's columns together)."""
+    if (seeds is None) == (uniforms is None):
+        raise TypeError("rewire_dataset: pass exactly one of seeds= or uniforms=")
+    edge_index, ptr = _dataset_layout(data)
+    count = int(ptr.numel()) - 1
+    if uniforms is None:
+        if len(seeds) != count:
+            raise ValueError(f"seeds: {len(seeds)} values for a dataset of {count} graphs")
+        iters = _sdrf._per_run("max_iterations", max_iterations, count)
+        uniforms = [np.random.RandomState(s).random_sample(max(int(m), 0)) for s, m in zip(seeds, iters)]
+    if curv_type is None:
+        p = _sdrf.dataset_ptr(ptr, count)
+        graphs = np.searchsorted(p, edge_index[0].cpu().numpy(), side="right") - 1
+        edge_ptr = np.concatenate([[0], np.cumsum(np.bincount(graphs, minlength=count))])
+        out = (edge_index, torch.from_numpy(edge_ptr).to(torch.long))
+        return out + ([None] * count,) if return_exceptions else out
+    return _sdrf.sdrf_dataset(edge_index, ptr, max_iterations, True, removal_bound, tau, uniforms=uniforms,
+                              curv_type=curv_type, return_exceptions=return_exceptions)

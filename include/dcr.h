@@ -290,6 +290,21 @@ int dcr_sdrf_create(int n, const int32_t* rowptr_host, const int32_t* order_host
 int dcr_sdrf_create_mode(int n, int mode, const int32_t* rowptr_host, const int32_t* order_host,
                          const int32_t* in_rowptr_host, const int32_t* in_order_host, int64_t max_additions,
                          dcr_sdrf** out);
+/* `count` states of one DCR_SDRF_MODE_* from one concatenated host input, e.g. the graphs of a dataset; synchronises.
+ * Graph g has num_nodes[g] >= 1 nodes; its nodes are the rows node_off[g] .. node_off[g] + num_nodes[g] - 1 of the
+ * concatenation, node_off[g] = num_nodes[0] + ... + num_nodes[g-1].  rowptr_host[N + 1] (N = node_off[count]) holds
+ * int64 offsets into order_host, starting at 0 and never decreasing; every list is in LOCAL ids of its graph, in the
+ * insertion order dcr_sdrf_create_mode takes.  BFC_DIRECTED also takes the predecessor lists in_rowptr_host /
+ * in_order_host the same way.  max_additions[g] is graph g's budget.  State g (out_host[g]) is exactly what
+ * dcr_sdrf_create_mode(num_nodes[g], mode, graph g's lists, max_additions[g]) makes, with the same validation, whose
+ * messages name the graph index, and the same sizes; it runs, edits, scores, forks and exports like any state.
+ * All slabs share one device allocation, 256-byte aligned each; every state holds a reference to it and the last
+ * dcr_sdrf_destroy frees it, in any order.  A fork of such a state owns its own slab.  Status 1 for count < 1, a graph
+ * without nodes, row offsets that do not start at 0 or decrease, or any per-graph rejection; on any failure nothing is
+ * allocated and no handle is written. */
+int dcr_sdrf_create_batch(int count, int mode, const int32_t* num_nodes, const int64_t* rowptr_host,
+                          const int32_t* order_host, const int64_t* in_rowptr_host, const int32_t* in_order_host,
+                          const int64_t* max_additions, dcr_sdrf** out_host);
 void dcr_sdrf_destroy(dcr_sdrf* s);
 /* Run up to `loops` iterations.  uniforms[draw_offset + t] is the t-th uniform of this call (device, fp64).
  * forced_choice >= 0 forces the candidate index of the FIRST iteration of this call (host re-decision after
@@ -371,6 +386,19 @@ int dcr_sdrf_export_order(dcr_sdrf* s, int32_t* rowptr_order, int32_t* order_out
  * beyond `capacity`.  Enqueues only. */
 int dcr_sdrf_export_edge_index(dcr_sdrf* s, int32_t* rowptr_order, int64_t* src, int64_t* dst, int64_t capacity,
                                void* stream);
+
+/* dcr_sdrf_export_edge_index of `count` states of one DCR_SDRF_MODE_* into one output, as a batched dataset: state b's
+ * columns follow state b-1's, with every node id shifted by node_offsets[b] (host int64; node_offsets[b] >= 0 and
+ * node_offsets[b] >= node_offsets[b-1] + n of state b-1).  Writes edge_ptr[count + 1] (device int64): state b's columns
+ * are edge_ptr[b] .. edge_ptr[b+1] - 1, edge_ptr[count] the total.  Same column order, self entries and directed rule as
+ * dcr_sdrf_export_edge_index; nothing is written at or beyond `capacity`.  workspace: device memory of at least
+ * dcr_sdrf_export_edge_index_batch_workspace_bytes(states, count) bytes, 8-byte aligned.  One host-to-device copy and
+ * three launches whatever `count` is (row counts, one scan, one warp per row); enqueues only.  Status 1 before any copy for
+ * count < 1, a null state, states of different modes, inconsistent offsets or a short workspace. */
+int64_t dcr_sdrf_export_edge_index_batch_workspace_bytes(dcr_sdrf* const* states, int count);
+int dcr_sdrf_export_edge_index_batch(dcr_sdrf* const* states, int count, const int64_t* node_offsets, int64_t* src,
+                                     int64_t* dst, int64_t capacity, int64_t* edge_ptr, void* workspace,
+                                     int64_t workspace_bytes, void* stream);
 
 /* DCR_SDRF_MODE_BFC_PAPER states only: rowptr[n+1] and the fp64 paper-flavour curvature of every directed entry in
  * SORTED order per row (the layout of dcr_sdrf_export's colidx_sorted / c32_sorted).  That mode keeps no fp32 curvature
